@@ -482,7 +482,7 @@ def bench_main(args, w, bm):
             objs = [None] * world
             dist.all_gather_object(objs, check)
 
-    e2e = None if args.no_e2e else _e2e_sharded(hb, H, A, B, w, max(1, min(args.steps, 3)), local_rank)
+    e2e = None if args.no_e2e else _e2e_sharded(hb, H, A, B, w, args.steps, local_rank)
 
     if rank == 0:
         peak, peak_src = bm.fp64_peak()

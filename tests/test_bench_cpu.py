@@ -3,6 +3,7 @@ import json
 import os
 import subprocess
 import sys
+import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -63,6 +64,48 @@ def test_config_cases_cover_the_baseline_configs():
     # the committed single-GPU values every world size is checked against
     exp = bench.expected_results()
     assert bench.expected_key(head) in exp and exp[bench.expected_key(head)]["products"] == 2255020
+
+
+class _FakeResult:
+    """Stands in for a product result: export_leaves / get_params as the engine's matrix answers them."""
+
+    def __init__(self, bi, bj, tiles, b):
+        self.bi, self.bj, self.tiles, self.b = bi, bj, tiles, b
+
+    def export_leaves(self, tiles=True, norms=True):
+        return self.bi, self.bj, None, self.tiles
+
+    def get_params(self):
+        return types.SimpleNamespace(blocksize=self.b)
+
+
+def test_dump_outputs_writes_sorted_float_tables_and_a_seeded_tile_sample(tmp_path, monkeypatch):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    b, n = 4, 300
+    rng = np.random.default_rng(1)
+    keys = rng.choice(64 * 64, n, replace=False)                 # distinct tiles, exported in no particular order
+    bi, bj = keys // 64, keys % 64
+    tiles = rng.standard_normal((n, b * b))
+    monkeypatch.setattr(bench, "DUMP_TABLE_MAX", 200)
+    monkeypatch.setattr(bench, "DUMP_TILE_BYTES", 50 * b * b * 8)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), _FakeResult(bi, bj, tiles, b), 1234, n)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and all(x.endswith(".npy") for x in names)
+    got = {x[:-4]: np.load(tmp_path / "a" / x) for x in names}
+    for x in names:      # same inputs, same files
+        assert np.array_equal(got[x[:-4]], np.load(tmp_path / "b" / x))
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert got["counts"].tolist() == [1234.0, n]
+    r, c = got["c_tiles_row"], got["c_tiles_col"]
+    assert len(r) == 200 and np.all(np.diff(r * 64 + c) > 0)    # a sample, in (row, col) order
+    dense = {(int(i), int(j)): t.reshape(b, b).T for i, j, t in zip(bi, bj, tiles)}
+    assert np.allclose(got["c_tiles_frob_sq"], [np.sum(dense[(int(i), int(j))] ** 2) for i, j in zip(r, c)])
+    assert got["c_sample_tiles"].shape == (50, b, b)
+    for i, j, t in zip(got["c_sample_row"], got["c_sample_col"], got["c_sample_tiles"]):
+        assert np.array_equal(t, dense[(int(i), int(j))])
 
 
 def test_peaks_name_their_source():

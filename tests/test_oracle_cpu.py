@@ -137,19 +137,19 @@ def test_flat_rule_equals_hierarchical_rule_on_port():
 
 @pytest.mark.parametrize("dtype,spamm,tau", [(np.float64, True, 1e-4), (np.float64, False, 0.0), (np.float32, True, 1e-3)])
 def test_single_tile_subproblem_is_the_full_products_tile(dtype, spamm, tau):
-    """oracle/sampled_check.reference_tile (block row of A times block column of B, run through the unmodified
-    reference) gives, for every sampled C tile, exactly the k-list and the values of that tile in the reference's
-    FULL product -- the property bench.py --check and the full-size GPU tests rely on."""
-    if not po.have_ref():
-        pytest.skip("oracle/_ref not built")
+    """oracle/sampled_check.reference_tile (block row of A times block column of B, run through the checker bench.py
+    --check uses: the unmodified reference where oracle/_ref is built, else the pinned port) gives, for every sampled
+    C tile, exactly the k-list and the values of that tile in the checker's FULL product -- the property bench.py
+    --check and the full-size GPU tests rely on."""
     from oracle import sampled_check as sc
+    K = sc.checker_class()
     n, b, lam = 1024, 32, 0.08
     W = min(G.decay_width(lam), n - 1)
     (ra, ca, va) = G.decay_coo(n, lam, W, 1, dtype=dtype)
     (rb, cb, vb) = G.decay_coo(n, lam, W, 2, dtype=dtype)
-    A = po.from_coo(po.RefMatrix, b, n, n, ra, ca, va, dtype)
-    B = po.from_coo(po.RefMatrix, b, n, n, rb, cb, vb, dtype)
-    Cf, nm, nb, tasks = po.RefMatrix.product(A, 0, B, 0, spamm=spamm, tau=tau, want_tasks=True)
+    A = po.from_coo(K, b, n, n, ra, ca, va, dtype)
+    B = po.from_coo(K, b, n, n, rb, cb, vb, dtype)
+    Cf, nm, nb, tasks = K.product(A, 0, B, 0, spamm=spamm, tau=tau, want_tasks=True)
     D = Cf.to_dense()
     cbi, cbj, _, _ = Cf.leaves(tiles=False)
     abi, abj, an, _ = A.leaves(tiles=False)
@@ -157,7 +157,7 @@ def test_single_tile_subproblem_is_the_full_products_tile(dtype, spamm, tau):
     rng = np.random.default_rng(3)
     for t in [0, len(cbi) - 1] + list(rng.integers(0, len(cbi), 6)):
         ci, cj = int(cbi[t]), int(cbj[t])
-        ks, tile, a_n, b_n = sc.reference_tile(po.RefMatrix, n, b, lam, W, (1, 2), ci, cj, spamm, tau, dtype)
+        ks, tile, a_n, b_n = sc.reference_tile(K, n, b, lam, W, (1, 2), ci, cj, spamm, tau, dtype)
         want = np.sort(tasks[(tasks[:, 0] == ci) & (tasks[:, 1] == cj), 2])
         assert np.array_equal(ks, want)
         want_tile = D[ci * b:(ci + 1) * b, cj * b:(cj + 1) * b].astype(np.float64)
@@ -169,7 +169,7 @@ def test_single_tile_subproblem_is_the_full_products_tile(dtype, spamm, tau):
         ci = int(cbi[len(cbi) // 2])
         cj = max(j for (i, j) in have if i == ci) + 1
         if cj < n // b:
-            ks, tile, _, _ = sc.reference_tile(po.RefMatrix, n, b, lam, W, (1, 2), ci, cj, spamm, tau, dtype)
+            ks, tile, _, _ = sc.reference_tile(K, n, b, lam, W, (1, 2), ci, cj, spamm, tau, dtype)
             assert len(ks) == 0
     # the flat-rule checksum over the reference's leaf norms equals the checksum of the reference's executed set
     bbi, bbj, bn, _ = B.leaves(tiles=False)
