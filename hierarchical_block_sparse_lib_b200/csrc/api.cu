@@ -426,7 +426,11 @@ int hbsm_stage_times_last(hbsm_stage_times* out) {
     return guarded([&] { *out = engine().last; });
 }
 int hbsm_set_gemm_variant(int variant) {
-    return guarded([&] { shared().gemm_variant.store(variant); });
+    return guarded([&] {
+        if (variant != 0 && variant != 1 && variant != 3)
+            throw Error(HBSM_E_ARG, "hbsm_b200: gemm variant " + std::to_string(variant) + " does not exist (0, 1 or 3)");
+        shared().gemm_variant.store(variant);
+    });
 }
 
 int hbsm_device_table(hbsm_handle h, size_t* n_tiles, const uint64_t** d_morton_keys, const void** d_norms,

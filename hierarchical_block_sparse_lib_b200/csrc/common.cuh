@@ -39,7 +39,7 @@ struct Error : public std::runtime_error {
 struct Shared {
     std::atomic<int> device{-1};
     std::atomic<uint64_t> launches{0};     // kernels launched by this library, all threads
-    std::atomic<int> gemm_variant{0};      // 0 auto (TMA-tiled DMMA), 1 generic scalar kernel, 2 bulk-copy DMMA kernel
+    std::atomic<int> gemm_variant{0};      // 0 tensor-core kernels, 1 generic FMA kernel, 3 fp32 single-C-tile kernels (hbsm_set_gemm_variant)
     std::mutex index_mutex;                // lazily built line indices of matrices shared between threads
 };
 Shared& shared();
@@ -90,7 +90,7 @@ struct Engine {
     uint64_t launches = 0;  // kernels launched by this thread
     bool ready = false;
     std::string name;
-    int last_gemm_kernel = 0;  // which leaf kernel the last product ran: 0 generic, 1 TMA-tiled DMMA, 2 bulk-copy DMMA
+    int last_gemm_kernel = 0;  // which leaf kernel the last product ran: 0 generic FMA, 1 fp64 TMA-tiled DMMA, 3 fp32 tcgen05
     hbsm_stage_times last{};
     // pinned, device-mapped host words: kernels post the few scalars the host needs between launches (sizes of the next
     // allocations) straight into host memory, so those read-backs never queue on a PCIe copy engine behind bulk transfers

@@ -1,4 +1,4 @@
-// gemm_common.cuh -- PTX wrappers shared by the leaf-GEMM kernels (mbarrier, TMA bulk copies) and the driver entry
+// gemm_common.cuh -- PTX wrappers shared by the leaf-GEMM kernels (mbarrier) and the driver entry
 // point for tensor-map encoding.
 #pragma once
 #include "matrix.cuh"
@@ -28,12 +28,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
             : "memory");
     } while (!ok);
 }
-// TMA 1-D bulk copy global -> shared, completion counted in bytes on an mbarrier (SASS: UBLKCP)
-__device__ __forceinline__ void tma_bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -56,10 +50,11 @@ inline EncodeTiledFn encode_tiled_fn() {
 
 struct GemmMeta { int ctile; int flags; };   // flags: 1 = first chunk of a C tile, 2 = last chunk, 4 = no more work
 
-// fp32 leaf GEMM on the 5th-generation tensor cores (gemm_f32.cu); false = blocksize/driver not supported
-// ckeys / task_k (C's Morton keys and the k of every product, may be null) let the 32-leaf path pair neighbouring C tiles
-bool launch_gemm_f32_tc(const Matrix& A, bool tA, const Matrix& B, bool tB, const uint2* ab, const uint64_t* begin,
-                        uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, float* Ct, const uint64_t* ckeys = nullptr,
-                        const uint32_t* task_k = nullptr, size_t n_products = 0);
+// fp32 leaf GEMM on the 5th-generation tensor cores (gemm_f32.cu) for leaves of 32, 64, 128 and 256.  Leaves of 32 and 64 run
+// the kernels over 2 x 2 groups of C tiles, which are built from ckeys and task_k (C's Morton keys and the k of every product);
+// single_tile runs the single-C-tile kernels there instead (the parity hook of hbsm_set_gemm_variant(3)).
+void launch_gemm_f32_tc(const Matrix& A, bool tA, const Matrix& B, bool tB, const uint2* ab, const uint64_t* begin,
+                        uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, float* Ct, const uint64_t* ckeys,
+                        const uint32_t* task_k, size_t n_products, bool single_tile);
 
 }  // namespace hbsm_b200

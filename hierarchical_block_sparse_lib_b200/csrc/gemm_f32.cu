@@ -26,8 +26,8 @@
 // K-major uses the canonical SWIZZLE_128B layout; MN-major 32-bit operands must use the 128B-swizzle-with-32B-atom
 // layout (4 k rows per atom; TMA CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, descriptor layout type 1).  All four (tA,tB)
 // combinations therefore only differ in the tensor map and a few descriptor fields -- no transposition pass.
-// The MMA is always issued with M = 128 (for 32- and 64-row tiles the upper accumulator rows are never read; the
-// instruction costs the same as M = 64), which keeps the simple TMEM layout "row i = lane i".
+// This kernel serves leaves of 128 and 256 (128-row compute tiles, M = 128: C row i is TMEM lane i); leaves of 32 and 64
+// have kernels of their own below.
 #include "gemm_common.cuh"
 
 namespace hbsm_b200 {
@@ -82,31 +82,29 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes
            (1ull << 46) | ((uint64_t)layout_type << 61);
 }
 
-template <int BS, int MM = 128>
+template <int BS>
 struct F32Cfg {
-    static constexpr int KC = BS == 128 ? 32 : BS;          // K-chunk per pipeline stage
+    static_assert(BS == 128, "128-row compute tiles");
+    static constexpr int KC = 32;                           // K-chunk per pipeline stage
     static constexpr int NCHUNK = BS / KC;
     static constexpr int OPER_BYTES = BS * KC * 4;          // one operand chunk (raw == hi), same again for lo
     static constexpr int STAGE_BYTES = 4 * OPER_BYTES;      // A_hi | A_lo | B_hi | B_lo
     static constexpr int NST = (196 * 1024 / STAGE_BYTES) > 8 ? 8 : (196 * 1024 / STAGE_BYTES);
-    static constexpr int TAIL_PAD = 16 * 1024;              // M=128 descriptors of a 32/64-row A may read past the last stage
     static constexpr int HEADER_BYTES = 1024;
-    static constexpr int SMEM_BYTES = 1024 + HEADER_BYTES + NST * STAGE_BYTES + TAIL_PAD;
+    static constexpr int SMEM_BYTES = 1024 + HEADER_BYTES + NST * STAGE_BYTES;
     // Independent TMEM accumulators per leaf product.  Back-to-back MMAs into ONE accumulator serialise on its
-    // read-modify-write latency (measured ~100 clk per N=64 MMA instead of the 32 clk dispatch floor), so the three
-    // terms lo*hi, hi*lo, hi*hi go to separate accumulators (two for 128-tiles: TMEM has 512 columns) and the epilogue
-    // adds them.  x2 for the double-buffered hand-off to the epilogue.
-    static constexpr int NACC = BS == 128 ? 2 : 3;
+    // read-modify-write latency (measured ~100 clk per N=64 MMA instead of the 32 clk dispatch floor), so the hi*hi term
+    // gets an accumulator of its own and lo*hi, hi*lo share the other (TMEM has 512 columns); the epilogue adds them.
+    // x2 for the double-buffered hand-off to the epilogue.
+    static constexpr int NACC = 2;
     static constexpr int ACC_COLS = NACC * BS;
-    static constexpr int TMEM_COLS = 2 * ACC_COLS <= 32 ? 32 : (2 * ACC_COLS <= 64 ? 64 : (2 * ACC_COLS <= 128 ? 128 : (2 * ACC_COLS <= 256 ? 256 : 512)));
-    static_assert(2 * ACC_COLS <= 512, "TMEM has 512 columns");
+    static constexpr int TMEM_COLS = 2 * ACC_COLS;
+    static_assert(TMEM_COLS == 512, "TMEM has 512 columns");
     static constexpr int THREADS = 512;
     static constexpr int CVT_WARPS = 4;
-    // TMEM lane quadrants holding live C rows: M = 128 puts row i in lane i; M = 64 puts row i in lane 32*(i/16) + i%16
-    static constexpr int EPI_Q = MM == 64 ? BS / 16 : (BS >= 128 ? 4 : (BS + 31) / 32);
-    static constexpr int EPI_H = BS >= 64 ? 2 : 1;                  // column halves: two warps share a quadrant
+    static constexpr int EPI_H = 2;                                 // column halves: two warps share a TMEM lane quadrant
     static constexpr int EPI_CW = BS / EPI_H;                       // columns per epilogue warp
-    static constexpr int EPI_WARPS = EPI_Q * EPI_H;
+    static constexpr int EPI_WARPS = 4 * EPI_H;
     static constexpr int KSTEPS = KC / 8;
     static_assert(NST >= 2, "pipeline needs two stages");
 };
@@ -125,16 +123,15 @@ struct F32Header {
     GemmMeta ring[16];
 };
 
-// LS = leaf size (H:167 blocksize), BS = the square compute tile one CTA accumulates (BS == LS for leaves up to 128; a
+// LS = leaf size (H:167 blocksize), BS = the square compute tile one CTA accumulates (BS == LS for 128-leaves; a
 // 256-leaf is processed as 2 x 2 C sub-tiles whose k-lists are the leaf's k-list with both 128-wide halves of each
 // operand: the tensor-map coordinates address the sub-blocks in place, ld = LS).
-template <int LS, int BS, int MM, bool TA, bool TB>
-__global__ void __launch_bounds__(F32Cfg<BS, MM>::THREADS, 1)
+template <int LS, int BS, bool TA, bool TB>
+__global__ void __launch_bounds__(F32Cfg<BS>::THREADS, 1)
 k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
               const uint2* __restrict__ ab, const uint64_t* __restrict__ begin, uint32_t n_ctiles,
-              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct, int raw_hi /* development switches, see f32_mode() */) {
-    using Cfg = F32Cfg<BS, MM>;
-    static_assert(MM == 128 || (MM == 64 && BS <= 64), "MMA M shape");
+              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct) {
+    using Cfg = F32Cfg<BS>;
     constexpr int S = LS / BS;            // sub-tiles per leaf side
     static_assert(LS % BS == 0 && (S == 1 || S == 2), "leaf / compute-tile shapes");
     constexpr int NST = Cfg::NST, KC = Cfg::KC;
@@ -229,7 +226,7 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             // instruction descriptor: D fp32 [4,6)=1, A/B tf32 [7,10)=[10,13)=2, a_major bit 15, b_major bit 16 (1 = MN-major),
             // N>>3 at [17,23), M>>4 at [24,29)
             constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((TA ? 0u : 1u) << 15) | ((TB ? 1u : 0u) << 16) |
-                                       ((uint32_t)(BS >> 3) << 17) | ((uint32_t)(MM >> 4) << 24);
+                                       ((uint32_t)(BS >> 3) << 17) | ((uint32_t)(BS >> 4) << 24);
             // K-major: SWIZZLE_128B (type 2), 8-row groups 1024 B apart.  MN-major fp32: 32-byte-atom swizzle (type 1), 4 k rows
             // per atom (SBO = 512 B), 32-element MN chunks one slab (LBO) apart.
             constexpr uint32_t A_LBO = TA ? 16 : KC * 128, B_LBO = TB ? KC * 128 : 16;
@@ -254,13 +251,11 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                     open = false;
                 }
                 tc_fence_after();
-                const uint32_t d_small = tmem_base + as * Cfg::ACC_COLS;                    // lo*hi (and hi*lo when NACC == 2)
-                const uint32_t d_small2 = d_small + (Cfg::NACC == 3 ? BS : 0);              // hi*lo
-                const uint32_t d_big = d_small + (Cfg::NACC - 1) * BS;                      // hi*hi
+                const uint32_t d_small = tmem_base + as * Cfg::ACC_COLS;                    // lo*hi + hi*lo
+                const uint32_t d_big = d_small + BS;                                        // hi*hi
                 const uint32_t sa = smem_u32(stages + (size_t)s * Cfg::STAGE_BYTES);
                 const uint32_t a_hi = sa, a_lo = sa + Cfg::OPER_BYTES, b_hi = sa + 2 * Cfg::OPER_BYTES, b_lo = sa + 3 * Cfg::OPER_BYTES;
                 // MN-major: 8 k rows = 1024 B per step; K-major: 32 B inside the 128-B row, next slab every 4 steps
-                if (!(raw_hi & 16)) {
 #pragma unroll
                 for (int ks = 0; ks < Cfg::KSTEPS; ++ks) {
                     const uint32_t ao = TA ? (uint32_t)((ks >> 2) * (BS * 128) + (ks & 3) * 32) : (uint32_t)(ks * 1024);
@@ -268,10 +263,9 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                     const uint64_t dah = umma_desc(a_hi + ao, A_LBO, A_SBO, A_LT), dal = umma_desc(a_lo + ao, A_LBO, A_SBO, A_LT);
                     const uint64_t dbh = umma_desc(b_hi + bo, B_LBO, B_SBO, B_LT), dbl = umma_desc(b_lo + bo, B_LBO, B_SBO, B_LT);
                     mma_tf32(d_small, dal, dbh, IDESC, open ? 1u : 0u);
-                    mma_tf32(d_small2, dah, dbl, IDESC, (open || Cfg::NACC == 2) ? 1u : 0u);
+                    mma_tf32(d_small, dah, dbl, IDESC, 1u);
                     mma_tf32(d_big, dah, dbh, IDESC, open ? 1u : 0u);
                     open = true;
-                }
                 }
                 tc_commit(smem_u32(&hd->empty[s]));             // stage free when these MMAs have read it
                 if (m.flags & 16) {                             // product complete: hand the accumulator to the epilogue
@@ -284,26 +278,26 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             }
         }
     } else if (warp >= 4 && warp < 4 + Cfg::CVT_WARPS) {
-        // ===== hi/lo split: raw fp32 (A at +0, B at +2*OPER) -> hi in place, lo at +OPER =====
+        // ===== hi/lo split: raw fp32 (A at +0, B at +2*OPER) stays in place as hi, lo at +OPER =====
         const unsigned tid = threadIdx.x - 128;
         for (uint32_t it = 0;; ++it) {
             const uint32_t s = it % NST, ph = (it / NST) & 1u;
             mbar_wait(smem_u32(&hd->full_raw[s]), ph);
             const int flags = hd->meta[s].flags;
-            if (!(flags & 4) && !(raw_hi & 4)) {
+            if (!(flags & 4)) {
                 unsigned char* st = stages + (size_t)s * Cfg::STAGE_BYTES;
 #pragma unroll
                 for (int op = 0; op < 2; ++op) {
-                    float4* hi = reinterpret_cast<float4*>(st + op * 2 * Cfg::OPER_BYTES);
+                    const float4* hi = reinterpret_cast<const float4*>(st + op * 2 * Cfg::OPER_BYTES);
                     float4* lo = reinterpret_cast<float4*>(st + op * 2 * Cfg::OPER_BYTES + Cfg::OPER_BYTES);
 #pragma unroll 4
                     for (int i = (int)tid; i < Cfg::OPER_BYTES / 16; i += Cfg::CVT_WARPS * 32) {
-                        float4 x = hi[i], h, l;
-                        h.x = __uint_as_float(__float_as_uint(x.x) & 0xFFFFE000u); l.x = x.x - h.x;
-                        h.y = __uint_as_float(__float_as_uint(x.y) & 0xFFFFE000u); l.y = x.y - h.y;
-                        h.z = __uint_as_float(__float_as_uint(x.z) & 0xFFFFE000u); l.z = x.z - h.z;
-                        h.w = __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u); l.w = x.w - h.w;
-                        if (!(raw_hi & 1)) hi[i] = h;   // raw_hi: the tensor core drops the 13 low mantissa bits itself
+                        const float4 x = hi[i];
+                        float4 l;
+                        l.x = x.x - __uint_as_float(__float_as_uint(x.x) & 0xFFFFE000u);
+                        l.y = x.y - __uint_as_float(__float_as_uint(x.y) & 0xFFFFE000u);
+                        l.z = x.z - __uint_as_float(__float_as_uint(x.z) & 0xFFFFE000u);
+                        l.w = x.w - __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u);
                         lo[i] = l;
                     }
                 }
@@ -313,11 +307,11 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             if (lane == 0) mbar_arrive(smem_u32(&hd->full_cvt[s]));
             if (flags & 4) break;
         }
-    } else if (warp >= 8 && ((warp - 8) & 3) < Cfg::EPI_Q && ((warp - 8) >> 2) < Cfg::EPI_H) {
+    } else if (warp >= 8 && (warp - 8) < Cfg::EPI_WARPS) {
         // ===== epilogue: warp (q,h) owns TMEM lanes [32q, 32q+32) = C rows, columns [h*CW, (h+1)*CW) =====
         const unsigned q = (warp - 8) & 3, h = (warp - 8) >> 2;
         constexpr int CW = Cfg::EPI_CW;
-        const int row = MM == 64 ? (lane < 16 ? (int)(q * 16 + lane) : BS) : (int)(q * 32 + lane);
+        const int row = (int)(q * 32 + lane);
         float acc[CW];
         for (uint32_t pc = 0;; ++pc) {
             const uint32_t as = pc & 1u;
@@ -327,7 +321,7 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             const int ctile = hd->acc_tile[as];
             tc_fence_after();
 #pragma unroll
-            for (int c0 = 0; c0 < CW && !(raw_hi & 8); c0 += 32) {
+            for (int c0 = 0; c0 < CW; c0 += 32) {
 #pragma unroll
                 for (int a = 0; a < Cfg::NACC; ++a) {      // small terms first, the hi*hi accumulator last
                     uint32_t r[32];
@@ -345,7 +339,7 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(smem_u32(&hd->tmem_empty[as]));
-            if ((flags & 2) && row < BS) {
+            if (flags & 2) {
                 const unsigned tile = (unsigned)ctile / (S * S), sub = (unsigned)ctile % (S * S);
                 float* C = Ct + (size_t)tile * LS * LS + (size_t)((sub / S) * BS + h * CW) * LS + (sub % S) * BS + row;
 #pragma unroll
@@ -379,9 +373,9 @@ struct Q4Cfg {
     static constexpr int OPER_BYTES = BS * KC * 4;
     static constexpr int PROD_BYTES = 4 * OPER_BYTES;        // one product: A (hi+lo) | B (hi+lo)
     // Products per pipeline stage.  The producer lane, the MMA-issuing lane and the hand-offs between the roles cost several
-    // hundred clocks PER STAGE whatever its size (measured with HBSM_F32_PROF: at one 32-leaf product per stage the issuing
-    // lane was busy 656 clk per product for 188 clk of MMAs), so a stage carries up to GP consecutive products of one C tile:
-    // 64 KiB of operands per stage at both leaf sizes.  The GP products are chained into ONE TMEM accumulator set (16 MMAs at
+    // hundred clocks PER STAGE whatever its size (measured, profiles/r02_f32_small_leaves.md: at one 32-leaf product per stage
+    // the issuing lane was busy 656 clk per product for 188 clk of MMAs), so a stage carries up to GP consecutive products of
+    // one C tile: 64 KiB of operands per stage at both leaf sizes.  The GP products are chained into ONE TMEM accumulator set (16 MMAs at
     // 32-leaves, 8 at 64; the tensor core truncates when it adds into the accumulator, so chains stay short: bias ~16 * 2^-24
     // relative, inside the 1e-5 bar); the epilogue adds the chains in k order with round-to-nearest fp32 adds.
     static constexpr int GP = BS == 32 ? 4 : 1;
@@ -415,13 +409,8 @@ template <int BS, bool TA, bool TB>
 __global__ void __launch_bounds__(Q4Cfg<BS>::THREADS, 1)
 k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
               const uint2* __restrict__ ab, const uint64_t* __restrict__ begin, uint32_t n_ctiles,
-              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct,
-              int dbg /* timing ablations with WRONG results, see f32_mode(): 4 no split, 8 no drain, 16 no MMAs, 64 no TMA */,
-              unsigned long long* __restrict__ prof /* null, or 16 counters: block 0's wait / total clocks per role (HBSM_F32_PROF=1) */) {
+              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct) {
     using Cfg = Q4Cfg<BS>;
-    const bool profiling = prof != nullptr && blockIdx.x == 0;
-    long long t_role0 = 0, t_wait = 0, t_wait2 = 0;
-#define HB_PWAIT(acc, call) do { if (profiling) { const long long t_ = clock64(); call; acc += clock64() - t_; } else { call; } } while (0)
     constexpr int NST = Cfg::NST, KC = Cfg::KC;
     extern __shared__ unsigned char smem_raw[];
     unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -447,7 +436,6 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = hd->tmem_base;
-    if (profiling) t_role0 = clock64();
 
     if (warp == 0) {
         // ===== TMA producer: raw operand slabs land in the "hi" positions of the stacked layout.  The warp walks the task
@@ -478,16 +466,15 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                     // "copies issued" is on the critical path)
                     const uint2 tj = Cfg::GP > 1 ? mine : make_uint2(__shfl_sync(0xffffffffu, mine.x, j0), __shfl_sync(0xffffffffu, mine.y, j0));
                     if (lane == 0) {
-                        HB_PWAIT(t_wait, mbar_wait(smem_u32(&hd->empty[s]), ph ^ 1u));
+                        mbar_wait(smem_u32(&hd->empty[s]), ph ^ 1u);
                         hd->ring[it & 15u].ctile = (int)tile;
                         hd->ring[it & 15u].flags = (pb + j0 == p0 ? 1 : 0) | (pb + j0 + n == p1 ? 2 : 0) | (n << 8);
-                        if (dbg & 64) mbar_arrive(fb);
-                        else mbar_arrive_expect_tx(fb, (uint32_t)n * 2u * Cfg::OPER_BYTES);
+                        mbar_arrive_expect_tx(fb, (uint32_t)n * 2u * Cfg::OPER_BYTES);
                     }
                     if (Cfg::GP > 1) __syncwarp();
                     // lanes j0 .. j0 + n - 1 issue one product's copies each (GP = 1: lane 0 issues for lane j0)
                     const int l = Cfg::GP > 1 ? (int)lane - j0 : (lane == 0 ? 0 : -1);
-                    if (l >= 0 && l < n && !(dbg & 64)) {
+                    if (l >= 0 && l < n) {
                         const uint2 t = tj;
                         const uint32_t sa = smem_u32(stages + (size_t)s * Cfg::STAGE_BYTES + (size_t)l * Cfg::PROD_BYTES);
                         const uint32_t sb = sa + 2 * Cfg::OPER_BYTES;
@@ -510,7 +497,6 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                 }
             }
         }
-        if (profiling && lane == 0) { prof[0] = (unsigned long long)t_wait; prof[1] = (unsigned long long)(clock64() - t_role0); prof[2] = it; }
         if (lane == 0) {   // one terminal stage per split group (each of them watches only its own stages)
             for (int e = 0; e < Cfg::CVT_GROUPS; ++e, ++it) {
                 const uint32_t s = it % NST, ph = (it / NST) & 1u;
@@ -534,12 +520,11 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             int in_chain = 0;
             for (uint32_t it = 0;; ++it) {
                 const uint32_t s = it % NST, ph = (it / NST) & 1u;
-                HB_PWAIT(t_wait, mbar_wait(smem_u32(&hd->full_cvt[s]), ph));
+                mbar_wait(smem_u32(&hd->full_cvt[s]), ph);
                 const GemmMeta m = hd->ring[it & 15u];
                 const uint32_t as = chain % Cfg::NSETS;
-                if (in_chain == 0) HB_PWAIT(t_wait2, mbar_wait(smem_u32(&hd->tmem_empty[as]), ((chain / Cfg::NSETS) & 1u) ^ 1u));   // epilogue drained this set
+                if (in_chain == 0) mbar_wait(smem_u32(&hd->tmem_empty[as]), ((chain / Cfg::NSETS) & 1u) ^ 1u);   // epilogue drained this set
                 if (m.flags & 4) {   // (a chain never spans C tiles, so none is open here)
-                    if (profiling) { prof[3] = (unsigned long long)t_wait; prof[4] = (unsigned long long)t_wait2; prof[5] = (unsigned long long)(clock64() - t_role0); }
                     mbar_arrive(smem_u32(&hd->tmem_full[as]));   // the epilogue finds the terminal entry in the ring itself
                     break;
                 }
@@ -549,7 +534,6 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                 const uint32_t s0 = smem_u32(stages + (size_t)s * Cfg::STAGE_BYTES);
                 // descriptors of the stage's first product, first K-step; the others differ in the start-address field only
                 const uint64_t da0 = umma_desc(s0, A_LBO, A_SBO, A_LT), db0 = umma_desc(s0 + 2 * Cfg::OPER_BYTES, B_LBO, B_SBO, B_LT);
-                if (!(dbg & 16))
                 for (int j = 0; j < n; ++j) {
 #pragma unroll
                     for (int ks = 0; ks < Cfg::KSTEPS; ++ks) {
@@ -572,10 +556,9 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
         const unsigned tid = ((warp - 2) % Cfg::CVT_WPG) * 32 + lane;
         for (uint32_t it = (warp - 2) / Cfg::CVT_WPG;; it += Cfg::CVT_GROUPS) {
             const uint32_t s = it % NST, ph = (it / NST) & 1u;
-            HB_PWAIT(t_wait, mbar_wait(smem_u32(&hd->full_raw[s]), ph));
+            mbar_wait(smem_u32(&hd->full_raw[s]), ph);
             const int flags = hd->ring[it & 15u].flags;
-            if (profiling && (flags & 4) && warp == 2 && lane == 0) { prof[6] = (unsigned long long)t_wait; prof[7] = (unsigned long long)(clock64() - t_role0); }
-            if (!(flags & 4) && !(dbg & 4))
+            if (!(flags & 4))
             for (int pj = 0; pj < (Cfg::GP == 1 ? 1 : (flags >> 8)); ++pj) {
                 unsigned char* st = stages + (size_t)s * Cfg::STAGE_BYTES + (size_t)pj * Cfg::PROD_BYTES;
 #pragma unroll
@@ -601,7 +584,7 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                     }
                 }
             }
-            if (!(flags & 4) && !(dbg & 4)) fence_proxy_async();
+            if (!(flags & 4)) fence_proxy_async();
             __syncwarp();
             if (lane == 0) mbar_arrive(smem_u32(&hd->full_cvt[s]));
             if (flags & 4) break;
@@ -617,14 +600,11 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
         uint32_t it_e = 0;            // stage sequence number of the next ring entry this warp consumes
         for (uint32_t pc = 0;; ++pc) {
             const uint32_t as = pc % Cfg::NSETS;
-            HB_PWAIT(t_wait, mbar_wait(smem_u32(&hd->tmem_full[as]), (pc / Cfg::NSETS) & 1u));
+            mbar_wait(smem_u32(&hd->tmem_full[as]), (pc / Cfg::NSETS) & 1u);
             // the accumulator set holds the stages [it_e, ...) of one chain: up to CH stages, closed early by the end of the C tile
             GemmMeta m = hd->ring[it_e & 15u];
             int flags = m.flags & 7;
-            if (flags & 4) {
-                if (profiling && warp == 8 && lane == 0) { prof[8] = (unsigned long long)t_wait; prof[9] = (unsigned long long)(clock64() - t_role0); prof[10] = pc; }
-                break;
-            }
+            if (flags & 4) break;
             ++it_e;
 #pragma unroll
             for (int c = 1; c < Cfg::CH; ++c) {
@@ -636,14 +616,9 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             const int ctile = m.ctile;
             tc_fence_after();
             uint32_t r1[32], r2[32];
-            if (!(dbg & 8)) {
-                tmem_ld32(tmem_base + ((q * 32u) << 16) + as * Cfg::NN + BS + h * 32, r2);   // x * B_lo
-                tmem_ld32(tmem_base + ((q * 32u) << 16) + as * Cfg::NN + h * 32, r1);        // x * B_hi
-                tmem_ld_wait();
-            } else {
-#pragma unroll
-                for (int j = 0; j < 32; ++j) { r1[j] = 0u; r2[j] = 0u; }
-            }
+            tmem_ld32(tmem_base + ((q * 32u) << 16) + as * Cfg::NN + BS + h * 32, r2);   // x * B_lo
+            tmem_ld32(tmem_base + ((q * 32u) << 16) + as * Cfg::NN + h * 32, r1);        // x * B_hi
+            tmem_ld_wait();
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(smem_u32(&hd->tmem_empty[as]));
@@ -673,31 +648,19 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
     __syncthreads();
     tc_fence_after();
     if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
-#undef HB_PWAIT
-}
-
-// development switches (HBSM_F32_MODE): bit 0 = leave the raw operand in place as "hi", bit 1 = issue M = 64 MMAs for leaves <= 64;
-// timing experiments with WRONG results: 4 = skip the hi/lo split, 8 = skip the TMEM drain, 16 = skip the MMAs, 64 = skip the
-// TMA loads (stacked kernel only);
-// 32 = use the three-MMA kernel for leaves of 32 / 64 as well (instead of the stacked-operand kernel); 128 = 32-leaves: the
-// single-tile stacked kernel instead of the grouped one
-int f32_mode() {
-    static int mode = -1;
-    if (mode < 0) { const char* e = getenv("HBSM_F32_MODE"); mode = e ? atoi(e) : 1; }   // default: raw operand as "hi"
-    return mode;
 }
 
 // 2-D fp32 view of a tile pool: dim0 = leaf row (contiguous), dim1 = leaf column + BS * tile; 128-B swizzled boxes
-bool make_f32_map(CUtensorMap* map, const void* tiles, size_t n_tiles, int LS, int box_rows, int box_cols, bool mn_major) {
+void make_f32_map(CUtensorMap* map, const void* tiles, size_t n_tiles, int LS, int box_rows, int box_cols, bool mn_major) {
     EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc) return false;
     cuuint64_t gdim[2] = {(cuuint64_t)LS, (cuuint64_t)LS * n_tiles};
     cuuint64_t gstr[1] = {(cuuint64_t)LS * 4};
     cuuint32_t box[2] = {(cuuint32_t)box_rows, (cuuint32_t)box_cols};
     cuuint32_t estr[2] = {1, 1};
-    return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(tiles), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    if (!enc || enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(tiles), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        throw Error(HBSM_E_CUDA, "hbsm_b200: the driver refused the tensor map of an fp32 leaf operand");
 }
 
 
@@ -1034,13 +997,13 @@ __global__ void k_g32_merge(const uint64_t* __restrict__ ckeys, const uint32_t* 
 }
 
 template <bool TA, bool TB>
-bool launch_g32_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys, const uint32_t* task_k,
+void launch_g32_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys, const uint32_t* task_k,
                      const uint32_t* tile_list, uint32_t n_ctiles, size_t n_products, float* Ct) {
     using Cfg = G32Cfg;
     CUtensorMap mapA, mapB, mapZ;
-    if (!make_f32_map(&mapA, A.tiles.p, A.L, 32, 32, 32, !TA)) return false;
-    if (!make_f32_map(&mapB, B.tiles.p, B.n_ext(), 32, 32, 32, TB)) return false;
-    if (!make_f32_map(&mapZ, zero_leaf_f32(), 1, 32, 32, 32, !TA)) return false;
+    make_f32_map(&mapA, A.tiles.p, A.L, 32, 32, 32, !TA);
+    make_f32_map(&mapB, B.tiles.p, B.n_ext(), 32, 32, 32, TB);
+    make_f32_map(&mapZ, zero_leaf_f32(), 1, 32, 32, 32, !TA);
     // (one zero map serves both operands: the swizzle mode only permutes where the zeros land)
     DevBuf<uint32_t> head(n_ctiles), cnt(n_ctiles);
     DevBuf<uint64_t> gpos((size_t)n_ctiles + 1), gbegin((size_t)n_ctiles + 1);
@@ -1065,15 +1028,14 @@ bool launch_g32_inst(const Matrix& A, const Matrix& B, const uint2* ab, const ui
     }
     const unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
     HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, mapZ, gops.p, gbegin.p, gtiles.p, gpos.p + n_ctiles, counter.p, Ct);
-    return true;
 }
 
-bool launch_g32(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys,
+void launch_g32(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys,
                 const uint32_t* task_k, const uint32_t* tile_list, uint32_t n, size_t n_products, float* Ct) {
-    if (!tA && !tB) return launch_g32_inst<false, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    if (!tA && tB) return launch_g32_inst<false, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    if (tA && !tB) return launch_g32_inst<true, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    return launch_g32_inst<true, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    if (!tA && !tB) launch_g32_inst<false, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    else if (!tA && tB) launch_g32_inst<false, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    else if (tA && !tB) launch_g32_inst<true, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    else launch_g32_inst<true, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
 }
 
 
@@ -1330,15 +1292,15 @@ k_gemm_f32_g64(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 }
 
 template <bool TA, bool TB>
-bool launch_g64_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys, const uint32_t* task_k,
+void launch_g64_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys, const uint32_t* task_k,
                      const uint32_t* tile_list, uint32_t n_ctiles, size_t n_products, float* Ct) {
     using Cfg = G64Cfg;
     CUtensorMap mapA, mapB, mapZa, mapZb;
     // K-major operand (k along leaf rows): box {32 k, 64 mn};  MN-major: box {32 mn, 32 k}
-    if (!make_f32_map(&mapA, A.tiles.p, A.L, 64, 32, TA ? 64 : 32, !TA)) return false;
-    if (!make_f32_map(&mapB, B.tiles.p, B.n_ext(), 64, 32, TB ? 32 : 64, TB)) return false;
-    if (!make_f32_map(&mapZa, zero_leaf_f32_64(), 1, 64, 32, TA ? 64 : 32, !TA)) return false;
-    if (!make_f32_map(&mapZb, zero_leaf_f32_64(), 1, 64, 32, TB ? 32 : 64, TB)) return false;
+    make_f32_map(&mapA, A.tiles.p, A.L, 64, 32, TA ? 64 : 32, !TA);
+    make_f32_map(&mapB, B.tiles.p, B.n_ext(), 64, 32, TB ? 32 : 64, TB);
+    make_f32_map(&mapZa, zero_leaf_f32_64(), 1, 64, 32, TA ? 64 : 32, !TA);
+    make_f32_map(&mapZb, zero_leaf_f32_64(), 1, 64, 32, TB ? 32 : 64, TB);
     DevBuf<uint32_t> head(n_ctiles), cnt(n_ctiles);
     DevBuf<uint64_t> gpos((size_t)n_ctiles + 1), gbegin((size_t)n_ctiles + 1);
     DevBuf<int4> gtiles(n_ctiles);
@@ -1362,54 +1324,52 @@ bool launch_g64_inst(const Matrix& A, const Matrix& B, const uint2* ab, const ui
     }
     const unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
     HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, mapZa, mapZb, gops.p, gbegin.p, gtiles.p, gpos.p + n_ctiles, counter.p, Ct);
-    return true;
 }
 
-bool launch_g64(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys,
+void launch_g64(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys,
                 const uint32_t* task_k, const uint32_t* tile_list, uint32_t n, size_t n_products, float* Ct) {
-    if (!tA && !tB) return launch_g64_inst<false, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    if (!tA && tB) return launch_g64_inst<false, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    if (tA && !tB) return launch_g64_inst<true, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    return launch_g64_inst<true, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    if (!tA && !tB) launch_g64_inst<false, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    else if (!tA && tB) launch_g64_inst<false, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    else if (tA && !tB) launch_g64_inst<true, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+    else launch_g64_inst<true, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
 }
 
-template <int LS, int BS, int MM, bool TA, bool TB>
-bool launch_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
+template <int LS, int BS, bool TA, bool TB>
+void launch_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
                  const uint32_t* tile_list, unsigned* counter, float* Ct) {
-    using Cfg = F32Cfg<BS, MM>;
+    using Cfg = F32Cfg<BS>;
     CUtensorMap mapA, mapB;
     // K-major operand (k along leaf rows): box {32 k, BS mn};  MN-major: box {32 mn, KC k}
-    if (!make_f32_map(&mapA, A.tiles.p, A.L, LS, 32, TA ? BS : Cfg::KC, !TA)) return false;
-    if (!make_f32_map(&mapB, B.tiles.p, B.n_ext(), LS, 32, TB ? Cfg::KC : BS, TB)) return false;
-    auto kfn = k_gemm_f32_tc<LS, BS, MM, TA, TB>;
+    make_f32_map(&mapA, A.tiles.p, A.L, LS, 32, TA ? BS : Cfg::KC, !TA);
+    make_f32_map(&mapB, B.tiles.p, B.n_ext(), LS, 32, TB ? Cfg::KC : BS, TB);
+    auto kfn = k_gemm_f32_tc<LS, BS, TA, TB>;
     static bool configured = false;
     if (!configured) {
         HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
     const uint64_t units = (uint64_t)n_ctiles * (LS / BS) * (LS / BS);
-    if (units >= 0x7fffffffull) return false;
+    if (units >= 0x7fffffffull) throw Error(HBSM_E_CUDA, "hbsm_b200: too many C sub-tiles for one fp32 leaf-GEMM launch");
     unsigned grid = (unsigned)std::min<uint64_t>(units, (uint64_t)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct, f32_mode());
-    return true;
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct);
 }
 
-template <int LS, int BS, int MM>
-bool launch_bs(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n,
+template <int LS, int BS>
+void launch_bs(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n,
                const uint32_t* tile_list, unsigned* counter, float* Ct) {
-    if (!tA && !tB) return launch_inst<LS, BS, MM, false, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    if (!tA && tB) return launch_inst<LS, BS, MM, false, true>(A, B, ab, begin, n, tile_list, counter, Ct);
-    if (tA && !tB) return launch_inst<LS, BS, MM, true, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    return launch_inst<LS, BS, MM, true, true>(A, B, ab, begin, n, tile_list, counter, Ct);
+    if (!tA && !tB) launch_inst<LS, BS, false, false>(A, B, ab, begin, n, tile_list, counter, Ct);
+    else if (!tA && tB) launch_inst<LS, BS, false, true>(A, B, ab, begin, n, tile_list, counter, Ct);
+    else if (tA && !tB) launch_inst<LS, BS, true, false>(A, B, ab, begin, n, tile_list, counter, Ct);
+    else launch_inst<LS, BS, true, true>(A, B, ab, begin, n, tile_list, counter, Ct);
 }
 
 template <int BS, bool TA, bool TB>
-bool launch_q4_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
+void launch_q4_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
                     const uint32_t* tile_list, unsigned* counter, float* Ct) {
     using Cfg = Q4Cfg<BS>;
     CUtensorMap mapA, mapB;
-    if (!make_f32_map(&mapA, A.tiles.p, A.L, BS, 32, BS, !TA)) return false;
-    if (!make_f32_map(&mapB, B.tiles.p, B.n_ext(), BS, 32, BS, TB)) return false;
+    make_f32_map(&mapA, A.tiles.p, A.L, BS, 32, BS, !TA);
+    make_f32_map(&mapB, B.tiles.p, B.n_ext(), BS, 32, BS, TB);
     auto kfn = k_gemm_f32_q4<BS, TA, TB>;
     static bool configured = false;
     if (!configured) {
@@ -1417,53 +1377,35 @@ bool launch_q4_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uin
         configured = true;
     }
     unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
-    static const bool want_prof = getenv("HBSM_F32_PROF") != nullptr;
-    DevBuf<unsigned long long> prof;
-    if (want_prof) { prof.alloc(16); prof.zero(); }
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct, f32_mode() & (4 | 8 | 16 | 64),
-              prof.p);
-    if (want_prof) {   // diagnosis only: synchronises
-        const std::vector<unsigned long long> h = prof.to_host();
-        fprintf(stderr, "[f32 q4<%d> block 0, clocks] producer: wait-empty %llu of %llu (%llu stages) | issuer: wait-split %llu wait-drain %llu of %llu | "
-                        "split warp 2: wait-TMA %llu of %llu | epilogue warp 8: wait-MMA %llu of %llu (%llu chains)\n",
-                BS, h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9], h[10]);
-    }
-    return true;
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct);
 }
 
 template <int BS>
-bool launch_q4(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n,
+void launch_q4(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n,
                const uint32_t* tile_list, unsigned* counter, float* Ct) {
-    if (!tA && !tB) return launch_q4_inst<BS, false, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    if (!tA && tB) return launch_q4_inst<BS, false, true>(A, B, ab, begin, n, tile_list, counter, Ct);
-    if (tA && !tB) return launch_q4_inst<BS, true, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    return launch_q4_inst<BS, true, true>(A, B, ab, begin, n, tile_list, counter, Ct);
+    if (!tA && !tB) launch_q4_inst<BS, false, false>(A, B, ab, begin, n, tile_list, counter, Ct);
+    else if (!tA && tB) launch_q4_inst<BS, false, true>(A, B, ab, begin, n, tile_list, counter, Ct);
+    else if (tA && !tB) launch_q4_inst<BS, true, false>(A, B, ab, begin, n, tile_list, counter, Ct);
+    else launch_q4_inst<BS, true, true>(A, B, ab, begin, n, tile_list, counter, Ct);
 }
 
 }  // namespace
 
-bool launch_gemm_f32_tc(const Matrix& A, bool tA, const Matrix& B, bool tB, const uint2* ab, const uint64_t* begin,
+void launch_gemm_f32_tc(const Matrix& A, bool tA, const Matrix& B, bool tB, const uint2* ab, const uint64_t* begin,
                         uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, float* Ct, const uint64_t* ckeys,
-                        const uint32_t* task_k, size_t n_products) {
-    // 32- and 64-leaves: 2 x 2 groups of C tiles, over the whole task list or a tile list (HBSM_F32_MODE bit 128 / variant 3 keep
-    // the single-tile kernels)
-    const bool single_tile = (f32_mode() & (32 | 128)) != 0 || shared().gemm_variant.load() == 3;   // variant 3: parity hook of the tests
-    if (A.b == 32 && ckeys && task_k && !single_tile)
-        return launch_g32(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct);
-    if (A.b == 64 && ckeys && task_k && !single_tile)
-        return launch_g64(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct);
-    if (!(f32_mode() & 32)) {   // leaves of 32 / 64: stacked hi/lo operands, one MMA per K-step
-        if (A.b == 32) return launch_q4<32>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-        if (A.b == 64) return launch_q4<64>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    }
+                        const uint32_t* task_k, size_t n_products, bool single_tile) {
     switch (A.b) {
-        case 32: return (f32_mode() & 2) ? launch_bs<32, 32, 64>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct)
-                                          : launch_bs<32, 32, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-        case 64: return (f32_mode() & 2) ? launch_bs<64, 64, 64>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct)
-                                          : launch_bs<64, 64, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-        case 128: return launch_bs<128, 128, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-        case 256: return launch_bs<256, 128, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-        default: return false;
+        case 32:
+            if (single_tile) launch_q4<32>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+            else launch_g32(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct);
+            break;
+        case 64:
+            if (single_tile) launch_q4<64>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+            else launch_g64(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct);
+            break;
+        case 128: launch_bs<128, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct); break;
+        case 256: launch_bs<256, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct); break;
+        default: throw Error(HBSM_E_ARG, "hbsm_b200: no fp32 tensor-core leaf kernel for this blocksize");
     }
 }
 

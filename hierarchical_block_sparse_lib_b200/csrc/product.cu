@@ -4,8 +4,8 @@
 //   symbolic  get_batches_multiply H:5478 / get_batches_spamm H:6291  -> task-list builder (count, scan, fill, sort by
 //             (Morton key of the C tile, k), segment heads = C's block table)
 //   numeric   multiply_batches H:7240 (+ BLAS gemm H:7273)            -> one persistent grouped leaf-GEMM kernel,
-//             C-stationary (a CTA owns a C tile for its whole k-list, no atomics on data), A/B tiles staged by TMA bulk
-//             copies into padded shared memory behind an mbarrier ring, FP64 DMMA (mma.sync m8n8k4) accumulation.
+//             C-stationary (a CTA owns a C tile for its whole k-list, no atomics on data), A/B tiles staged by TMA tensor
+//             copies into shared memory behind an mbarrier ring, FP64 DMMA (mma.sync m8n8k4) accumulation.
 //
 // Executed set (SURVEY 0.3, 9): exact = every (ci,k,cj) with both tiles present; SpAMM additionally requires
 // fl(nsq(A_tile) * nsq(B_tile)) > fl(tau*tau) evaluated in Treal with a strict '>' (H:2008, H:6651).  The hierarchical
@@ -158,206 +158,7 @@ __global__ void __launch_bounds__(256) k_gemm_generic(const T* __restrict__ At, 
 }
 
 // ---------------------------------------------------------------------------------------------------
-// FP64 leaf GEMM: persistent, warp-specialised, TMA bulk copies + mbarrier ring + DMMA
-// ---------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
-
-// Shared-memory staging layout of one pipeline stage = one K-chunk (KC wide) of op(A) and of op(B).
-// Leaves are column-major with leading dimension BS (H:715), so a K-chunk is a set of contiguous "pieces":
-//   op(A) = A   : KC pieces (columns k) of BS doubles  -> smem [k][i], ld = BS + 4
-//   op(A) = A^T : BS pieces (columns i) of KC doubles  -> smem [i][k], ld = KC + 4
-//   op(B) = B   : BS pieces (columns n) of KC doubles  -> smem [n][k], ld = KC + 4
-//   op(B) = B^T : KC pieces (columns k) of BS doubles  -> smem [k][n], ld = BS + 4
-// ld == 4 (mod 16) doubles makes every DMMA fragment load (4 consecutive elements along one axis x 4 along the
-// other per half-warp) hit 16 distinct 8-byte banks: conflict-free for all four (tA,tB) without swizzling.
-template <int BS, int KC, bool TA, bool TB>
-struct GemmCfg {
-    static constexpr int LDA = TA ? KC + 4 : BS + 4;
-    static constexpr int A_PIECES = TA ? BS : KC;
-    static constexpr int A_PIECE_ELEMS = TA ? KC : BS;
-    static constexpr int A_ELEMS = A_PIECES * LDA;
-    static constexpr int LDB = TB ? BS + 4 : KC + 4;
-    static constexpr int B_PIECES = TB ? KC : BS;
-    static constexpr int B_PIECE_ELEMS = TB ? BS : KC;
-    static constexpr int B_ELEMS = B_PIECES * LDB;
-    static constexpr int STAGE_BYTES = (A_ELEMS + B_ELEMS) * 8;
-    static constexpr int TX_BYTES = 2 * BS * KC * 8;
-    static constexpr int NCHUNK = BS / KC;
-    static constexpr int SMEM_BUDGET = 220 * 1024;
-    static constexpr int NST_RAW = SMEM_BUDGET / STAGE_BYTES;
-    static constexpr int NST = NST_RAW > 8 ? 8 : NST_RAW;
-    static constexpr int CONSUMER_WARPS = 8;
-    static constexpr int THREADS = (CONSUMER_WARPS + 1) * 32;
-    static constexpr int WM = BS / 2, WN = BS / 4;   // warp grid 2 (rows) x 4 (cols)
-    static constexpr int MB = WM / 8, NB = WN / 8;
-    static constexpr int HEADER_BYTES = 1024;        // barriers + per-stage metadata
-    static constexpr int SMEM_BYTES = HEADER_BYTES + NST * STAGE_BYTES;
-    static_assert(NST >= 2, "pipeline needs two stages");
-    static_assert(BS % KC == 0 && KC % 16 == 0 && BS % 32 == 0, "tile shape");
-};
-
-
-template <int BS, int KC, bool TA, bool TB>
-__global__ void __launch_bounds__(GemmCfg<BS, KC, TA, TB>::THREADS, 1)
-k_gemm_f64(const double* __restrict__ At, const double* __restrict__ Bt, const uint2* __restrict__ ab,
-           const uint64_t* __restrict__ begin, uint32_t n_ctiles, const uint32_t* __restrict__ tile_list,
-           unsigned* __restrict__ next_tile, double* __restrict__ Ct) {
-    using Cfg = GemmCfg<BS, KC, TA, TB>;
-    constexpr int NST = Cfg::NST;
-    extern __shared__ __align__(128) unsigned char smem[];
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem);           // [NST]
-    uint64_t* empty_bar = full_bar + NST;                             // [NST]
-    GemmMeta* meta = reinterpret_cast<GemmMeta*>(empty_bar + NST);    // [NST]
-    unsigned char* stages = smem + Cfg::HEADER_BYTES;
-    const unsigned warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NST; ++s) {
-            mbar_init(smem_u32(&full_bar[s]), 1);
-            mbar_init(smem_u32(&empty_bar[s]), Cfg::CONSUMER_WARPS);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    constexpr size_t BB = (size_t)BS * BS;
-    if (warp == Cfg::CONSUMER_WARPS) {
-        // ===== producer warp: dynamic C-tile scheduler (Morton order => concurrently running CTAs share A rows /
-        // B columns in L2) + TMA bulk copies, running ahead of the consumers by up to NST chunks =====
-        uint32_t it = 0;
-        for (;;) {
-            unsigned tile = 0;
-            if (lane == 0) tile = atomicAdd(next_tile, 1u);
-            tile = __shfl_sync(0xffffffffu, tile, 0);
-            if (tile >= n_ctiles) break;
-            if (tile_list) tile = tile_list[tile];
-            const uint64_t p0 = begin[tile], p1 = begin[tile + 1];
-            for (uint64_t p = p0; p < p1; ++p) {
-                const uint2 t = ab[p];
-                const double* A = At + (size_t)t.x * BB;
-                const double* B = Bt + (size_t)t.y * BB;
-#pragma unroll 1
-                for (int ch = 0; ch < Cfg::NCHUNK; ++ch, ++it) {
-                    const uint32_t s = it % NST, ph = (it / NST) & 1u;
-                    mbar_wait(smem_u32(&empty_bar[s]), ph ^ 1u);
-                    const uint32_t fb = smem_u32(&full_bar[s]);
-                    if (lane == 0) {
-                        int fl = 0;
-                        if (p == p0 && ch == 0) fl |= 1;
-                        if (p + 1 == p1 && ch == Cfg::NCHUNK - 1) fl |= 2;
-                        meta[s].ctile = (int)tile;
-                        meta[s].flags = fl;
-                        mbar_arrive_expect_tx(fb, Cfg::TX_BYTES);
-                    }
-                    __syncwarp();
-                    const uint32_t sa = smem_u32(stages + (size_t)s * Cfg::STAGE_BYTES);
-                    const uint32_t sb = sa + Cfg::A_ELEMS * 8;
-                    const int k0 = ch * KC;
-                    for (int pc = lane; pc < Cfg::A_PIECES; pc += 32) {
-                        const double* src = TA ? A + (size_t)pc * BS + k0 : A + (size_t)(k0 + pc) * BS;
-                        tma_bulk_g2s(sa + pc * Cfg::LDA * 8, src, Cfg::A_PIECE_ELEMS * 8, fb);
-                    }
-                    for (int pc = lane; pc < Cfg::B_PIECES; pc += 32) {
-                        const double* src = TB ? B + (size_t)(k0 + pc) * BS : B + (size_t)pc * BS + k0;
-                        tma_bulk_g2s(sb + pc * Cfg::LDB * 8, src, Cfg::B_PIECE_ELEMS * 8, fb);
-                    }
-                }
-            }
-        }
-        // end-of-work marker
-        const uint32_t s = it % NST, ph = (it / NST) & 1u;
-        mbar_wait(smem_u32(&empty_bar[s]), ph ^ 1u);
-        if (lane == 0) {
-            meta[s].ctile = -1;
-            meta[s].flags = 4;
-            mbar_arrive(smem_u32(&full_bar[s]));
-        }
-        return;
-    }
-
-    // ===== consumer warps: 2 x 4 warp grid over the BS x BS C tile, accumulators in registers =====
-    const int wm0 = (int)(warp >> 2) * Cfg::WM, wn0 = (int)(warp & 3) * Cfg::WN;
-    const int g = (int)(lane >> 2), t = (int)(lane & 3);
-    double acc[Cfg::MB][Cfg::NB][2];
-    // per-thread element offsets of fragment (mb=0 / nb=0, ks=0) inside a stage
-    const int a_off = TA ? (wm0 + g) * Cfg::LDA + t : t * Cfg::LDA + (wm0 + g);
-    const int b_off = TB ? t * Cfg::LDB + (wn0 + g) : (wn0 + g) * Cfg::LDB + t;
-    constexpr int A_MB_STRIDE = TA ? 8 * Cfg::LDA : 8;          // +8 rows of op(A)
-    constexpr int A_KS_STRIDE = TA ? 4 : 4 * Cfg::LDA;          // +4 in k
-    constexpr int B_NB_STRIDE = TB ? 8 : 8 * Cfg::LDB;          // +8 columns of op(B)
-    constexpr int B_KS_STRIDE = TB ? 4 * Cfg::LDB : 4;
-    uint32_t it = 0;
-    for (;; ++it) {
-        const uint32_t s = it % NST, ph = (it / NST) & 1u;
-        mbar_wait(smem_u32(&full_bar[s]), ph);
-        const GemmMeta m = meta[s];
-        if (m.flags & 4) break;
-        if (m.flags & 1) {
-#pragma unroll
-            for (int i = 0; i < Cfg::MB; ++i)
-#pragma unroll
-                for (int j = 0; j < Cfg::NB; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-        }
-        const double* As = reinterpret_cast<const double*>(stages + (size_t)s * Cfg::STAGE_BYTES) + a_off;
-        const double* Bs = reinterpret_cast<const double*>(stages + (size_t)s * Cfg::STAGE_BYTES) + Cfg::A_ELEMS + b_off;
-#pragma unroll
-        for (int ks = 0; ks < KC / 4; ++ks) {
-            double a[Cfg::MB], b[Cfg::NB];
-#pragma unroll
-            for (int i = 0; i < Cfg::MB; ++i) a[i] = As[i * A_MB_STRIDE + ks * A_KS_STRIDE];
-#pragma unroll
-            for (int j = 0; j < Cfg::NB; ++j) b[j] = Bs[j * B_NB_STRIDE + ks * B_KS_STRIDE];
-#pragma unroll
-            for (int i = 0; i < Cfg::MB; ++i)
-#pragma unroll
-                for (int j = 0; j < Cfg::NB; ++j) dmma884(acc[i][j][0], acc[i][j][1], a[i], b[j]);
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(smem_u32(&empty_bar[s]));
-        if (m.flags & 2) {
-            double* C = Ct + (size_t)m.ctile * BB;
-#pragma unroll
-            for (int i = 0; i < Cfg::MB; ++i)
-#pragma unroll
-                for (int j = 0; j < Cfg::NB; ++j) {
-                    const int row = wm0 + i * 8 + g, col = wn0 + j * 8 + 2 * t;
-                    C[(size_t)col * BS + row] = acc[i][j][0];
-                    C[(size_t)(col + 1) * BS + row] = acc[i][j][1];
-                }
-        }
-    }
-}
-
-template <int BS, int KC, bool TA, bool TB>
-void launch_gemm_f64_inst(const double* At, const double* Bt, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
-                          const uint32_t* tile_list, unsigned* counter, double* Ct) {
-    using Cfg = GemmCfg<BS, KC, TA, TB>;
-    auto kfn = k_gemm_f64<BS, KC, TA, TB>;
-    static bool configured = false;
-    if (!configured) {
-        HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        configured = true;
-    }
-    unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, At, Bt, ab, begin, n_ctiles, tile_list, counter, Ct);
-}
-
-template <int BS, int KC>
-void launch_gemm_f64(bool tA, bool tB, const double* At, const double* Bt, const uint2* ab, const uint64_t* begin,
-                     uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, double* Ct) {
-    if (!tA && !tB) launch_gemm_f64_inst<BS, KC, false, false>(At, Bt, ab, begin, n_ctiles, tile_list, counter, Ct);
-    else if (!tA && tB) launch_gemm_f64_inst<BS, KC, false, true>(At, Bt, ab, begin, n_ctiles, tile_list, counter, Ct);
-    else if (tA && !tB) launch_gemm_f64_inst<BS, KC, true, false>(At, Bt, ab, begin, n_ctiles, tile_list, counter, Ct);
-    else launch_gemm_f64_inst<BS, KC, true, true>(At, Bt, ab, begin, n_ctiles, tile_list, counter, Ct);
-}
-
-
-// ---------------------------------------------------------------------------------------------------
-// FP64 leaf GEMM, TMA-tiled variant (the default): one cp.async.bulk.tensor per operand chunk.
+// FP64 leaf GEMM: persistent, warp-specialised, one cp.async.bulk.tensor per operand chunk + mbarrier ring + DMMA.
 //
 // A leaf (column-major, ld = BS) is described to TMA as the 4-D tensor  [tile][r/4][c][r%4]  (innermost last), i.e.
 //   dim0 = r % 4 (stride 8 B), dim1 = c (stride BS*8 B), dim2 = r / 4 (stride 32 B), dim3 = tile (stride BS*BS*8 B).
@@ -375,6 +176,12 @@ __device__ __forceinline__ void tma_tile_g2s(uint32_t dst, const CUtensorMap* ma
         "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
         ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar)
         : "memory");
+}
+
+__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
+    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
+                 : "+d"(c0), "+d"(c1)
+                 : "d"(a), "d"(b));
 }
 
 template <int BS, int KC>
@@ -541,27 +348,26 @@ k_gemm_f64_tma(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 }
 
 // tensor map of a tile pool in the interleaved-by-4-rows view; k_rows: the K-chunk runs along leaf rows
-bool make_tile_map(CUtensorMap* map, const void* tiles, size_t n_tiles, int LS, int BS, int KC, bool k_rows, int esize,
+void make_tile_map(CUtensorMap* map, const void* tiles, size_t n_tiles, int LS, int BS, int KC, bool k_rows, int esize,
                    CUtensorMapDataType dt) {
     EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc) return false;
     const int grp = 32 / esize;   // rows per 32-byte group (4 doubles / 8 floats)
     cuuint64_t gdim[4] = {(cuuint64_t)grp, (cuuint64_t)LS, (cuuint64_t)(LS / grp), (cuuint64_t)n_tiles};
     cuuint64_t gstr[3] = {(cuuint64_t)LS * esize, 32ull, (cuuint64_t)LS * LS * esize};
     cuuint32_t box[4] = {(cuuint32_t)grp, (cuuint32_t)(k_rows ? BS : KC), (cuuint32_t)(k_rows ? KC / grp : BS / grp), 1u};
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(map, dt, 4, const_cast<void*>(tiles), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS;
+    if (!enc || enc(map, dt, 4, const_cast<void*>(tiles), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        throw Error(HBSM_E_CUDA, "hbsm_b200: the driver refused the tensor map of an fp64 leaf operand");
 }
 
 template <int LS, int BS, int KC, bool TA, bool TB>
-bool launch_gemm_f64_tma_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
+void launch_gemm_f64_tma_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
                               const uint32_t* tile_list, unsigned* counter, double* Ct) {
     using Cfg = TmaCfg<BS, KC>;
     CUtensorMap mapA, mapB;
-    if (!make_tile_map(&mapA, A.tiles.p, A.L, LS, BS, KC, TA, 8, CU_TENSOR_MAP_DATA_TYPE_FLOAT64)) return false;
-    if (!make_tile_map(&mapB, B.tiles.p, B.n_ext(), LS, BS, KC, !TB, 8, CU_TENSOR_MAP_DATA_TYPE_FLOAT64)) return false;
+    make_tile_map(&mapA, A.tiles.p, A.L, LS, BS, KC, TA, 8, CU_TENSOR_MAP_DATA_TYPE_FLOAT64);
+    make_tile_map(&mapB, B.tiles.p, B.n_ext(), LS, BS, KC, !TB, 8, CU_TENSOR_MAP_DATA_TYPE_FLOAT64);
     auto kfn = k_gemm_f64_tma<LS, BS, KC, TA, TB>;
     static bool configured = false;
     if (!configured) {
@@ -569,19 +375,18 @@ bool launch_gemm_f64_tma_inst(const Matrix& A, const Matrix& B, const uint2* ab,
         configured = true;
     }
     const uint64_t units = (uint64_t)n_ctiles * (LS / BS) * (LS / BS);
-    if (units >= 0x7fffffffull) return false;
+    if (units >= 0x7fffffffull) throw Error(HBSM_E_CUDA, "hbsm_b200: too many C sub-tiles for one fp64 leaf-GEMM launch");
     unsigned grid = (unsigned)std::min<uint64_t>(units, (uint64_t)engine().sm_count);
     HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct);
-    return true;
 }
 
 template <int LS, int BS, int KC>
-bool launch_gemm_f64_tma(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin,
+void launch_gemm_f64_tma(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin,
                          uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, double* Ct) {
-    if (!tA && !tB) return launch_gemm_f64_tma_inst<LS, BS, KC, false, false>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    if (!tA && tB) return launch_gemm_f64_tma_inst<LS, BS, KC, false, true>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    if (tA && !tB) return launch_gemm_f64_tma_inst<LS, BS, KC, true, false>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    return launch_gemm_f64_tma_inst<LS, BS, KC, true, true>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+    if (!tA && !tB) launch_gemm_f64_tma_inst<LS, BS, KC, false, false>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+    else if (!tA && tB) launch_gemm_f64_tma_inst<LS, BS, KC, false, true>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+    else if (tA && !tB) launch_gemm_f64_tma_inst<LS, BS, KC, true, false>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+    else launch_gemm_f64_tma_inst<LS, BS, KC, true, true>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
 }
 
 struct TaskList {
@@ -741,45 +546,22 @@ __global__ void k_split_lists(const uint32_t* __restrict__ own_only, const uint6
     else later[i - pos[i]] = (uint32_t)i;
 }
 
-// one leaf-GEMM launch over `n` C tiles: all of them (tile_list == nullptr) or the listed subset
+// one leaf-GEMM launch over `n` C tiles: all of them (tile_list == nullptr) or the listed subset.
+// One kernel per (dtype, leaf size); hbsm_set_gemm_variant only swaps in the parity references of the tests:
+//   dtype, leaf                        kernel                                                last_gemm_kernel
+//   fp64, 32 / 64 / 128 / 256          k_gemm_f64_tma                                        1
+//   fp32, 32 / 64                      k_gemm_f32_g32 / _g64 (2 x 2 groups of C tiles);      3
+//                                      variant 3: k_gemm_f32_q4<32 / 64> (single C tiles)
+//   fp32, 128 / 256                    k_gemm_f32_tc                                         3
+//   any other leaf size, or variant 1  k_gemm_generic (plain FMA)                            0
 void launch_leaf_gemm(const Matrix& A, bool tA, const Matrix& B, bool tB, const TaskList& tl, const uint32_t* tile_list, size_t n,
                       char* ct) {
+    if (n == 0) return;
     Engine& e = engine();
     const int variant = shared().gemm_variant.load();
-    if (n == 0) return;
     const uint32_t nn = (uint32_t)n;
-    const bool fast64 = A.dtype == HBSM_F64 && variant != 1 && (A.b == 32 || A.b == 64 || A.b == 128 || A.b == 256);
-    if (fast64) {
-        DevBuf<unsigned> counter(1);
-        counter.zero();
-        const double* At = (const double*)A.tiles.p;
-        const double* Bt = (const double*)B.tiles.p;
-        bool done = false;
-        if (variant == 0 || A.b == 256) {   // TMA-tiled kernel; falls back to the bulk-copy kernel if the driver refuses the map
-            if (A.b == 64) done = launch_gemm_f64_tma<64, 64, 64>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            else if (A.b == 32) done = launch_gemm_f64_tma<32, 32, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            else if (A.b == 128) done = launch_gemm_f64_tma<128, 128, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            else done = launch_gemm_f64_tma<256, 128, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            e.last_gemm_kernel = done ? 1 : 2;
-        }
-        if (!done && A.b == 256) throw Error(HBSM_E_CUDA, "hbsm_b200: the driver refused the tensor map for 256-leaves");
-        if (!done) {
-            if (A.b == 64) launch_gemm_f64<64, 64>(tA, tB, At, Bt, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            else if (A.b == 32) launch_gemm_f64<32, 32>(tA, tB, At, Bt, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            else launch_gemm_f64<128, 32>(tA, tB, At, Bt, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (double*)ct);
-            e.last_gemm_kernel = 2;
-        }
-        return;   // `counter` is released in stream order
-    }
-    bool done = false;
-    if (A.dtype == HBSM_F32 && variant != 1) {   // fp32: split-TF32 on tcgen05 (gemm_f32.cu) for b in {32,64,128,256}
-        DevBuf<unsigned> counter(1);
-        counter.zero();
-        done = launch_gemm_f32_tc(A, tA, B, tB, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (float*)ct, tl.ckeys.p, tl.task_k.p,
-                                  tl.n_products);
-        if (done) e.last_gemm_kernel = 3;
-    }
-    if (!done) {
+    const bool tensor_leaf = A.b == 32 || A.b == 64 || A.b == 128 || A.b == 256;
+    if (variant == 1 || !tensor_leaf) {
         if (A.dtype == HBSM_F64) {
             auto kfn = k_gemm_generic<double>;
             HB_LAUNCH(kfn, nn, 256, 0, (const double*)A.tiles.p, (const double*)B.tiles.p, tl.ab.p, tl.begin.p, tile_list, A.b,
@@ -790,6 +572,23 @@ void launch_leaf_gemm(const Matrix& A, bool tA, const Matrix& B, bool tB, const 
                       tA ? 1 : 0, tB ? 1 : 0, (float*)ct);
         }
         e.last_gemm_kernel = 0;
+        return;
+    }
+    DevBuf<unsigned> counter(1);   // the persistent kernels' C-tile scheduler; released in stream order
+    counter.zero();
+    if (A.dtype == HBSM_F64) {
+        double* Ct = (double*)ct;
+        switch (A.b) {
+            case 32: launch_gemm_f64_tma<32, 32, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
+            case 64: launch_gemm_f64_tma<64, 64, 64>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
+            case 128: launch_gemm_f64_tma<128, 128, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
+            default: launch_gemm_f64_tma<256, 128, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
+        }
+        e.last_gemm_kernel = 1;
+    } else {   // split-TF32 on tcgen05 (gemm_f32.cu)
+        launch_gemm_f32_tc(A, tA, B, tB, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (float*)ct, tl.ckeys.p, tl.task_k.p,
+                           tl.n_products, variant == 3);
+        e.last_gemm_kernel = 3;
     }
 }
 

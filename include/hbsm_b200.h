@@ -47,7 +47,7 @@ typedef struct hbsm_stage_times_s {
     uint64_t n_products;  /* P: leaf products executed */
     uint64_t n_ctiles;    /* tiles of C */
     uint64_t gpu_launches;/* kernels launched by the call */
-    uint64_t gemm_kernel; /* leaf kernel used: 0 generic FMA, 1 TMA-tiled DMMA, 2 bulk-copy DMMA */
+    uint64_t gemm_kernel; /* leaf kernel used: 0 generic FMA, 1 fp64 TMA-tiled DMMA, 3 fp32 tcgen05 (2 is retired) */
 } hbsm_stage_times;
 
 /* ---- library ---- */
@@ -188,8 +188,9 @@ int hbsm_export_tile_tasks(hbsm_handle C, int bi, int bj, size_t cap, int64_t* k
 /* leaves in ascending Morton order; norms/tiles may be NULL; cap=0 -> count */
 int hbsm_export_leaves(hbsm_handle h, size_t cap, int64_t* bi, int64_t* bj, void* norms_cached, void* tiles, size_t* n);
 int hbsm_stage_times_last(hbsm_stage_times* out);
-int hbsm_set_gemm_variant(int variant);    /* 0 = auto (TMA-tiled DMMA / grouped tcgen05), 1 = generic FMA kernel (debug/parity), 2 = bulk-copy DMMA,
-                                            * 3 = fp32: single-C-tile tcgen05 kernels instead of the 2x2-group ones (parity) */
+int hbsm_set_gemm_variant(int variant);    /* 0 = auto (TMA-tiled DMMA / grouped tcgen05), 1 = generic FMA kernel (debug/parity),
+                                            * 3 = fp32: single-C-tile tcgen05 kernels instead of the 2x2-group ones (parity);
+                                            * any other value: HBSM_E_ARG */
 
 /* ---- device-side interface (multi-GPU plumbing, device-resident benchmarks) ---- */
 /* borrowed pointers into the matrix's device block table: valid until the matrix is modified */

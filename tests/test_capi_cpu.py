@@ -80,6 +80,19 @@ def test_handle_bookkeeping_without_device():
     assert (r.value, c.value) == (0b101, 0b011)
 
 
+def test_gemm_variant_accepts_only_the_existing_kernels():
+    """0 (tensor-core kernels), 1 (generic FMA) and 3 (fp32 single-C-tile) select leaf kernels; anything else is refused."""
+    L = _capi.lib()
+    try:
+        for v in (0, 1, 3):
+            assert L.hbsm_set_gemm_variant(v) == 0, v
+        for v in (2, 4, -1):
+            assert L.hbsm_set_gemm_variant(v) == _capi.HBSM_E_ARG, v
+            assert b"variant" in L.hbsm_last_error()
+    finally:
+        assert L.hbsm_set_gemm_variant(0) == 0
+
+
 @pytest.mark.skipif(have_gpu(), reason="a GPU is present: the loud-failure path cannot be exercised")
 def test_compute_fails_loudly_without_gpu():
     L = _capi.lib()
