@@ -13,6 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 
 HBSM_F64, HBSM_F32 = 0, 1
 HBSM_OK, HBSM_E_CUDA, HBSM_E_ARG, HBSM_E_RUNTIME = 0, 1, 2, 3
+HBSM_OP_N, HBSM_OP_T, HBSM_OP_SYM_UPPER = 0, 1, 2
 
 
 class StageTimes(C.Structure):
@@ -91,6 +92,10 @@ SIGNATURES = {
     "hbsm_symm_square": (_I, [_H, _H]),
     "hbsm_symm_rk": (_I, [_H, _I, _H]),
     "hbsm_symm_square_spamm": (_I, [_H, _H, C.c_double, C.POINTER(_sz), C.POINTER(_sz)]),
+    "hbsm_multiply_dense": (_I, [_H, _I, _I, _P, _I, _P, _I, C.c_double, C.c_double]),
+    "hbsm_multiply_dense_device": (_I, [_H, _I, _I, _P, _I, _P, _I, C.c_double, C.c_double, _P]),
+    "hbsm_spectral_norm": (_I, [_H, _I, _I, C.c_double, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double),
+                               C.POINTER(_I)]),
     "hbsm_export_tasks": (_I, [_H, _sz, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_export_leaves": (_I, [_H, _sz, _P, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_task_checksum": (_I, [_H, C.POINTER(C.c_uint64)]),

@@ -375,6 +375,39 @@ int hbsm_symm_square_spamm(hbsm_handle A, hbsm_handle C, double tau, size_t* n_b
     });
 }
 
+int hbsm_multiply_dense(hbsm_handle A, int op, int m, const void* X, int ldx, void* Y, int ldy, double alpha, double beta) {
+    return guarded([&] { dense_product_host(M(A), op, m, X, ldx, Y, ldy, alpha, beta); });
+}
+int hbsm_multiply_dense_device(hbsm_handle A, int op, int m, const void* d_X, int ldx, void* d_Y, int ldy, double alpha,
+                               double beta, void* cuda_stream) {
+    return guarded([&] {
+        Matrix& a = M(A);
+        validate_dense(a, op, m, ldx, ldy, d_X, d_Y);   // before either stream is touched
+        if (m == 0) return;
+        ensure_engine();
+        // the caller's stream -> engine stream -> the caller's stream, by events: no host synchronisation
+        static thread_local cudaEvent_t ev_in = nullptr, ev_out = nullptr;
+        if (!ev_in) HB_CUDA(cudaEventCreateWithFlags(&ev_in, cudaEventDisableTiming));
+        if (!ev_out) HB_CUDA(cudaEventCreateWithFlags(&ev_out, cudaEventDisableTiming));
+        const cudaStream_t s = (cudaStream_t)cuda_stream;
+        HB_CUDA(cudaEventRecord(ev_in, s));
+        HB_CUDA(cudaStreamWaitEvent(engine().stream, ev_in, 0));
+        dense_product_device(a, op, m, d_X, ldx, d_Y, ldy, alpha, beta);
+        HB_CUDA(cudaEventRecord(ev_out, engine().stream));
+        HB_CUDA(cudaStreamWaitEvent(s, ev_out, 0));
+    });
+}
+int hbsm_spectral_norm(hbsm_handle A, int symmetric_upper, int max_iter, double rel_tol, double* norm, double* lambda_min,
+                       double* lambda_max, int* n_iter) {
+    return guarded([&] {
+        const SpectralResult r = spectral_norm(M(A), symmetric_upper != 0, max_iter, rel_tol);
+        if (norm) *norm = r.norm;
+        if (lambda_min) *lambda_min = r.lambda_min;
+        if (lambda_max) *lambda_max = r.lambda_max;
+        if (n_iter) *n_iter = r.n_iter;
+    });
+}
+
 int hbsm_export_tasks(hbsm_handle Ch, size_t cap, int64_t* ci, int64_t* cj, int64_t* k, size_t* n) {
     return guarded([&] {
         Matrix& C = M(Ch);

@@ -173,6 +173,14 @@ struct DevBuf {
 
 inline void sync_stream() { HB_CUDA(cudaStreamSynchronize(engine().stream)); }
 
+// splitmix64: the hash of the seeded generators (generate_decay, generators.py), the task checksum and the Lanczos start vector
+__host__ __device__ inline uint64_t splitmix64(uint64_t x) {
+    x += 0x9E3779B97F4A7C15ull;
+    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+    return x ^ (x >> 31);
+}
+
 // ---- Morton keys: digit = 2*colbit + rowbit (H:52-56), most significant level first ----
 __host__ __device__ inline uint64_t spread_bits(uint32_t x) {
     uint64_t v = x;

@@ -744,12 +744,6 @@ __global__ void __launch_bounds__(256) k_mask_diag(const uint64_t* __restrict__ 
 }
 
 // ---- banded exponential-decay generator (SURVEY 8d): a_ij = (0.5 + 0.5 u(seed,i,j)) exp(-lambda |i-j|), |i-j| <= W ----
-__host__ __device__ inline uint64_t splitmix64(uint64_t x) {
-    x += 0x9E3779B97F4A7C15ull;
-    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-    return x ^ (x >> 31);
-}
 __host__ __device__ inline double hash_u01(uint64_t seed, uint64_t i, uint64_t j) {
     uint64_t h = splitmix64(seed ^ splitmix64(i * 0x100000001B3ull + splitmix64(j)));
     return (double)(h >> 11) * (1.0 / 9007199254740992.0);

@@ -161,6 +161,14 @@ void op_product_from_host(Matrix& A, const HostTiles& ha, bool tA, Matrix& B, co
                           size_t* n_mults, size_t* n_blocks);
 void op_product_abort();
 void product_row_counts(const Matrix& A, bool tA, const Matrix& B, bool tB, const ProductOpts& o, uint64_t* d_out);
+// ---- dense.cu: Y = alpha*op(A)*X + beta*Y with dense column-major X, Y in A's dtype (op: HBSM_OP_*), Lanczos on it ----
+void validate_dense(const Matrix& A, int op, int m, long long ldx, long long ldy, const void* X, const void* Y);   // HBSM_E_ARG
+void dense_product_device(const Matrix& A, int op, int m, const void* d_X, long long ldx, void* d_Y, long long ldy, double alpha,
+                          double beta);   // engine stream
+void dense_product_host(const Matrix& A, int op, int m, const void* X, long long ldx, void* Y, long long ldy, double alpha,
+                        double beta);     // synchronous
+struct SpectralResult { double norm, lambda_min, lambda_max; int n_iter; };
+SpectralResult spectral_norm(const Matrix& A, bool symmetric_upper, int max_iter, double rel_tol);
 // ---- sharded.cu: one process per GPU, NCCL resolved at run time ----
 void comm_set_library(const char* path);
 void comm_unique_id(void* out128);

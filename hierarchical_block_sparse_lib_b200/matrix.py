@@ -297,6 +297,89 @@ class HierarchicalBlockSparseMatrix:
         check(lib().hbsm_generate_decay(self._h, int(n), _ptr(table), int(W), int(seed), int(bool(symmetric)),
                                         int(row_tile_lo), int(row_tile_hi)))
 
+    # ---- engine extras: block-sparse times dense multivector, spectral estimates ----
+    def multiply_dense(self, X, op="N", alpha=1.0, beta=0.0, Y=None):
+        """Y = alpha * op(A) * X + beta * Y with op "N" (A), "T" (A^T) or "SYM_UPPER" (triu(A) + striu(A)^T); returns Y.
+
+        X and Y are 1-D or 2-D, column-major with unit stride along dim 0 (any column stride >= the row count: it becomes
+        the leading dimension).  numpy X of another layout or dtype is copied into a Fortran-ordered array; numpy Y must
+        already have that layout and A's dtype, as it is written in place.  torch CUDA tensors of A's dtype and that layout
+        run on the device, ordered on torch.cuda.current_stream(), without copies; other CUDA layouts are refused."""
+        ops = {"N": _capi.HBSM_OP_N, "T": _capi.HBSM_OP_T, "SYM_UPPER": _capi.HBSM_OP_SYM_UPPER}
+        if op not in ops:
+            raise ValueError("multiply_dense: op must be one of %s" % sorted(ops))
+        o = ops[op]
+        M = self.get_n_cols() if o == _capi.HBSM_OP_T else self.get_n_rows()
+        K = self.get_n_rows() if o == _capi.HBSM_OP_T else self.get_n_cols()
+        if type(X).__module__.startswith("torch") and X.is_cuda:
+            return self._multiply_dense_torch(o, M, K, X, float(alpha), float(beta), Y)
+        vec = np.ndim(X) == 1
+        X = np.asarray(X)
+        if not _column_major(X, self.dtype):
+            X = np.asfortranarray(X, dtype=self.dtype)
+        m = 1 if vec else X.shape[1]
+        if X.shape[0] != K:
+            raise ValueError("multiply_dense: X has %d rows, op(A) has %d columns" % (X.shape[0], K))
+        if Y is None:
+            Y = np.zeros(M if vec else (M, m), self.dtype, order="F")
+        elif not isinstance(Y, np.ndarray) or not _column_major(Y, self.dtype):
+            raise ValueError("multiply_dense: Y must be a %s array with unit stride along dim 0" % self.dtype)
+        if Y.shape[0] != M or (Y.shape[1] if Y.ndim == 2 else 1) != m:
+            raise ValueError("multiply_dense: Y has shape %s, expected (%d, %d)" % (Y.shape, M, m))
+        check(lib().hbsm_multiply_dense(self._h, o, m, _ptr(X), _ld(X, K), _ptr(Y), _ld(Y, M), float(alpha), float(beta)))
+        return Y
+
+    def _multiply_dense_torch(self, o, M, K, X, alpha, beta, Y):
+        import torch
+        tdt = {np.dtype(np.float64): torch.float64, np.dtype(np.float32): torch.float32}[self.dtype]
+
+        def ok(t):
+            return t.is_cuda and t.dtype == tdt and t.dim() in (1, 2) and (t.shape[0] <= 1 or t.stride(0) == 1)
+        if not ok(X):
+            raise ValueError("multiply_dense: a CUDA X must be a 1-D or 2-D %s tensor with unit stride along dim 0 (got %s, "
+                             "strides %s); it is never copied" % (tdt, X.dtype, tuple(X.stride())))
+        m = 1 if X.dim() == 1 else X.shape[1]
+        if X.shape[0] != K:
+            raise ValueError("multiply_dense: X has %d rows, op(A) has %d columns" % (X.shape[0], K))
+        if Y is None:
+            Y = torch.zeros(M, device=X.device, dtype=tdt) if X.dim() == 1 else \
+                torch.zeros((m, M), device=X.device, dtype=tdt).t()
+        elif not (type(Y).__module__.startswith("torch") and ok(Y)):
+            raise ValueError("multiply_dense: with a CUDA X, Y must be a CUDA %s tensor with unit stride along dim 0" % tdt)
+        if Y.shape[0] != M or (Y.shape[1] if Y.dim() == 2 else 1) != m:
+            raise ValueError("multiply_dense: Y has shape %s, expected (%d, %d)" % (tuple(Y.shape), M, m))
+        ldx = max(1, K) if X.dim() == 1 or m <= 1 else X.stride(1)
+        ldy = max(1, M) if Y.dim() == 1 or m <= 1 else Y.stride(1)
+        stream = torch.cuda.current_stream(X.device).cuda_stream
+        check(lib().hbsm_multiply_dense_device(self._h, o, m, C.c_void_p(X.data_ptr()), int(ldx), C.c_void_p(Y.data_ptr()),
+                                               int(ldy), alpha, beta, C.c_void_p(stream)))
+        return Y
+
+    def spectral_norm_estimate(self, symmetric_upper=False, max_iter=200, rel_tol=1e-8):
+        """||A||_2 by Lanczos, on A^T A or (symmetric_upper) on triu(A) + striu(A)^T.  Returns (norm, lambda_min,
+        lambda_max, n_iter): the extreme Ritz values of the operator Lanczos ran on -- the eigenvalue bounds of
+        triu(A) + striu(A)^T with symmetric_upper, those of A^T A (squared singular values) without, as in the C ABI."""
+        nrm = C.c_double(0); lo = C.c_double(0); hi = C.c_double(0); it = C.c_int(0)
+        check(lib().hbsm_spectral_norm(self._h, int(bool(symmetric_upper)), int(max_iter), float(rel_tol), C.byref(nrm),
+                                       C.byref(lo), C.byref(hi), C.byref(it)))
+        return nrm.value, lo.value, hi.value, it.value
+
+
+def _column_major(a, dtype):
+    """numpy array usable in place: the dtype, 1-D or 2-D, unit stride along dim 0, column stride a multiple of the item size."""
+    if a.dtype != dtype or a.ndim not in (1, 2):
+        return False
+    s = a.itemsize
+    if a.shape[0] > 1 and a.strides[0] != s:
+        return False
+    return a.ndim == 1 or a.shape[1] <= 1 or (a.strides[1] % s == 0 and a.strides[1] >= s * max(1, a.shape[0]))
+
+
+def _ld(a, rows):
+    if a.ndim == 1 or a.shape[1] <= 1:
+        return max(1, rows)
+    return a.strides[1] // a.itemsize
+
 
 def decay_table(lam, W):
     return np.ascontiguousarray(np.exp(-float(lam) * np.arange(W + 1, dtype=np.float64)))

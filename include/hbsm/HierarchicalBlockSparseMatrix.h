@@ -44,6 +44,7 @@ template <class Treal>
 class HierarchicalBlockSparseMatrix {
 public:
     typedef Treal real;   // H:40
+    typedef HierarchicalBlockSparseMatrix<Treal> Self;
 
     struct Params {       // H:167-169
         int blocksize;
@@ -197,6 +198,25 @@ public:
         if (no_of_resizes) *no_of_resizes = nr;
     }
     hbsm_handle handle() const { return h_; }
+    // Y = alpha * op(A) * X + beta * Y on host arrays (column-major, leading dimensions ldx / ldy); op is HBSM_OP_N,
+    // HBSM_OP_T or HBSM_OP_SYM_UPPER (triu(A) + striu(A)^T); leaf sizes up to 256.  The reference's get_row_sums / get_col_sums stubs below still
+    // throw; A*1 and A^T*1 are multiply_dense with X = ones.
+    static void multiply_dense(Self const& A, int op, int m, const Treal* X, int ldx, Treal* Y, int ldy, Treal alpha, Treal beta) {
+        detail::check(hbsm_multiply_dense(A.h_, op, m, X, ldx, Y, ldy, (double)alpha, (double)beta));
+    }
+    // ||A||_2 by Lanczos, on A^T A, or on triu(A) + striu(A)^T when symmetric_upper.  lambda_min / lambda_max receive the
+    // extreme Ritz values of that operator: the eigenvalue bounds of triu(A) + striu(A)^T, or those of A^T A (squared
+    // singular values) without symmetric_upper.  The reference's spectral_norm() stub below still throws.
+    Treal spectral_norm_estimate(bool symmetric_upper, int max_iter, Treal rel_tol, int* n_iter = NULL, Treal* lambda_min = NULL,
+                                 Treal* lambda_max = NULL) const {
+        double nrm = 0, lo = 0, hi = 0;
+        int it = 0;
+        detail::check(hbsm_spectral_norm(h_, symmetric_upper ? 1 : 0, max_iter, (double)rel_tol, &nrm, &lo, &hi, &it));
+        if (n_iter) *n_iter = it;
+        if (lambda_min) *lambda_min = (Treal)lo;
+        if (lambda_max) *lambda_max = (Treal)hi;
+        return (Treal)nrm;
+    }
     // ---- multi-GPU extras (not in the reference; one process per GPU, see hbsm::comm below and INTEGRATION.md) ----
     // Every rank holds matrices with the FULL logical dimensions but only the tiles of its slab of block rows (C row for
     // op(A), contraction index for op(B)) and receives the same slab of C.  publish() is the distributed half of
@@ -442,7 +462,6 @@ public:
 private:
     hbsm_handle h_;
 
-    typedef HierarchicalBlockSparseMatrix<Treal> Self;
     bool quadrant(int q, Self& out) const {
         int e = 0;
         out.set_params(get_params());

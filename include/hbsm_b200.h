@@ -176,6 +176,28 @@ int hbsm_symm_rk(hbsm_handle A, int transposed, hbsm_handle C);
 /* SpAMM-pruned symmetric square: triu(spamm(sym(A), sym(A), tau)) -- BASELINE config 3's tau sweep */
 int hbsm_symm_square_spamm(hbsm_handle A, hbsm_handle C, double tau, size_t* n_block_multiplies, size_t* n_resizes);
 
+/* ---- block-sparse times dense multivector and spectral estimates (engine extras; the reference's spectral_norm,
+ * get_row_sums, ... stubs are unchanged) ----
+ * Y = alpha * op(A) * X + beta * Y.  X (K x m) and Y (M x m), K x M the shape of op(A), are dense column-major arrays in A's
+ * dtype with leading dimensions ldx >= max(1, K), ldy >= max(1, M); rows of Y between M and ldy are never touched.
+ * op: HBSM_OP_N (A), HBSM_OP_T (A^T), HBSM_OP_SYM_UPPER (triu(A) + striu(A)^T of a square A: tiles below the diagonal and
+ * the strict lower part of diagonal tiles are ignored).  beta == 0 never reads Y.  Deterministic (bitwise repeatable).
+ * Only A's own tiles are used (a committed halo plays no part).  m == 0 is a no-op.  Leaf sizes up to 256 (any size, not
+ * only powers of two); a larger leaf size returns HBSM_E_ARG, from hbsm_spectral_norm too. */
+enum { HBSM_OP_N = 0, HBSM_OP_T = 1, HBSM_OP_SYM_UPPER = 2 };
+/* host arrays; staged with cudaMemcpyAsync, synchronous like the other host-pointer calls */
+int hbsm_multiply_dense(hbsm_handle A, int op, int m, const void* X, int ldx, void* Y, int ldy, double alpha, double beta);
+/* device arrays; ordered after the work already queued on cuda_stream (any stream, 0 included), and the work queued there
+ * afterwards sees Y complete; no host synchronisation */
+int hbsm_multiply_dense_device(hbsm_handle A, int op, int m, const void* d_X, int ldx, void* d_Y, int ldy,
+                               double alpha, double beta, void* cuda_stream);
+/* ||A||_2 by Lanczos: symmetric_upper = 0 -> on A^T A (one N and one T product per step), 1 -> on triu(A)+striu(A)^T
+ * (lambda_min / lambda_max may be NULL; they receive the extreme Ritz values of the operator: the eigenvalue bounds of
+ * triu(A)+striu(A)^T for 1, those of A^T A -- squared singular values -- for 0).  Stops when the residual bound of the extreme Ritz pair (for 1: of both extreme pairs) is <= rel_tol * the
+ * largest |Ritz value|, on breakdown, or after max_iter steps; *n_iter = steps used (0 for a matrix without tiles). */
+int hbsm_spectral_norm(hbsm_handle A, int symmetric_upper, int max_iter, double rel_tol,
+                       double* norm, double* lambda_min, double* lambda_max, int* n_iter);
+
 /* ---- parity / bench hooks ---- */
 /* executed products of the call that produced C, sorted by (Morton key of (ci,cj), k); cap=0 -> count */
 int hbsm_export_tasks(hbsm_handle C, size_t cap, int64_t* ci, int64_t* cj, int64_t* k, size_t* n);
