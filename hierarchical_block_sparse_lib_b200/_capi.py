@@ -26,6 +26,15 @@ class StageTimes(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class TruncInfo(C.Structure):
+    """hbsm_trunc_info"""
+    _fields_ = [("n_dropped", C.c_size_t), ("drop_nsq", C.c_double), ("n_frob", C.c_size_t), ("err_bound", C.c_double),
+                ("certified_by_lanczos", C.c_int), ("n_decisions", C.c_int), ("lanczos_steps", C.c_longlong)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 _H = C.c_void_p
 _sz = C.c_size_t
 _P = C.c_void_p
@@ -96,6 +105,8 @@ SIGNATURES = {
     "hbsm_multiply_dense_device": (_I, [_H, _I, _I, _P, _I, _P, _I, C.c_double, C.c_double, _P]),
     "hbsm_spectral_norm": (_I, [_H, _I, _I, C.c_double, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double),
                                C.POINTER(_I)]),
+    "hbsm_spectral_block_trunc": (_I, [_H, _I, C.c_double, _I, _H, C.POINTER(TruncInfo)]),
+    "hbsm_truncation_spectral_errors": (_I, [_H, _I, _sz, _P, _I, C.c_double, _P, _P]),
     "hbsm_export_tasks": (_I, [_H, _sz, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_export_leaves": (_I, [_H, _sz, _P, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_task_checksum": (_I, [_H, C.POINTER(C.c_uint64)]),

@@ -408,6 +408,26 @@ int hbsm_spectral_norm(hbsm_handle A, int symmetric_upper, int max_iter, double 
     });
 }
 
+int hbsm_spectral_block_trunc(hbsm_handle A, int symmetric_upper, double eps, int max_iter, hbsm_handle C, hbsm_trunc_info* info) {
+    return guarded([&] {
+        if (C == A) throw Error(HBSM_E_ARG, "hbsm_b200: spectral_block_trunc: target must not alias the source");
+        const TruncInfo t = spectral_block_trunc(M(A), symmetric_upper != 0, eps, max_iter, M(C));
+        if (info) {
+            info->n_dropped = t.n_dropped;
+            info->drop_nsq = t.drop_nsq;
+            info->n_frob = t.n_frob;
+            info->err_bound = t.err_bound;
+            info->certified_by_lanczos = t.certified_by_lanczos ? 1 : 0;
+            info->n_decisions = t.n_decisions;
+            info->lanczos_steps = t.lanczos_steps;
+        }
+    });
+}
+int hbsm_truncation_spectral_errors(hbsm_handle A, int symmetric_upper, size_t n, const double* taus, int max_iter, double rel_tol,
+                                    double* out_norms, int* out_iters) {
+    return guarded([&] { truncation_spectral_errors(M(A), symmetric_upper != 0, n, taus, max_iter, rel_tol, out_norms, out_iters); });
+}
+
 int hbsm_export_tasks(hbsm_handle Ch, size_t cap, int64_t* ci, int64_t* cj, int64_t* k, size_t* n) {
     return guarded([&] {
         Matrix& C = M(Ch);

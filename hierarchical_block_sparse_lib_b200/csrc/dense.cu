@@ -432,20 +432,24 @@ DenseOp dense_shape(const Matrix& A, int op) {
     return op == HBSM_OP_T ? DenseOp{A.N, A.M} : DenseOp{A.M, A.N};
 }
 
+LineView line_view(const LineIndex& ix) { return LineView{ix.ptr.p, ix.other.p, ix.tile.p}; }
+
+OpView view_for(const Matrix& A, int op) {   // A's own line indices that op walks
+    OpView v;
+    if (op != HBSM_OP_T) v.row = line_view(line_index(A, false));
+    if (op != HBSM_OP_N) v.col = line_view(line_index(A, true));
+    return v;
+}
+
 template <typename T, int MC>
-void launch_dense_mc(const Matrix& A, int op, int m, const T* X, long long ldx, T* Y, long long ldy, double alpha, double beta) {
+void launch_dense_mc(const Matrix& A, const OpView& v, int op, int m, const T* X, long long ldx, T* Y, long long ldy, double alpha,
+                     double beta) {
     Engine& e = engine();
     const DenseOp s = dense_shape(A, op);
     DenseArgs<T> g{};
     g.tiles = (const T*)A.tiles.p;
-    if (op != HBSM_OP_T) {
-        const LineIndex& ix = line_index(A, false);
-        g.rptr = ix.ptr.p; g.rother = ix.other.p; g.rtile = ix.tile.p;
-    }
-    if (op != HBSM_OP_N) {
-        const LineIndex& ix = line_index(A, true);
-        g.cptr = ix.ptr.p; g.cother = ix.other.p; g.ctile = ix.tile.p;
-    }
+    g.rptr = v.row.ptr; g.rother = v.row.other; g.rtile = v.row.tile;
+    g.cptr = v.col.ptr; g.cother = v.col.other; g.ctile = v.col.tile;
     g.X = X; g.Y = Y; g.ldx = ldx; g.ldy = ldy;
     g.b = A.b; g.Mop = s.Mop; g.K = s.K; g.m = m; g.op = op;
     g.n_brows = (s.Mop + A.b - 1) / A.b;
@@ -492,10 +496,33 @@ void launch_dense_mc(const Matrix& A, int op, int m, const T* X, long long ldx, 
 }
 
 template <typename T>
-void launch_dense(const Matrix& A, int op, int m, const T* X, long long ldx, T* Y, long long ldy, double alpha, double beta) {
-    if (m <= 8) launch_dense_mc<T, 8>(A, op, m, X, ldx, Y, ldy, alpha, beta);
-    else if (m <= 16) launch_dense_mc<T, 16>(A, op, m, X, ldx, Y, ldy, alpha, beta);
-    else launch_dense_mc<T, 32>(A, op, m, X, ldx, Y, ldy, alpha, beta);
+void launch_dense(const Matrix& A, const OpView& v, int op, int m, const T* X, long long ldx, T* Y, long long ldy, double alpha,
+                  double beta) {
+    if (m <= 8) launch_dense_mc<T, 8>(A, v, op, m, X, ldx, Y, ldy, alpha, beta);
+    else if (m <= 16) launch_dense_mc<T, 16>(A, v, op, m, X, ldx, Y, ldy, alpha, beta);
+    else launch_dense_mc<T, 32>(A, v, op, m, X, ldx, Y, ldy, alpha, beta);
+}
+
+// Decision tests of one Lanczos step (decision mode).  theta_lo / theta_hi: extreme Ritz values; r_lo / r_hi: the residual
+// bounds of their pairs (0 on breakdown: the Ritz values are exact).  For the symmetric operator the Ritz values lie inside
+// [lambda_min, lambda_max], so |theta| > eps proves ||op|| > eps.  Acceptance needs theta_hi + r_hi <= eps and
+// theta_lo - r_lo >= -eps with the extreme pairs converged (r <= conv * max|theta|): a residual bound only places an
+// eigenvalue near theta, and before the pair has converged a larger eigenvalue may not have entered the Krylov space yet.
+// For E^T E the same holds with eps^2 and theta_hi alone.  Returns true when decided.
+bool decide(LanczosDecision& d, bool symmetric_upper, double theta_lo, double theta_hi, double r_lo, double r_hi, double conv) {
+    const double scale = std::max(std::fabs(theta_lo), std::fabs(theta_hi));
+    if (symmetric_upper) {
+        const double up = std::max(theta_hi + r_hi, r_lo - theta_lo);
+        d.bound = up;
+        if (scale > d.eps) { d.feasible = false; return true; }
+        if (up <= d.eps && r_hi <= conv * scale && r_lo <= conv * scale) { d.feasible = true; return true; }
+    } else {
+        const double e2 = d.eps * d.eps;
+        d.bound = std::sqrt(std::max(theta_hi + r_hi, 0.0));
+        if (theta_hi > e2) { d.feasible = false; return true; }
+        if (theta_hi + r_hi <= e2 && r_hi <= conv * scale) { d.feasible = true; return true; }
+    }
+    return false;
 }
 
 }  // namespace
@@ -516,8 +543,9 @@ void dense_product_device(const Matrix& A, int op, int m, const void* d_X, long 
     const DenseOp s = dense_shape(A, op);
     if (m == 0 || s.Mop == 0) return;
     ensure_engine();
-    if (A.dtype == HBSM_F64) launch_dense<double>(A, op, m, (const double*)d_X, ldx, (double*)d_Y, ldy, alpha, beta);
-    else launch_dense<float>(A, op, m, (const float*)d_X, ldx, (float*)d_Y, ldy, alpha, beta);
+    const OpView v = view_for(A, op);
+    if (A.dtype == HBSM_F64) launch_dense<double>(A, v, op, m, (const double*)d_X, ldx, (double*)d_Y, ldy, alpha, beta);
+    else launch_dense<float>(A, v, op, m, (const float*)d_X, ldx, (float*)d_Y, ldy, alpha, beta);
 }
 
 void dense_product_host(const Matrix& A, int op, int m, const void* X, long long ldx, void* Y, long long ldy, double alpha,
@@ -552,6 +580,17 @@ SpectralResult spectral_norm(const Matrix& A, bool symmetric_upper, int max_iter
     SpectralResult res{};
     if (A.L == 0 || A.M == 0 || A.N == 0) return res;
     ensure_engine();
+    return lanczos(A, own_view(A), symmetric_upper, max_iter, rel_tol, nullptr);
+}
+
+OpView own_view(const Matrix& A) { return view_for(A, HBSM_OP_SYM_UPPER); }
+
+// The Lanczos core of spectral_norm on any operator view.  In decision mode (dec != nullptr) the run stops when decide()
+// settles ||op|| <= dec->eps (with the extreme pairs converged to rel_tol) or > dec->eps, on breakdown (decided with the exact
+// Ritz values), or at max_iter / the dimension, where an undecided run counts as infeasible.
+SpectralResult lanczos(const Matrix& A, const OpView& view, bool symmetric_upper, int max_iter, double rel_tol, LanczosDecision* dec) {
+    SpectralResult res{};
+    if (dec) { dec->feasible = false; dec->bound = 0.0; }
     const size_t n = (size_t)A.N, es = A.esize();
     DevBuf<char> V(n * es), P(n * es), W(n * es), tmp(symmetric_upper ? 1 : (size_t)A.M * es);
     DevBuf<double> part(LZ_BLOCKS), scal(2);
@@ -578,10 +617,10 @@ SpectralResult spectral_norm(const Matrix& A, bool symmetric_upper, int max_iter
         double beta_prev = 0.0, tnorm = 0.0;
         for (int j = 0;; ++j) {
             if (symmetric_upper) {
-                launch_dense<T>(A, HBSM_OP_SYM_UPPER, 1, (const T*)v, (long long)n, (T*)W.p, (long long)n, 1.0, 0.0);
+                launch_dense<T>(A, view, HBSM_OP_SYM_UPPER, 1, (const T*)v, (long long)n, (T*)W.p, (long long)n, 1.0, 0.0);
             } else {
-                launch_dense<T>(A, HBSM_OP_N, 1, (const T*)v, (long long)n, (T*)tmp.p, (long long)A.M, 1.0, 0.0);
-                launch_dense<T>(A, HBSM_OP_T, 1, (const T*)tmp.p, (long long)A.M, (T*)W.p, (long long)n, 1.0, 0.0);
+                launch_dense<T>(A, view, HBSM_OP_N, 1, (const T*)v, (long long)n, (T*)tmp.p, (long long)A.M, 1.0, 0.0);
+                launch_dense<T>(A, view, HBSM_OP_T, 1, (const T*)tmp.p, (long long)A.M, (T*)W.p, (long long)n, 1.0, 0.0);
             }
             dot(v, W.p, scal.p);
             HB_LAUNCH(k_lz_update<T>, grid, DN_THREADS, 0, (T*)W.p, (const T*)v, (const T*)vp, n, scal.p, beta_prev, part.p);
@@ -598,7 +637,9 @@ SpectralResult spectral_norm(const Matrix& A, bool symmetric_upper, int max_iter
             res.n_iter = j + 1;
             const bool converged = bound_hi <= rel_tol * scale && (!symmetric_upper || bound_lo <= rel_tol * scale);
             const bool breakdown = bj <= 16.0 * std::sqrt((double)n) * eps * tnorm;
-            if (converged || breakdown || res.n_iter >= max_iter || (size_t)res.n_iter >= n) {
+            const bool decided = dec && (breakdown ? decide(*dec, symmetric_upper, theta[0], theta[k - 1], 0.0, 0.0, rel_tol)
+                                                   : decide(*dec, symmetric_upper, theta[0], theta[k - 1], bound_lo, bound_hi, rel_tol));
+            if ((dec ? decided : converged) || breakdown || res.n_iter >= max_iter || (size_t)res.n_iter >= n) {
                 res.lambda_min = theta[0];
                 res.lambda_max = theta[k - 1];
                 break;

@@ -838,6 +838,10 @@ void dispatch(int dtype, F&& f) {
     else f((float)0);
 }
 
+int key_bits_for(const Matrix& A) { return std::max(1, 2 * A.vdepth()); }
+
+}  // namespace
+
 // compact helper: exclusive scan of flags -> positions, returns total (synchronises)
 size_t scan_flags(const DevBuf<uint32_t>& flags, size_t n, DevBuf<uint64_t>& pos) {
     pos.alloc(n + 1);
@@ -847,10 +851,6 @@ size_t scan_flags(const DevBuf<uint32_t>& flags, size_t n, DevBuf<uint64_t>& pos
     sync_stream();
     return (size_t)total;
 }
-
-int key_bits_for(const Matrix& A) { return std::max(1, 2 * A.vdepth()); }
-
-}  // namespace
 
 // ---------------------------------------------------------------------------------------------------
 // assembly
@@ -1386,8 +1386,7 @@ void op_copy(Matrix& C, const Matrix& A) {   // H:1490
     sync_stream();
 }
 
-bool op_trunc(const Matrix& A, Matrix& C, double trunc_value) {   // H:4935: C = copy of A without the small subtrees
-    if (&C == &A) throw Error(HBSM_E_ARG, "hbsm_b200: frob_block_trunc: target must not alias the source");
+bool trunc_begin(const Matrix& A, Matrix& C) {
     ensure_engine();
     C.clear();
     if (A.empty()) return false;    // copy of an empty matrix
@@ -1402,15 +1401,19 @@ bool op_trunc(const Matrix& A, Matrix& C, double trunc_value) {   // H:4935: C =
         sync_stream();
         return false;
     }
-    DevBuf<char> fresh(A.L * A.esize());
-    compute_leaf_norms(A, fresh.p);
-    DevBuf<uint32_t> keep(A.L);
+    return true;
+}
+
+void trunc_keep_flags(const Matrix& A, const void* d_nsq, double trunc_value, uint32_t* keep) {
     const float tf = (float)trunc_value;
-    HB_LAUNCH(k_trunc_flags, blocks_for(A.L, 256), 256, 0, (const void*)fresh.p, A.L, A.dtype == HBSM_F64 ? 1 : 0,
-              trunc_value * trunc_value, tf * tf, keep.p);
+    HB_LAUNCH(k_trunc_flags, blocks_for(A.L, 256), 256, 0, d_nsq, A.L, A.dtype == HBSM_F64 ? 1 : 0, trunc_value * trunc_value,
+              tf * tf, keep);
+}
+
+size_t trunc_compact(const Matrix& A, const DevBuf<uint32_t>& keep, Matrix& C) {
     DevBuf<uint64_t> pos;
     size_t nk = scan_flags(keep, A.L, pos);
-    if (nk == 0) return true;
+    if (nk == 0) return 0;
     DevBuf<uint64_t> okeys(nk);
     DevBuf<uint32_t> src(nk);
     HB_LAUNCH(k_compact_keys, blocks_for(A.L, 256), 256, 0, A.keys.p, A.L, keep.p, pos.p, okeys.p, src.p);
@@ -1422,7 +1425,17 @@ bool op_trunc(const Matrix& A, Matrix& C, double trunc_value) {   // H:4935: C =
     });
     C.set_table(std::move(okeys), std::move(t), nk);
     sync_stream();
-    return nk < A.L;
+    return nk;
+}
+
+bool op_trunc(const Matrix& A, Matrix& C, double trunc_value) {   // H:4935: C = copy of A without the small subtrees
+    if (&C == &A) throw Error(HBSM_E_ARG, "hbsm_b200: frob_block_trunc: target must not alias the source");
+    if (!trunc_begin(A, C)) return false;
+    DevBuf<char> fresh(A.L * A.esize());
+    compute_leaf_norms(A, fresh.p);
+    DevBuf<uint32_t> keep(A.L);
+    trunc_keep_flags(A, fresh.p, trunc_value, keep.p);
+    return trunc_compact(A, keep, C) < A.L;
 }
 
 bool op_extract_quadrant(const Matrix& A, int q, Matrix& C) {

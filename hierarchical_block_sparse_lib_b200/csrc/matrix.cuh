@@ -116,6 +116,15 @@ void op_upper(const Matrix& A, Matrix& C);
 void op_rescale(Matrix& C, const Matrix& A, double alpha);
 void op_copy(Matrix& C, const Matrix& A);
 bool op_trunc(const Matrix& A, Matrix& C, double trunc_value);   // frob_block_trunc, H:4935; true if something was removed
+// the pieces every truncation shares.  trunc_begin: C = A's shape, n_mults and stale root norm, without tiles; false when
+// nothing can be dropped (unsized, no tiles, or a single leaf, which is copied whole).  trunc_keep_flags: keep[t] = 0 iff
+// leaf t's ||.||_F^2 (d_nsq, Treal) < trunc_value^2 in Treal.  trunc_compact: C's tiles = A's tiles with keep[t] != 0, in
+// A's order, with zero (stale) cached norms; returns how many.  scan_flags: exclusive scan of n flags into pos[n + 1],
+// returns the total (synchronises).
+bool trunc_begin(const Matrix& A, Matrix& C);
+void trunc_keep_flags(const Matrix& A, const void* d_nsq, double trunc_value, uint32_t* keep);
+size_t trunc_compact(const Matrix& A, const DevBuf<uint32_t>& keep, Matrix& C);
+size_t scan_flags(const DevBuf<uint32_t>& flags, size_t n, DevBuf<uint64_t>& pos);
 bool op_extract_quadrant(const Matrix& A, int q, Matrix& C);        // false = absent; child q (0=TL 1=BL 2=TR 3=BR, H:52-56) as its own matrix
 void op_assemble_quadrants(Matrix& C, int M, int N, const Matrix* quads[4]);   // inverse; null / empty = absent child
 void op_leaf_inv_chol(const Matrix& A, Matrix& Z, int zdim, int valid);   // dense leaf step of inv_chol, H:3118-3147
@@ -169,6 +178,31 @@ void dense_product_host(const Matrix& A, int op, int m, const void* X, long long
                         double beta);     // synchronous
 struct SpectralResult { double norm, lambda_min, lambda_max; int n_iter; };
 SpectralResult spectral_norm(const Matrix& A, bool symmetric_upper, int max_iter, double rel_tol);
+// The operator the dense product walks: A's tiles through row and column line arrays (ptr[n_lines + 1], other, tile), each
+// line contiguous and ascending in `other` -- A's own line indices, or any subset of them (spectral_trunc.cu's masked index)
+struct LineView { const uint32_t *ptr = nullptr, *other = nullptr, *tile = nullptr; };
+struct OpView { LineView row, col; };
+OpView own_view(const Matrix& A);   // A's own row and column line indices (built if needed)
+// Decision mode of the Lanczos driver: stop as soon as ||op||_2 <= eps or > eps is decided (dense.cu, decide())
+struct LanczosDecision {
+    double eps;        // in
+    bool feasible;     // out: the operator's norm is <= eps (certified up to the Lanczos caveat), false when undecided
+    double bound;      // out: the upper estimate of the norm at the last step (theta + residual bound, in norm units)
+};
+// Lanczos on the operator of `view` (A's shape, dtype and leaf size); dec == nullptr: the full-convergence run of
+// spectral_norm (A validated and holding tiles); else decision mode, accepting only once the extreme pairs converged to rel_tol.
+SpectralResult lanczos(const Matrix& A, const OpView& view, bool symmetric_upper, int max_iter, double rel_tol, LanczosDecision* dec);
+// ---- spectral_trunc.cu: truncation with spectral-norm error control ----
+struct TruncInfo {
+    size_t n_dropped, n_frob;
+    double drop_nsq, err_bound;
+    bool certified_by_lanczos;
+    int n_decisions;
+    long long lanczos_steps;
+};
+TruncInfo spectral_block_trunc(const Matrix& A, bool symmetric_upper, double eps, int max_iter, Matrix& C);
+void truncation_spectral_errors(const Matrix& A, bool symmetric_upper, size_t n, const double* taus, int max_iter, double rel_tol,
+                                double* out_norms, int* out_iters);
 // ---- sharded.cu: one process per GPU, NCCL resolved at run time ----
 void comm_set_library(const char* path);
 void comm_unique_id(void* out128);

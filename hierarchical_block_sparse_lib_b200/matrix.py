@@ -364,6 +364,31 @@ class HierarchicalBlockSparseMatrix:
                                        C.byref(lo), C.byref(hi), C.byref(it)))
         return nrm.value, lo.value, hi.value, it.value
 
+    # ---- engine extras: truncation with spectral-norm error control ----
+    def spectral_block_trunc(self, matrix_truncated, eps, symmetric_upper=False, max_iter=100):
+        """matrix_truncated = self without the leaves of the largest nsq level v (leaf ||.||_F^2) whose error E_v -- the
+        dropped leaves, or triu(E_v) + striu(E_v)^T with symmetric_upper -- the search accepts with ||E_v||_2 <= eps.  The
+        result equals frob_block_trunc at any tau with v < tau^2 <= the next level.  Returns the hbsm_trunc_info as a dict:
+        n_dropped, drop_nsq (-1 when nothing is dropped), n_frob, err_bound, certified_by_lanczos, n_decisions,
+        lanczos_steps.  Acceptance beyond the Frobenius bound is a Lanczos estimate (see include/hbsm_b200.h)."""
+        info = _capi.TruncInfo()
+        check(lib().hbsm_spectral_block_trunc(self._h, int(bool(symmetric_upper)), float(eps), int(max_iter), matrix_truncated._h,
+                                              C.byref(info)))
+        d = info.as_dict()
+        d["certified_by_lanczos"] = bool(d["certified_by_lanczos"])
+        return d
+
+    def truncation_spectral_errors(self, taus, symmetric_upper=False, max_iter=200, rel_tol=1e-8):
+        """For each tau, the Lanczos estimate of ||E_tau||_2, E_tau = the leaves frob_block_trunc(tau) would drop (triu +
+        striu^T with symmetric_upper), exactly as spectral_norm_estimate reports it for a matrix of E_tau's tiles.  Returns
+        (norms float64, n_iter int32) numpy arrays."""
+        t = np.ascontiguousarray(np.atleast_1d(np.asarray(taus, np.float64)))
+        out = np.zeros(len(t), np.float64)
+        its = np.zeros(len(t), np.int32)
+        check(lib().hbsm_truncation_spectral_errors(self._h, int(bool(symmetric_upper)), len(t), _ptr(t), int(max_iter),
+                                                    float(rel_tol), _ptr(out), _ptr(its)))
+        return out, its
+
 
 def _column_major(a, dtype):
     """numpy array usable in place: the dtype, 1-D or 2-D, unit stride along dim 0, column stride a multiple of the item size."""

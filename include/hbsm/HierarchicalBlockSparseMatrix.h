@@ -217,6 +217,24 @@ public:
         if (lambda_max) *lambda_max = (Treal)hi;
         return (Treal)nrm;
     }
+    // C = *this without the leaves of the largest ||.||_F^2 level whose error matrix E (triu(E) + striu(E)^T when
+    // symmetric_upper) has ||E||_2 <= eps by the search of hbsm_spectral_block_trunc; info (may be NULL) receives its record.
+    // The reference's get_spectral_squared_of_error_matrix / spectral_norm stubs below still throw.
+    void spectral_block_trunc(HierarchicalBlockSparseMatrix<Treal>& C, Treal eps, bool symmetric_upper, int max_iter,
+                              hbsm_trunc_info* info = NULL) const {
+        hbsm_trunc_info t;
+        detail::check(hbsm_spectral_block_trunc(h_, symmetric_upper ? 1 : 0, (double)eps, max_iter, C.h_, &t));
+        if (info) *info = t;
+    }
+    // out[i] = Lanczos estimate of ||E_i||_2, E_i = the leaves frob_block_trunc(taus[i]) would drop (hbsm_truncation_spectral_errors)
+    void get_spectral_errors_of_truncation(std::vector<Treal>& out, std::vector<Treal> const& taus, bool symmetric_upper, int max_iter,
+                                           Treal rel_tol) const {
+        std::vector<double> t(taus.begin(), taus.end()), nrm(taus.size());
+        std::vector<int> it(taus.size());
+        detail::check(hbsm_truncation_spectral_errors(h_, symmetric_upper ? 1 : 0, t.size(), t.empty() ? NULL : &t[0], max_iter,
+                                                      (double)rel_tol, nrm.empty() ? NULL : &nrm[0], it.empty() ? NULL : &it[0]));
+        out.assign(nrm.begin(), nrm.end());
+    }
     // ---- multi-GPU extras (not in the reference; one process per GPU, see hbsm::comm below and INTEGRATION.md) ----
     // Every rank holds matrices with the FULL logical dimensions but only the tiles of its slab of block rows (C row for
     // op(A), contraction index for op(B)) and receives the same slab of C.  publish() is the distributed half of

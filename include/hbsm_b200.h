@@ -198,6 +198,43 @@ int hbsm_multiply_dense_device(hbsm_handle A, int op, int m, const void* d_X, in
 int hbsm_spectral_norm(hbsm_handle A, int symmetric_upper, int max_iter, double rel_tol,
                        double* norm, double* lambda_min, double* lambda_max, int* n_iter);
 
+/* ---- truncation with spectral-norm error control (engine extras; the reference's get_spectral_squared_of_error_matrix
+ * H:421 and spectral_norm H:427 stubs are unchanged) ----
+ * A truncation at level v drops exactly the leaves whose fresh ||.||_F^2 (nsq, hbsm_leaf_norms) is <= v; E_v is the dropped
+ * part.  The error operator is E_v, or triu(E_v) + striu(E_v)^T with symmetric_upper, where tiles below the diagonal play no
+ * part: they are never dropped and never counted.  A single leaf (depth 0) is never truncated, as in hbsm_frob_block_trunc.
+ *
+ * hbsm_spectral_block_trunc: C = A without the leaves of the largest level v the search accepts with ||E_v||_2 <= eps.
+ * C is exactly what hbsm_frob_block_trunc(A, C, tau) leaves for any tau with v < tau^2 <= the next distinct nsq (when A has
+ * no tiles below the diagonal, with symmetric_upper): the same tiles, n_mults and stale cached norms.  The search runs over
+ * the distinct levels between two rigorous brackets: the Frobenius bound (sum of nsq, of 2 nsq with symmetric_upper) <=
+ * eps^2 accepts without Lanczos; a leaf off the diagonal with nsq > b eps^2 can never be dropped.  Each level in between is
+ * decided by Lanczos on E_v, stopped as soon as it can decide: an extreme Ritz value above eps (eps^2 on E^T E) rejects,
+ * Ritz value + residual bound <= eps, once the extreme Ritz pairs have converged to a relative residual bound of 1e-3,
+ * accepts, breakdown decides with the exact Ritz values, and max_iter without a decision rejects.  Caveat: the accepting test
+ * is an estimate, not a proof -- an extreme eigenvector (nearly) orthogonal to the hashed start vector can escape the Krylov
+ * space, and then ||E_v||_2 may exceed eps.  Rejections are rigorous.
+ * HBSM_E_ARG (before any device work): eps < 0 or NaN, max_iter < 1, C == A, symmetric_upper with a non-square A, leaf size
+ * above 256.  Deterministic (bitwise repeatable). */
+typedef struct {
+    size_t n_dropped;          /* leaves dropped */
+    double drop_nsq;           /* the level v: the largest dropped nsq; -1 when nothing is dropped */
+    size_t n_frob;             /* leaves the Frobenius bound alone drops at eps */
+    double err_bound;          /* the certificate of the chosen level, in norm units: sqrt(Frobenius bound), or the Lanczos
+                                * upper estimate theta + residual bound */
+    int certified_by_lanczos;  /* 1: the chosen level lies above the Frobenius bracket and was accepted by Lanczos */
+    int n_decisions;           /* Lanczos decisions run */
+    long long lanczos_steps;   /* Lanczos steps over all decisions */
+} hbsm_trunc_info;
+int hbsm_spectral_block_trunc(hbsm_handle A, int symmetric_upper, double eps, int max_iter, hbsm_handle C, hbsm_trunc_info* info);
+/* out_norms[i] = ||E_i||_2 (triu + striu^T with symmetric_upper), E_i = the leaves hbsm_frob_block_trunc(A, C, taus[i])
+ * would drop (nsq < taus[i]^2 in A's dtype), estimated exactly as hbsm_spectral_norm(max_iter, rel_tol) would for a matrix
+ * holding only E_i's tiles (the same bits); out_iters[i] = its Lanczos steps (0 when E_i is empty).  HBSM_E_ARG (before any
+ * device work): max_iter < 1, rel_tol <= 0, symmetric_upper with a non-square A, leaf size above 256, n > 0 with a null
+ * taus / out_norms / out_iters. */
+int hbsm_truncation_spectral_errors(hbsm_handle A, int symmetric_upper, size_t n, const double* taus, int max_iter, double rel_tol,
+                                    double* out_norms, int* out_iters);
+
 /* ---- parity / bench hooks ---- */
 /* executed products of the call that produced C, sorted by (Morton key of (ci,cj), k); cap=0 -> count */
 int hbsm_export_tasks(hbsm_handle C, size_t cap, int64_t* ci, int64_t* cj, int64_t* k, size_t* n);
