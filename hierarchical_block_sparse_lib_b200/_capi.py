@@ -107,6 +107,7 @@ SIGNATURES = {
                                C.POINTER(_I)]),
     "hbsm_spectral_block_trunc": (_I, [_H, _I, C.c_double, _I, _H, C.POINTER(TruncInfo)]),
     "hbsm_truncation_spectral_errors": (_I, [_H, _I, _sz, _P, _I, C.c_double, _P, _P]),
+    "hbsm_multiply_accumulate": (_I, [_H, _I, _H, _I, _H, C.c_double, C.c_double, _I, C.c_double, _I, C.POINTER(_sz), C.POINTER(_sz)]),
     "hbsm_export_tasks": (_I, [_H, _sz, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_export_leaves": (_I, [_H, _sz, _P, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_task_checksum": (_I, [_H, C.POINTER(C.c_uint64)]),

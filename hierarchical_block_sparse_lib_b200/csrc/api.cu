@@ -191,6 +191,19 @@ int hbsm_spamm(hbsm_handle A, int tA, hbsm_handle B, int tB, hbsm_handle C, doub
         op_product(M(A), tA != 0, M(B), tB != 0, M(C), o, n_block_multiplies, n_resizes);
     });
 }
+int hbsm_multiply_accumulate(hbsm_handle A, int tA, hbsm_handle B, int tB, hbsm_handle C, double alpha, double beta,
+                             int spamm, double tau, int updated, size_t* n_block_multiplies, size_t* n_resizes) {
+    return guarded([&] {
+        ProductOpts o;
+        o.spamm = spamm != 0;
+        o.tau = tau;
+        o.updated = updated != 0;
+        o.c_old = &M(C);
+        o.alpha = alpha;
+        o.beta = beta;
+        op_product(M(A), tA != 0, M(B), tB != 0, M(C), o, n_block_multiplies, n_resizes);
+    });
+}
 int hbsm_product_begin_ex(hbsm_handle A, int tA, hbsm_handle B, int tB, hbsm_handle C, int spamm, double tau, int updated,
                           int defer_halo_tiles, int upper_only) {
     return guarded([&] {

@@ -181,6 +181,17 @@ __host__ __device__ inline uint64_t splitmix64(uint64_t x) {
     return x ^ (x >> 31);
 }
 
+// explicitly rounded fp arithmetic: never contracted into an FMA, so a sum of products has the bits of the separate operations
+template <typename T> struct DT;
+template <> struct DT<double> {
+    static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
+    static __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
+};
+template <> struct DT<float> {
+    static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
+    static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
+};
+
 // ---- Morton keys: digit = 2*colbit + rowbit (H:52-56), most significant level first ----
 __host__ __device__ inline uint64_t spread_bits(uint32_t x) {
     uint64_t v = x;

@@ -126,11 +126,12 @@ struct F32Header {
 // LS = leaf size (H:167 blocksize), BS = the square compute tile one CTA accumulates (BS == LS for 128-leaves; a
 // 256-leaf is processed as 2 x 2 C sub-tiles whose k-lists are the leaf's k-list with both 128-wide halves of each
 // operand: the tensor-map coordinates address the sub-blocks in place, ld = LS).
-template <int LS, int BS, bool TA, bool TB>
+template <int LS, int BS, bool TA, bool TB, bool ACC>
 __global__ void __launch_bounds__(F32Cfg<BS>::THREADS, 1)
 k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
               const uint2* __restrict__ ab, const uint64_t* __restrict__ begin, uint32_t n_ctiles,
-              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct) {
+              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct,
+              AccEpi<float> epi) {
     using Cfg = F32Cfg<BS>;
     constexpr int S = LS / BS;            // sub-tiles per leaf side
     static_assert(LS % BS == 0 && (S == 1 || S == 2), "leaf / compute-tile shapes");
@@ -342,8 +343,14 @@ k_gemm_f32_tc(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
             if (flags & 2) {
                 const unsigned tile = (unsigned)ctile / (S * S), sub = (unsigned)ctile % (S * S);
                 float* C = Ct + (size_t)tile * LS * LS + (size_t)((sub / S) * BS + h * CW) * LS + (sub % S) * BS + row;
+                if constexpr (ACC) {   // the old values in the store's own pattern
+                    const float* O = epi.old_at(tile, (size_t)LS * LS, (size_t)((sub / S) * BS + h * CW) * LS + (sub % S) * BS + row);
 #pragma unroll
-                for (int j = 0; j < CW; ++j) C[(size_t)j * LS] = acc[j];   // 32 lanes = 32 consecutive rows: 128 B per store
+                    for (int j = 0; j < CW; ++j) C[(size_t)j * LS] = epi.apply(acc[j], O, (size_t)j * LS);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < CW; ++j) C[(size_t)j * LS] = acc[j];   // 32 lanes = 32 consecutive rows: 128 B per store
+                }
             }
         }
     }
@@ -405,11 +412,12 @@ struct Q4Cfg {
     static constexpr int KSTEPS = KC / 8;
 };
 
-template <int BS, bool TA, bool TB>
+template <int BS, bool TA, bool TB, bool ACC>
 __global__ void __launch_bounds__(Q4Cfg<BS>::THREADS, 1)
 k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
               const uint2* __restrict__ ab, const uint64_t* __restrict__ begin, uint32_t n_ctiles,
-              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct) {
+              const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, float* __restrict__ Ct,
+              AccEpi<float> epi) {
     using Cfg = Q4Cfg<BS>;
     constexpr int NST = Cfg::NST, KC = Cfg::KC;
     extern __shared__ unsigned char smem_raw[];
@@ -637,8 +645,15 @@ k_gemm_f32_q4(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ 
                 asm volatile("bar.sync 1, %0;" ::"r"(Cfg::EPI_WARPS * 32) : "memory");
                 if (!lo_rows && crow < BS) {
                     float* C = Ct + (size_t)ctile * BS * BS + (size_t)(h * 32) * BS + crow;
+                    if constexpr (ACC) {
+                        const float* O = epi.old_at((size_t)ctile, (size_t)BS * BS, (size_t)(h * 32) * BS + crow);
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) C[(size_t)j * BS] = __fadd_rn(acc[j], my_stg[j * 32 + lane]);
+                        for (int j = 0; j < 32; ++j)
+                            C[(size_t)j * BS] = epi.apply(__fadd_rn(acc[j], my_stg[j * 32 + lane]), O, (size_t)j * BS);
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) C[(size_t)j * BS] = __fadd_rn(acc[j], my_stg[j * 32 + lane]);
+                    }
                 }
                 asm volatile("bar.sync 1, %0;" ::"r"(Cfg::EPI_WARPS * 32) : "memory");
             }
@@ -720,12 +735,12 @@ struct G32Header {
 };
 static_assert(sizeof(G32Header) <= G32Cfg::HEADER_BYTES, "header");
 
-template <bool TA, bool TB>
+template <bool TA, bool TB, bool ACC>
 __global__ void __launch_bounds__(G32Cfg::THREADS, 1)
 k_gemm_f32_g32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const __grid_constant__ CUtensorMap mapZ,
                const uint4* __restrict__ gops /* {A row 0, A row 1, B col 0, B col 1} tiles per super-product; P32_NONE = zero tile */,
                const uint64_t* __restrict__ gbegin, const int4* __restrict__ gtiles, const uint64_t* __restrict__ n_groups_dev,
-               unsigned* __restrict__ next_group, float* __restrict__ Ct) {
+               unsigned* __restrict__ next_group, float* __restrict__ Ct, AccEpi<float> epi) {
     using Cfg = G32Cfg;
     constexpr int NST = Cfg::NST, BS = Cfg::BS;
     extern __shared__ unsigned char smem_raw[];
@@ -914,8 +929,15 @@ k_gemm_f32_g32(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                 const int ctile = member == 0 ? tiles.x : (member == 1 ? tiles.y : (member == 2 ? tiles.z : tiles.w));
                 if (!lo_rows && ctile >= 0) {
                     float* C = Ct + (size_t)ctile * BS * BS + lane;
+                    if constexpr (ACC) {
+                        const float* O = epi.old_at((size_t)ctile, (size_t)BS * BS, lane);
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) C[(size_t)j * BS] = __fadd_rn(acc[j], my_stg[j * 32 + lane]);
+                        for (int j = 0; j < 32; ++j)
+                            C[(size_t)j * BS] = epi.apply(__fadd_rn(acc[j], my_stg[j * 32 + lane]), O, (size_t)j * BS);
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) C[(size_t)j * BS] = __fadd_rn(acc[j], my_stg[j * 32 + lane]);
+                    }
                 }
                 asm volatile("bar.sync 1, %0;" ::"r"(Cfg::EPI_WARPS * 32) : "memory");
             }
@@ -996,9 +1018,9 @@ __global__ void k_g32_merge(const uint64_t* __restrict__ ckeys, const uint32_t* 
     else gtiles[g] = make_int4(tile[0], tile[1], tile[2], tile[3]);
 }
 
-template <bool TA, bool TB>
+template <bool TA, bool TB, bool ACC>
 void launch_g32_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys, const uint32_t* task_k,
-                     const uint32_t* tile_list, uint32_t n_ctiles, size_t n_products, float* Ct) {
+                     const uint32_t* tile_list, uint32_t n_ctiles, size_t n_products, float* Ct, const AccEpi<float>& epi) {
     using Cfg = G32Cfg;
     CUtensorMap mapA, mapB, mapZ;
     make_f32_map(&mapA, A.tiles.p, A.L, 32, 32, 32, !TA);
@@ -1020,22 +1042,23 @@ void launch_g32_inst(const Matrix& A, const Matrix& B, const uint2* ab, const ui
               gops.p);
     DevBuf<unsigned> counter(1);
     counter.zero();
-    auto kfn = k_gemm_f32_g32<TA, TB>;
+    auto kfn = k_gemm_f32_g32<TA, TB, ACC>;
     static bool configured = false;
     if (!configured) {
         HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
     const unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, mapZ, gops.p, gbegin.p, gtiles.p, gpos.p + n_ctiles, counter.p, Ct);
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, mapZ, gops.p, gbegin.p, gtiles.p, gpos.p + n_ctiles, counter.p, Ct, epi);
 }
 
+template <bool ACC>
 void launch_g32(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys,
-                const uint32_t* task_k, const uint32_t* tile_list, uint32_t n, size_t n_products, float* Ct) {
-    if (!tA && !tB) launch_g32_inst<false, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    else if (!tA && tB) launch_g32_inst<false, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    else if (tA && !tB) launch_g32_inst<true, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    else launch_g32_inst<true, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+                const uint32_t* task_k, const uint32_t* tile_list, uint32_t n, size_t n_products, float* Ct, const AccEpi<float>& e) {
+    if (!tA && !tB) launch_g32_inst<false, false, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
+    else if (!tA && tB) launch_g32_inst<false, true, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
+    else if (tA && !tB) launch_g32_inst<true, false, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
+    else launch_g32_inst<true, true, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
 }
 
 
@@ -1075,12 +1098,12 @@ const float* zero_leaf_f32_64() {
     return z;
 }
 
-template <bool TA, bool TB>
+template <bool TA, bool TB, bool ACC>
 __global__ void __launch_bounds__(G64Cfg::THREADS, 1)
 k_gemm_f32_g64(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const __grid_constant__ CUtensorMap mapZa,
                const __grid_constant__ CUtensorMap mapZb, const uint4* __restrict__ gops, const uint64_t* __restrict__ gbegin,
                const int4* __restrict__ gtiles, const uint64_t* __restrict__ n_groups_dev, unsigned* __restrict__ next_group,
-               float* __restrict__ Ct) {
+               float* __restrict__ Ct, AccEpi<float> epi) {
     using Cfg = G64Cfg;
     constexpr int NST = Cfg::NST, BS = Cfg::BS, KC = Cfg::KC;
     extern __shared__ unsigned char smem_raw[];
@@ -1279,8 +1302,14 @@ k_gemm_f32_g64(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
                 const int ctile = member == 0 ? tiles.x : (member == 1 ? tiles.y : (member == 2 ? tiles.z : tiles.w));
                 if (ctile >= 0) {
                     float* C = Ct + (size_t)ctile * BS * BS + crow;
+                    if constexpr (ACC) {
+                        const float* O = epi.old_at((size_t)ctile, (size_t)BS * BS, crow);
 #pragma unroll
-                    for (int j = 0; j < 64; ++j) C[(size_t)j * BS] = acc[j];
+                        for (int j = 0; j < 64; ++j) C[(size_t)j * BS] = epi.apply(acc[j], O, (size_t)j * BS);
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < 64; ++j) C[(size_t)j * BS] = acc[j];
+                    }
                 }
             }
         }
@@ -1291,9 +1320,9 @@ k_gemm_f32_g64(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
     if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
 }
 
-template <bool TA, bool TB>
+template <bool TA, bool TB, bool ACC>
 void launch_g64_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys, const uint32_t* task_k,
-                     const uint32_t* tile_list, uint32_t n_ctiles, size_t n_products, float* Ct) {
+                     const uint32_t* tile_list, uint32_t n_ctiles, size_t n_products, float* Ct, const AccEpi<float>& epi) {
     using Cfg = G64Cfg;
     CUtensorMap mapA, mapB, mapZa, mapZb;
     // K-major operand (k along leaf rows): box {32 k, 64 mn};  MN-major: box {32 mn, 32 k}
@@ -1316,33 +1345,34 @@ void launch_g64_inst(const Matrix& A, const Matrix& B, const uint2* ab, const ui
               gops.p);
     DevBuf<unsigned> counter(1);
     counter.zero();
-    auto kfn = k_gemm_f32_g64<TA, TB>;
+    auto kfn = k_gemm_f32_g64<TA, TB, ACC>;
     static bool configured = false;
     if (!configured) {
         HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
     const unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, mapZa, mapZb, gops.p, gbegin.p, gtiles.p, gpos.p + n_ctiles, counter.p, Ct);
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, mapZa, mapZb, gops.p, gbegin.p, gtiles.p, gpos.p + n_ctiles, counter.p, Ct, epi);
 }
 
+template <bool ACC>
 void launch_g64(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, const uint64_t* ckeys,
-                const uint32_t* task_k, const uint32_t* tile_list, uint32_t n, size_t n_products, float* Ct) {
-    if (!tA && !tB) launch_g64_inst<false, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    else if (!tA && tB) launch_g64_inst<false, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    else if (tA && !tB) launch_g64_inst<true, false>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
-    else launch_g64_inst<true, true>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct);
+                const uint32_t* task_k, const uint32_t* tile_list, uint32_t n, size_t n_products, float* Ct, const AccEpi<float>& e) {
+    if (!tA && !tB) launch_g64_inst<false, false, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
+    else if (!tA && tB) launch_g64_inst<false, true, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
+    else if (tA && !tB) launch_g64_inst<true, false, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
+    else launch_g64_inst<true, true, ACC>(A, B, ab, begin, ckeys, task_k, tile_list, n, n_products, Ct, e);
 }
 
-template <int LS, int BS, bool TA, bool TB>
+template <int LS, int BS, bool TA, bool TB, bool ACC>
 void launch_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
-                 const uint32_t* tile_list, unsigned* counter, float* Ct) {
+                 const uint32_t* tile_list, unsigned* counter, float* Ct, const AccEpi<float>& epi) {
     using Cfg = F32Cfg<BS>;
     CUtensorMap mapA, mapB;
     // K-major operand (k along leaf rows): box {32 k, BS mn};  MN-major: box {32 mn, KC k}
     make_f32_map(&mapA, A.tiles.p, A.L, LS, 32, TA ? BS : Cfg::KC, !TA);
     make_f32_map(&mapB, B.tiles.p, B.n_ext(), LS, 32, TB ? Cfg::KC : BS, TB);
-    auto kfn = k_gemm_f32_tc<LS, BS, TA, TB>;
+    auto kfn = k_gemm_f32_tc<LS, BS, TA, TB, ACC>;
     static bool configured = false;
     if (!configured) {
         HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
@@ -1351,62 +1381,66 @@ void launch_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64
     const uint64_t units = (uint64_t)n_ctiles * (LS / BS) * (LS / BS);
     if (units >= 0x7fffffffull) throw Error(HBSM_E_CUDA, "hbsm_b200: too many C sub-tiles for one fp32 leaf-GEMM launch");
     unsigned grid = (unsigned)std::min<uint64_t>(units, (uint64_t)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct);
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct, epi);
 }
 
-template <int LS, int BS>
+template <int LS, int BS, bool ACC>
 void launch_bs(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n,
-               const uint32_t* tile_list, unsigned* counter, float* Ct) {
-    if (!tA && !tB) launch_inst<LS, BS, false, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    else if (!tA && tB) launch_inst<LS, BS, false, true>(A, B, ab, begin, n, tile_list, counter, Ct);
-    else if (tA && !tB) launch_inst<LS, BS, true, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    else launch_inst<LS, BS, true, true>(A, B, ab, begin, n, tile_list, counter, Ct);
+               const uint32_t* tile_list, unsigned* counter, float* Ct, const AccEpi<float>& e) {
+    if (!tA && !tB) launch_inst<LS, BS, false, false, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
+    else if (!tA && tB) launch_inst<LS, BS, false, true, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
+    else if (tA && !tB) launch_inst<LS, BS, true, false, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
+    else launch_inst<LS, BS, true, true, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
 }
 
-template <int BS, bool TA, bool TB>
+template <int BS, bool TA, bool TB, bool ACC>
 void launch_q4_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
-                    const uint32_t* tile_list, unsigned* counter, float* Ct) {
+                    const uint32_t* tile_list, unsigned* counter, float* Ct, const AccEpi<float>& epi) {
     using Cfg = Q4Cfg<BS>;
     CUtensorMap mapA, mapB;
     make_f32_map(&mapA, A.tiles.p, A.L, BS, 32, BS, !TA);
     make_f32_map(&mapB, B.tiles.p, B.n_ext(), BS, 32, BS, TB);
-    auto kfn = k_gemm_f32_q4<BS, TA, TB>;
+    auto kfn = k_gemm_f32_q4<BS, TA, TB, ACC>;
     static bool configured = false;
     if (!configured) {
         HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         configured = true;
     }
     unsigned grid = std::min<unsigned>(n_ctiles, (unsigned)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct);
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct, epi);
 }
 
-template <int BS>
+template <int BS, bool ACC>
 void launch_q4(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n,
-               const uint32_t* tile_list, unsigned* counter, float* Ct) {
-    if (!tA && !tB) launch_q4_inst<BS, false, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    else if (!tA && tB) launch_q4_inst<BS, false, true>(A, B, ab, begin, n, tile_list, counter, Ct);
-    else if (tA && !tB) launch_q4_inst<BS, true, false>(A, B, ab, begin, n, tile_list, counter, Ct);
-    else launch_q4_inst<BS, true, true>(A, B, ab, begin, n, tile_list, counter, Ct);
+               const uint32_t* tile_list, unsigned* counter, float* Ct, const AccEpi<float>& e) {
+    if (!tA && !tB) launch_q4_inst<BS, false, false, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
+    else if (!tA && tB) launch_q4_inst<BS, false, true, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
+    else if (tA && !tB) launch_q4_inst<BS, true, false, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
+    else launch_q4_inst<BS, true, true, ACC>(A, B, ab, begin, n, tile_list, counter, Ct, e);
 }
 
 }  // namespace
 
 void launch_gemm_f32_tc(const Matrix& A, bool tA, const Matrix& B, bool tB, const uint2* ab, const uint64_t* begin,
                         uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, float* Ct, const uint64_t* ckeys,
-                        const uint32_t* task_k, size_t n_products, bool single_tile) {
-    switch (A.b) {
-        case 32:
-            if (single_tile) launch_q4<32>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-            else launch_g32(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct);
-            break;
-        case 64:
-            if (single_tile) launch_q4<64>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-            else launch_g64(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct);
-            break;
-        case 128: launch_bs<128, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct); break;
-        case 256: launch_bs<256, 128>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct); break;
-        default: throw Error(HBSM_E_ARG, "hbsm_b200: no fp32 tensor-core leaf kernel for this blocksize");
-    }
+                        const uint32_t* task_k, size_t n_products, bool single_tile, const AccArgs* acc) {
+    const AccEpi<float> e = acc ? acc->epi<float>() : AccArgs().epi<float>();
+    with_acc(acc, [&](auto on) {
+        constexpr bool ACC = decltype(on)::value;
+        switch (A.b) {
+            case 32:
+                if (single_tile) launch_q4<32, ACC>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e);
+                else launch_g32<ACC>(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct, e);
+                break;
+            case 64:
+                if (single_tile) launch_q4<64, ACC>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e);
+                else launch_g64<ACC>(tA, tB, A, B, ab, begin, ckeys, task_k, tile_list, n_ctiles, n_products, Ct, e);
+                break;
+            case 128: launch_bs<128, 128, ACC>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e); break;
+            case 256: launch_bs<256, 128, ACC>(tA, tB, A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e); break;
+            default: throw Error(HBSM_E_ARG, "hbsm_b200: no fp32 tensor-core leaf kernel for this blocksize");
+        }
+    });
 }
 
 }  // namespace hbsm_b200

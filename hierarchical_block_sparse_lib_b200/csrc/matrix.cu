@@ -141,16 +141,6 @@ void commit_halo(Matrix& A, size_t n_halo) {
 
 namespace {
 
-template <typename T> struct DT;
-template <> struct DT<double> {
-    static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
-    static __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
-};
-template <> struct DT<float> {
-    static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
-    static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
-};
-
 inline unsigned blocks_for(size_t n, unsigned threads) { return (unsigned)((n + threads - 1) / threads); }
 
 // lower_bound over sorted keys; returns index or -1 if absent
@@ -669,17 +659,19 @@ __global__ void k_compact_keys(const uint64_t* __restrict__ keys, size_t n, cons
     okeys[pos[i]] = keys[i];
     src[pos[i]] = (uint32_t)i;
 }
-// copy tile src[t] -> t; mode 0 plain copy * alpha (alpha_on), mode 1: diagonal tiles keep only row <= col
+// copy tile src[o] -> o for o = dst[t] (dst == nullptr: o = t); mode 0 plain copy * alpha (alpha_on), mode 1: diagonal
+// tiles keep only row <= col
 template <typename T>
 __global__ void __launch_bounds__(256) k_copy_tiles(const T* __restrict__ tin, const uint32_t* __restrict__ src,
                                                      const uint64_t* __restrict__ okeys, int b, int mask_diag,
-                                                     int scale, T alpha, T* __restrict__ tout) {
+                                                     int scale, T alpha, T* __restrict__ tout, const uint32_t* __restrict__ dst) {
     const size_t bb = (size_t)b * b;
-    const size_t si = src ? (size_t)src[blockIdx.x] : (size_t)blockIdx.x;
+    const size_t o = dst ? (size_t)dst[blockIdx.x] : (size_t)blockIdx.x;
+    const size_t si = src ? (size_t)src[o] : o;
     const T* in = tin + si * bb;
-    T* out = tout + (size_t)blockIdx.x * bb;
+    T* out = tout + o * bb;
     bool diag = false;
-    if (mask_diag) { uint64_t k = okeys[blockIdx.x]; diag = morton_row(k) == morton_col(k); }
+    if (mask_diag) { uint64_t k = okeys[o]; diag = morton_row(k) == morton_col(k); }
     for (size_t i = (size_t)blockIdx.y * blockDim.x + threadIdx.x; i < bb; i += (size_t)gridDim.y * blockDim.x) {
         T v = in[i];
         if (diag && (int)(i % b) > (int)(i / b)) v = (T)0;
@@ -959,7 +951,7 @@ void assign_tiles_device(Matrix& A, size_t n_tiles, const uint64_t* d_keys, cons
     dispatch(A.dtype, [&](auto z) {
         using T = decltype(z);
         dim3 grid((unsigned)n_tiles, (unsigned)std::max<size_t>(1, std::min<size_t>(8, A.tile_elems() / 1024)));
-        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)d_tiles, idx.p, skeys.p, A.b, 0, 0, (T)1, (T*)t.p);
+        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)d_tiles, idx.p, skeys.p, A.b, 0, 0, (T)1, (T*)t.p, (const uint32_t*)nullptr);
     });
     A.set_table(std::move(skeys), std::move(t), n_tiles);
     if (d_norms) {
@@ -967,7 +959,7 @@ void assign_tiles_device(Matrix& A, size_t n_tiles, const uint64_t* d_keys, cons
         dispatch(A.dtype, [&](auto z) {
             using T = decltype(z);
             HB_LAUNCH(k_copy_tiles<T>, dim3((unsigned)n_tiles, 1), 32, 0, (const T*)d_norms, idx.p, A.keys.p, 1, 0, 0, (T)1,
-                      (T*)A.norms.p);
+                      (T*)A.norms.p, (const uint32_t*)nullptr);
         });
     }
     sync_stream();
@@ -1259,6 +1251,36 @@ static unsigned slices_for(const Matrix& A) {
     return (unsigned)std::max<size_t>(1, std::min<size_t>(8, A.tile_elems() * A.esize() / 8192));
 }
 
+size_t key_union(const uint64_t* ka, size_t na, const uint64_t* kb, size_t nb, DevBuf<uint64_t>& ukeys, DevBuf<uint32_t>& src_a,
+                 DevBuf<uint32_t>& src_b) {
+    DevBuf<uint32_t> keep_b(std::max<size_t>(nb, 1));
+    DevBuf<uint64_t> bpre;
+    size_t n_bonly = 0;
+    if (nb) {
+        HB_LAUNCH(k_union_mark, blocks_for(nb, 256), 256, 0, ka, na, kb, nb, keep_b.p);
+        n_bonly = scan_flags(keep_b, nb, bpre);
+    } else {
+        bpre.alloc(1);
+        bpre.zero();
+    }
+    const size_t nu = na + n_bonly;
+    ukeys.alloc(nu);
+    src_a.alloc(nu);
+    src_b.alloc(nu);
+    if (na) HB_LAUNCH(k_union_pos_a, blocks_for(na, 256), 256, 0, ka, na, kb, nb, bpre.p, ukeys.p, src_a.p, src_b.p);
+    if (nb) HB_LAUNCH(k_union_pos_b, blocks_for(nb, 256), 256, 0, ka, na, kb, nb, keep_b.p, bpre.p, ukeys.p, src_a.p, src_b.p);
+    return nu;
+}
+
+void scale_tiles_into(const Matrix& X, const uint32_t* src, const uint32_t* dst, size_t n, double alpha, void* tout) {
+    if (n == 0) return;
+    dispatch(X.dtype, [&](auto z) {
+        using T = decltype(z);
+        dim3 grid((unsigned)n, slices_for(X));
+        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)X.tiles.p, src, (const uint64_t*)nullptr, X.b, 0, 1, (T)alpha, (T*)tout, dst);
+    });
+}
+
 void op_add(const Matrix& A, const Matrix& B, Matrix& C) {   // H:1644
     C.clear();
     if (A.empty() && B.empty()) return;
@@ -1272,21 +1294,9 @@ void op_add(const Matrix& A, const Matrix& B, Matrix& C) {   // H:1644
     C.n_mults = A.n_mults + B.n_mults;   // H:1719
     const size_t na = A.L, nb = B.L;
     if (na + nb == 0) return;
-    DevBuf<uint32_t> keep_b(std::max<size_t>(nb, 1));
-    DevBuf<uint64_t> bpre;
-    size_t n_bonly = 0;
-    if (nb) {
-        HB_LAUNCH(k_union_mark, blocks_for(nb, 256), 256, 0, A.keys.p, na, B.keys.p, nb, keep_b.p);
-        n_bonly = scan_flags(keep_b, nb, bpre);
-    } else {
-        bpre.alloc(1);
-        bpre.zero();
-    }
-    const size_t nu = na + n_bonly;
-    DevBuf<uint64_t> ukeys(nu);
-    DevBuf<uint32_t> src_a(nu), src_b(nu);
-    if (na) HB_LAUNCH(k_union_pos_a, blocks_for(na, 256), 256, 0, A.keys.p, na, B.keys.p, nb, bpre.p, ukeys.p, src_a.p, src_b.p);
-    if (nb) HB_LAUNCH(k_union_pos_b, blocks_for(nb, 256), 256, 0, A.keys.p, na, B.keys.p, nb, keep_b.p, bpre.p, ukeys.p, src_a.p, src_b.p);
+    DevBuf<uint64_t> ukeys;
+    DevBuf<uint32_t> src_a, src_b;
+    const size_t nu = key_union(A.keys.p, na, B.keys.p, nb, ukeys, src_a, src_b);
     DevBuf<char> t(nu * C.tile_bytes());
     dispatch(C.dtype, [&](auto z) {
         using T = decltype(z);
@@ -1341,7 +1351,7 @@ void op_upper(const Matrix& A, Matrix& C) {   // H:3515
     dispatch(A.dtype, [&](auto z) {
         using T = decltype(z);
         dim3 grid((unsigned)nk, slices_for(A));
-        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)A.tiles.p, src.p, okeys.p, A.b, 1, 0, (T)1, (T*)t.p);
+        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)A.tiles.p, src.p, okeys.p, A.b, 1, 0, (T)1, (T*)t.p, (const uint32_t*)nullptr);
     });
     C.set_table(std::move(okeys), std::move(t), nk);
     sync_stream();
@@ -1361,7 +1371,7 @@ void op_rescale(Matrix& C, const Matrix& A, double alpha) {   // H:3078
     dispatch(A.dtype, [&](auto z) {
         using T = decltype(z);
         dim3 grid((unsigned)A.L, slices_for(A));
-        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)A.tiles.p, (const uint32_t*)nullptr, okeys.p, A.b, 0, 1, (T)alpha, (T*)t.p);
+        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)A.tiles.p, (const uint32_t*)nullptr, okeys.p, A.b, 0, 1, (T)alpha, (T*)t.p, (const uint32_t*)nullptr);
     });
     C.set_table(std::move(okeys), std::move(t), A.L);
     sync_stream();
@@ -1421,7 +1431,7 @@ size_t trunc_compact(const Matrix& A, const DevBuf<uint32_t>& keep, Matrix& C) {
     dispatch(A.dtype, [&](auto z) {
         using T = decltype(z);
         dim3 grid((unsigned)nk, slices_for(A));
-        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)A.tiles.p, src.p, okeys.p, A.b, 0, 0, (T)1, (T*)t.p);
+        HB_LAUNCH(k_copy_tiles<T>, grid, 256, 0, (const T*)A.tiles.p, src.p, okeys.p, A.b, 0, 0, (T)1, (T*)t.p, (const uint32_t*)nullptr);
     });
     C.set_table(std::move(okeys), std::move(t), nk);
     sync_stream();

@@ -125,6 +125,12 @@ bool trunc_begin(const Matrix& A, Matrix& C);
 void trunc_keep_flags(const Matrix& A, const void* d_nsq, double trunc_value, uint32_t* keep);
 size_t trunc_compact(const Matrix& A, const DevBuf<uint32_t>& keep, Matrix& C);
 size_t scan_flags(const DevBuf<uint32_t>& flags, size_t n, DevBuf<uint64_t>& pos);
+// merge-union of two ascending key lists (op_add's): ukeys ascending, src_a[u] / src_b[u] = the index of ukeys[u] in ka / kb, or
+// 0xffffffff where absent; returns the union's size (synchronises)
+size_t key_union(const uint64_t* ka, size_t na, const uint64_t* kb, size_t nb, DevBuf<uint64_t>& ukeys, DevBuf<uint32_t>& src_a,
+                 DevBuf<uint32_t>& src_b);
+// for t < n: tile o = dst[t] of tout = fl(alpha * tile src[o] of X), alpha rounded to X's dtype first (op_rescale's arithmetic)
+void scale_tiles_into(const Matrix& X, const uint32_t* src, const uint32_t* dst, size_t n, double alpha, void* tout);
 bool op_extract_quadrant(const Matrix& A, int q, Matrix& C);        // false = absent; child q (0=TL 1=BL 2=TR 3=BR, H:52-56) as its own matrix
 void op_assemble_quadrants(Matrix& C, int M, int N, const Matrix* quads[4]);   // inverse; null / empty = absent child
 void op_leaf_inv_chol(const Matrix& A, Matrix& Z, int zdim, int valid);   // dense leaf step of inv_chol, H:3118-3147
@@ -148,6 +154,10 @@ struct ProductOpts {
     double tau = 0.0;
     bool updated = true;
     bool upper_only = false;   // keep only C tiles with ci <= cj (symm_square / symm_rk)
+    // accumulating product (hbsm_multiply_accumulate): C <- alpha*P + beta*C_old, where C_old is c_old's table when the product
+    // begins (c_old is C itself; it may also be A or B).  nullptr: the plain product, C overwritten.
+    const Matrix* c_old = nullptr;
+    double alpha = 1.0, beta = 0.0;
 };
 void op_product(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix& C, const ProductOpts& o,
                 size_t* n_mults, size_t* n_blocks);

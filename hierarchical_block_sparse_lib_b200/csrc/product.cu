@@ -132,15 +132,17 @@ __global__ void k_task_finish(const uint64_t* __restrict__ keys, const uint32_t*
 // generic leaf GEMM (any blocksize, both dtypes): one CTA per C tile, plain FMA from global/L2.  Used for the
 // blocksizes without a tensor-pipe kernel and as the debug/parity variant (hbsm_set_gemm_variant(1)).
 // ---------------------------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool ACC>
 __global__ void __launch_bounds__(256) k_gemm_generic(const T* __restrict__ At, const T* __restrict__ Bt,
                                                        const uint2* __restrict__ ab, const uint64_t* __restrict__ begin,
                                                        const uint32_t* __restrict__ tile_list, int b, int tA, int tB,
-                                                       T* __restrict__ Ct) {
+                                                       T* __restrict__ Ct, AccEpi<T> epi) {
     const size_t bb = (size_t)b * b;
     const size_t ctile = tile_list ? tile_list[blockIdx.x] : blockIdx.x;   // optional indirection: a subset of C's tiles
     const uint64_t p0 = begin[ctile], p1 = begin[ctile + 1];
     T* C = Ct + ctile * bb;
+    const T* O = nullptr;
+    if constexpr (ACC) O = epi.old_at(ctile, bb, 0);
     for (size_t idx = threadIdx.x; idx < bb; idx += blockDim.x) {
         const int i = (int)(idx % b), j = (int)(idx / b);
         T acc = 0;
@@ -153,7 +155,8 @@ __global__ void __launch_bounds__(256) k_gemm_generic(const T* __restrict__ At, 
                 acc = fma(a, bv, acc);
             }
         }
-        C[idx] = acc;
+        if constexpr (ACC) C[idx] = epi.apply(acc, O, idx);
+        else C[idx] = acc;
     }
 }
 
@@ -202,11 +205,12 @@ struct TmaCfg {
 };
 
 // LS = leaf size, BS = compute tile of one CTA (BS == LS up to 128; a 256-leaf is 2 x 2 sub-tiles addressed in place)
-template <int LS, int BS, int KC, bool TA, bool TB>
+template <int LS, int BS, int KC, bool TA, bool TB, bool ACC>
 __global__ void __launch_bounds__(TmaCfg<BS, KC>::THREADS, 1)
 k_gemm_f64_tma(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                const uint2* __restrict__ ab, const uint64_t* __restrict__ begin, uint32_t n_ctiles,
-               const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, double* __restrict__ Ct) {
+               const uint32_t* __restrict__ tile_list, unsigned* __restrict__ next_tile, double* __restrict__ Ct,
+               AccEpi<double> epi) {
     using Cfg = TmaCfg<BS, KC>;
     constexpr int NST = Cfg::NST;
     constexpr int S = LS / BS;
@@ -335,13 +339,20 @@ k_gemm_f64_tma(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
         if (m.flags & 2) {
             const unsigned tile = (unsigned)m.ctile / (S * S), sub = (unsigned)m.ctile % (S * S);
             double* C = Ct + (size_t)tile * LS * LS + (size_t)((sub / S) * BS) * LS + (sub % S) * BS;
+            const double* O = nullptr;
+            if constexpr (ACC) O = epi.old_at(tile, (size_t)LS * LS, (size_t)((sub / S) * BS) * LS + (sub % S) * BS);
 #pragma unroll
             for (int i = 0; i < Cfg::MB; ++i)
 #pragma unroll
                 for (int j = 0; j < Cfg::NB; ++j) {
                     const int row = wm0 + i * 8 + g, col = wn0 + j * 8 + 2 * t;
-                    C[(size_t)col * LS + row] = acc[i][j][0];
-                    C[(size_t)(col + 1) * LS + row] = acc[i][j][1];
+                    if constexpr (ACC) {   // the old values in the store's own pattern
+                        C[(size_t)col * LS + row] = epi.apply(acc[i][j][0], O, (size_t)col * LS + row);
+                        C[(size_t)(col + 1) * LS + row] = epi.apply(acc[i][j][1], O, (size_t)(col + 1) * LS + row);
+                    } else {
+                        C[(size_t)col * LS + row] = acc[i][j][0];
+                        C[(size_t)(col + 1) * LS + row] = acc[i][j][1];
+                    }
                 }
         }
     }
@@ -361,14 +372,14 @@ void make_tile_map(CUtensorMap* map, const void* tiles, size_t n_tiles, int LS, 
         throw Error(HBSM_E_CUDA, "hbsm_b200: the driver refused the tensor map of an fp64 leaf operand");
 }
 
-template <int LS, int BS, int KC, bool TA, bool TB>
+template <int LS, int BS, int KC, bool TA, bool TB, bool ACC>
 void launch_gemm_f64_tma_inst(const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin, uint32_t n_ctiles,
-                              const uint32_t* tile_list, unsigned* counter, double* Ct) {
+                              const uint32_t* tile_list, unsigned* counter, double* Ct, const AccEpi<double>& epi) {
     using Cfg = TmaCfg<BS, KC>;
     CUtensorMap mapA, mapB;
     make_tile_map(&mapA, A.tiles.p, A.L, LS, BS, KC, TA, 8, CU_TENSOR_MAP_DATA_TYPE_FLOAT64);
     make_tile_map(&mapB, B.tiles.p, B.n_ext(), LS, BS, KC, !TB, 8, CU_TENSOR_MAP_DATA_TYPE_FLOAT64);
-    auto kfn = k_gemm_f64_tma<LS, BS, KC, TA, TB>;
+    auto kfn = k_gemm_f64_tma<LS, BS, KC, TA, TB, ACC>;
     static bool configured = false;
     if (!configured) {
         HB_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
@@ -377,16 +388,16 @@ void launch_gemm_f64_tma_inst(const Matrix& A, const Matrix& B, const uint2* ab,
     const uint64_t units = (uint64_t)n_ctiles * (LS / BS) * (LS / BS);
     if (units >= 0x7fffffffull) throw Error(HBSM_E_CUDA, "hbsm_b200: too many C sub-tiles for one fp64 leaf-GEMM launch");
     unsigned grid = (unsigned)std::min<uint64_t>(units, (uint64_t)engine().sm_count);
-    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct);
+    HB_LAUNCH(kfn, grid, Cfg::THREADS, Cfg::SMEM_BYTES, mapA, mapB, ab, begin, n_ctiles, tile_list, counter, Ct, epi);
 }
 
-template <int LS, int BS, int KC>
+template <int LS, int BS, int KC, bool ACC>
 void launch_gemm_f64_tma(bool tA, bool tB, const Matrix& A, const Matrix& B, const uint2* ab, const uint64_t* begin,
-                         uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, double* Ct) {
-    if (!tA && !tB) launch_gemm_f64_tma_inst<LS, BS, KC, false, false>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    else if (!tA && tB) launch_gemm_f64_tma_inst<LS, BS, KC, false, true>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    else if (tA && !tB) launch_gemm_f64_tma_inst<LS, BS, KC, true, false>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
-    else launch_gemm_f64_tma_inst<LS, BS, KC, true, true>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct);
+                         uint32_t n_ctiles, const uint32_t* tile_list, unsigned* counter, double* Ct, const AccEpi<double>& e) {
+    if (!tA && !tB) launch_gemm_f64_tma_inst<LS, BS, KC, false, false, ACC>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e);
+    else if (!tA && tB) launch_gemm_f64_tma_inst<LS, BS, KC, false, true, ACC>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e);
+    else if (tA && !tB) launch_gemm_f64_tma_inst<LS, BS, KC, true, false, ACC>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e);
+    else launch_gemm_f64_tma_inst<LS, BS, KC, true, true, ACC>(A, B, ab, begin, n_ctiles, tile_list, counter, Ct, e);
 }
 
 struct TaskList {
@@ -481,10 +492,11 @@ int coord_bits(const Matrix& A, const Matrix& B, int cm, int cn, int b) {
     return std::max(d, 1);
 }
 
-void check_operands(const Matrix& A, bool tA, const Matrix& B, bool tB, const Matrix& C, bool spamm, int& AM, int& BN) {
+// accumulate: C may be sized, with the product's shape, dtype and leaf size
+void check_operands(const Matrix& A, bool tA, const Matrix& B, bool tB, const Matrix& C, bool spamm, bool accumulate, int& AM, int& BN) {
     const char* fn = spamm ? "get_batches_spamm" : "get_batches_multiply";
     char msg[200];
-    if (!C.empty()) {   // H:5681 / H:6493
+    if (!accumulate && !C.empty()) {   // H:5681 / H:6493
         snprintf(msg, sizeof msg, "Error in HierarchicalBlockSparseMatrix::%s(): non-empty matrix to write result!%s", fn,
                  spamm ? "" : " wow");
         throw_ref(msg);
@@ -498,6 +510,8 @@ void check_operands(const Matrix& A, bool tA, const Matrix& B, bool tB, const Ma
         snprintf(msg, sizeof msg, "Error in HierarchicalBlockSparseMatrix::%s(): matrices have bad sizes!", fn);
         throw_ref(msg);
     }
+    if (accumulate && !C.empty() && (C.M != AM || C.N != BN || C.dtype != A.dtype || C.b != A.b))
+        throw Error(HBSM_E_ARG, "hbsm_b200: multiply_accumulate: C differs from op(A)*op(B) in shape, dtype or blocksize");
 }
 
 }  // namespace
@@ -546,6 +560,24 @@ __global__ void k_split_lists(const uint32_t* __restrict__ own_only, const uint6
     else later[i - pos[i]] = (uint32_t)i;
 }
 
+// accumulating product, per tile u of the union of P's C tiles (ckeys, begin) and C_old's tiles: its product range (empty
+// for a tile only in C_old: it starts where the next P tile starts) and whether it has products
+__global__ void k_union_ranges(const uint64_t* __restrict__ ukeys, const uint32_t* __restrict__ src_p, size_t nu,
+                               const uint64_t* __restrict__ ckeys, size_t nct, const uint64_t* __restrict__ begin,
+                               uint64_t* __restrict__ ubegin, uint32_t* __restrict__ has_products) {
+    size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= nu) return;
+    size_t j = src_p[u];
+    if (j == ACC_NONE) {
+        size_t lo = 0, hi = nct;
+        while (lo < hi) { size_t mid = (lo + hi) >> 1; if (ckeys[mid] < ukeys[u]) lo = mid + 1; else hi = mid; }
+        j = lo;
+    }
+    ubegin[u] = begin[j];
+    has_products[u] = src_p[u] != ACC_NONE ? 1u : 0u;
+    if (u == nu - 1) ubegin[nu] = begin[nct];
+}
+
 // one leaf-GEMM launch over `n` C tiles: all of them (tile_list == nullptr) or the listed subset.
 // One kernel per (dtype, leaf size); hbsm_set_gemm_variant only swaps in the parity references of the tests:
 //   dtype, leaf                        kernel                                                last_gemm_kernel
@@ -554,23 +586,31 @@ __global__ void k_split_lists(const uint32_t* __restrict__ own_only, const uint6
 //                                      variant 3: k_gemm_f32_q4<32 / 64> (single C tiles)
 //   fp32, 128 / 256                    k_gemm_f32_tc                                         3
 //   any other leaf size, or variant 1  k_gemm_generic (plain FMA)                            0
+//   a task list without products       k_gemm_generic (the only kernel that takes empty k-lists: the zero leaf of a
+//                                      single-leaf accumulate whose one leaf product SpAMM skips)  0
+// acc (may be null): the accumulating epilogue, in every kernel
 void launch_leaf_gemm(const Matrix& A, bool tA, const Matrix& B, bool tB, const TaskList& tl, const uint32_t* tile_list, size_t n,
-                      char* ct) {
+                      char* ct, const AccArgs* acc = nullptr) {
     if (n == 0) return;
     Engine& e = engine();
     const int variant = shared().gemm_variant.load();
     const uint32_t nn = (uint32_t)n;
     const bool tensor_leaf = A.b == 32 || A.b == 64 || A.b == 128 || A.b == 256;
-    if (variant == 1 || !tensor_leaf) {
-        if (A.dtype == HBSM_F64) {
-            auto kfn = k_gemm_generic<double>;
-            HB_LAUNCH(kfn, nn, 256, 0, (const double*)A.tiles.p, (const double*)B.tiles.p, tl.ab.p, tl.begin.p, tile_list, A.b,
-                      tA ? 1 : 0, tB ? 1 : 0, (double*)ct);
-        } else {
-            auto kfn = k_gemm_generic<float>;
-            HB_LAUNCH(kfn, nn, 256, 0, (const float*)A.tiles.p, (const float*)B.tiles.p, tl.ab.p, tl.begin.p, tile_list, A.b,
-                      tA ? 1 : 0, tB ? 1 : 0, (float*)ct);
-        }
+    const AccArgs plain;
+    const AccArgs& ea = acc ? *acc : plain;
+    if (variant == 1 || !tensor_leaf || tl.n_products == 0) {
+        with_acc(acc, [&](auto on) {
+            constexpr bool ACC = decltype(on)::value;
+            if (A.dtype == HBSM_F64) {
+                auto kfn = k_gemm_generic<double, ACC>;
+                HB_LAUNCH(kfn, nn, 256, 0, (const double*)A.tiles.p, (const double*)B.tiles.p, tl.ab.p, tl.begin.p, tile_list, A.b,
+                          tA ? 1 : 0, tB ? 1 : 0, (double*)ct, ea.epi<double>());
+            } else {
+                auto kfn = k_gemm_generic<float, ACC>;
+                HB_LAUNCH(kfn, nn, 256, 0, (const float*)A.tiles.p, (const float*)B.tiles.p, tl.ab.p, tl.begin.p, tile_list, A.b,
+                          tA ? 1 : 0, tB ? 1 : 0, (float*)ct, ea.epi<float>());
+            }
+        });
         e.last_gemm_kernel = 0;
         return;
     }
@@ -578,16 +618,20 @@ void launch_leaf_gemm(const Matrix& A, bool tA, const Matrix& B, bool tB, const 
     counter.zero();
     if (A.dtype == HBSM_F64) {
         double* Ct = (double*)ct;
-        switch (A.b) {
-            case 32: launch_gemm_f64_tma<32, 32, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
-            case 64: launch_gemm_f64_tma<64, 64, 64>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
-            case 128: launch_gemm_f64_tma<128, 128, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
-            default: launch_gemm_f64_tma<256, 128, 32>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct); break;
-        }
+        const AccEpi<double> ep = ea.epi<double>();
+        with_acc(acc, [&](auto on) {
+            constexpr bool ACC = decltype(on)::value;
+            switch (A.b) {
+                case 32: launch_gemm_f64_tma<32, 32, 32, ACC>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct, ep); break;
+                case 64: launch_gemm_f64_tma<64, 64, 64, ACC>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct, ep); break;
+                case 128: launch_gemm_f64_tma<128, 128, 32, ACC>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct, ep); break;
+                default: launch_gemm_f64_tma<256, 128, 32, ACC>(tA, tB, A, B, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, Ct, ep); break;
+            }
+        });
         e.last_gemm_kernel = 1;
     } else {   // split-TF32 on tcgen05 (gemm_f32.cu)
         launch_gemm_f32_tc(A, tA, B, tB, tl.ab.p, tl.begin.p, nn, tile_list, counter.p, (float*)ct, tl.ckeys.p, tl.task_k.p,
-                           tl.n_products, variant == 3);
+                           tl.n_products, variant == 3, acc);
         e.last_gemm_kernel = 3;
     }
 }
@@ -605,6 +649,8 @@ struct PendingProduct {
     size_t n_first = 0;
     bool first_pending = false, first_is_list = false;
     bool upper_only = false;     // finish zeroes the strict lower part of C's diagonal tiles (H:3563 via triu)
+    bool replace_table = false;  // finish installs the planned table even without products (accumulate into a sized C)
+    size_t old_mults = 0;        // C_old's n_mults when it takes part (accumulate, beta != 0)
     uint64_t launches0 = 0;
     EventTimer t_total, t_norm, t_index, t_task, t_gemm, t_gemm2;
 };
@@ -621,13 +667,23 @@ void op_product_begin(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix
     PendingProduct& P = pending();
     if (P.active) throw Error(HBSM_E_ARG, "hbsm_b200: a product is already in flight (finish it first)");
     int AM = 0, BN = 0;
-    check_operands(A, tA, B, tB, C, o.spamm, AM, BN);
+    const bool accumulate = o.c_old != nullptr;
+    if (accumulate && (o.c_old != &C || defer_halo_tiles || !launch || o.upper_only))
+        throw Error(HBSM_E_ARG, "hbsm_b200: an accumulating product runs in one call, on C's own table");
+    check_operands(A, tA, B, tB, C, o.spamm, accumulate, AM, BN);
     Engine& e = engine();
     P.launches0 = e.launches;
     P.t_total.start();
-    C.dtype = A.dtype;
-    C.b = A.b;
-    C.resize(AM, BN);
+    // accumulate into a sized C: its table (C_old) stays in place -- C may be A or B -- until finish installs the new one
+    const bool sized_old = accumulate && C.sized;
+    const bool use_old = sized_old && o.beta != 0.0 && C.L > 0;   // beta == 0: C_old is not read (BLAS)
+    P.replace_table = sized_old;
+    P.old_mults = sized_old && o.beta != 0.0 ? C.n_mults : 0;
+    if (!sized_old) {
+        C.dtype = A.dtype;
+        C.b = A.b;
+        C.resize(AM, BN);
+    }
     const int kbits = coord_bits(A, B, AM, BN, A.b);
     if (3 * kbits > 64) throw Error(HBSM_E_ARG, "hbsm_b200: block grid too deep for 64-bit task keys (depth > 21)");
 
@@ -677,14 +733,63 @@ void op_product_begin(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix
         n_first = (size_t)read_scalars(pos.p + nct, nullptr).first;
         P.n_later = nct - n_first;
     }
+    // a single-leaf product always has its leaf: when SpAMM skips the one leaf product, P is the zero leaf of resize(), and an
+    // accumulating product runs it as a C tile with an empty k-list, so its epilogue gives fl(fl(alpha * 0) + fl(beta * c))
+    const bool zero_leaf = accumulate && P.tl.n_products == 0 && Matrix::depth_for(AM, BN, A.b) == 0;
+    if (zero_leaf) {
+        P.tl.ckeys.alloc(1);
+        P.tl.ckeys.zero();
+        P.tl.begin.alloc(2);
+        P.tl.begin.zero();
+        P.tl.n_ctiles = 1;
+        n_first = 1;
+        P.replace_table = true;
+    }
     P.t_task.stop();
 
-    if (P.tl.n_products > 0) P.ct.alloc(P.tl.n_ctiles * C.tile_bytes());   // before the timer: a growing pool stalls the host here
+    // accumulate, beta != 0: C's table becomes the union of P's tiles and C_old's; the leaf GEMMs run over the union tiles with
+    // products (gemm_list, ascending) and read their old values through old_of, the C_old-only tiles get fl(beta * c)
+    AccArgs acc;
+    DevBuf<uint32_t> old_of, gemm_list, old_only;
+    size_t n_old_only = 0;
+    if (use_old) {
+        const size_t nct = P.tl.n_ctiles;
+        DevBuf<uint64_t> ukeys;
+        DevBuf<uint32_t> src_p;
+        const size_t nu = key_union(P.tl.ckeys.p, nct, C.keys.p, C.L, ukeys, src_p, old_of);
+        DevBuf<uint64_t> ubegin(nu + 1), pos(nu + 1);
+        DevBuf<uint32_t> has(nu);
+        if (nct == 0) {   // no C tile from the product: an empty task table to range over
+            P.tl.begin.alloc(1);
+            P.tl.begin.zero();
+        }
+        HB_LAUNCH(k_union_ranges, blocks_for(nu, 256), 256, 0, ukeys.p, src_p.p, nu, P.tl.ckeys.p, nct, P.tl.begin.p, ubegin.p, has.p);
+        exclusive_scan_u32(has.p, pos.p, nu);
+        gemm_list.alloc(std::max<size_t>(nct, 1));
+        n_old_only = nu - nct;
+        old_only.alloc(std::max<size_t>(n_old_only, 1));
+        HB_LAUNCH(k_split_lists, blocks_for(nu, 256), 256, 0, has.p, pos.p, nu, gemm_list.p, old_only.p);
+        P.tl.ckeys = std::move(ukeys);
+        P.tl.begin = std::move(ubegin);
+        P.tl.n_ctiles = nu;
+        first.release();
+        n_first = nct;
+        acc.idx = old_of.p;
+    }
+    if (accumulate) {
+        acc.old = C.tiles.p;
+        acc.alpha = o.alpha;
+        acc.beta = o.beta;
+    }
+    const bool fill = P.tl.n_products > 0 || zero_leaf || (use_old && P.tl.n_ctiles > 0);
+    if (fill) P.ct.alloc(P.tl.n_ctiles * C.tile_bytes());   // before the timer: a growing pool stalls the host here
     P.t_gemm.start();
-    if (P.tl.n_products > 0) {
-        if (launch) launch_leaf_gemm(A, tA, B, tB, P.tl, split ? first.p : nullptr, n_first, P.ct.p);
+    if (P.tl.n_products > 0 || zero_leaf) {
+        if (accumulate) launch_leaf_gemm(A, tA, B, tB, P.tl, use_old ? gemm_list.p : nullptr, n_first, P.ct.p, &acc);
+        else if (launch) launch_leaf_gemm(A, tA, B, tB, P.tl, split ? first.p : nullptr, n_first, P.ct.p);
         else if (launch_in_finish) { P.first_pending = true; P.first_is_list = split; P.n_first = n_first; }
     }
+    if (use_old) scale_tiles_into(C, old_of.p, old_only.p, n_old_only, o.beta, P.ct.p);
     P.t_gemm.stop();
     P.A = &A; P.B = &B; P.C = &C; P.tA = tA; P.tB = tB;
     P.upper_only = o.upper_only;
@@ -706,19 +811,26 @@ void op_product_finish(Matrix& C, cudaEvent_t wait_for, size_t* n_mults, size_t*
     P.t_gemm2.start();
     if (P.n_later > 0) launch_leaf_gemm(*P.A, P.tA, *P.B, P.tB, P.tl, P.later.p, P.n_later, P.ct.p);
     P.t_gemm2.stop();
-    if (P.tl.n_products > 0) {
+    if (P.tl.n_products > 0 || P.replace_table) {
+        // (an accumulating product releases C_old's buffers here, in stream order behind the kernels that read them)
         const size_t nct = P.tl.n_ctiles;
+        C.drop_tasks();
         C.set_table(std::move(P.tl.ckeys), std::move(P.ct), nct);
-        C.task_begin = std::move(P.tl.begin);
-        C.task_k = std::move(P.tl.task_k);
-        C.n_tasks = P.tl.n_products;
+        C.root_norm_cached = 0.0;   // stale with the leaf norms, as after resize()
+        if (nct > 0) {
+            C.task_begin = std::move(P.tl.begin);
+            C.task_k = std::move(P.tl.task_k);
+            C.n_tasks = P.tl.n_products;
+        }
         if (P.upper_only) mask_diag_upper(C);   // triu of the diagonal tiles (the off-diagonal ones were never planned)
     }
     P.t_total.stop();
     sync_stream();
     P.later.release();
     P.first.release();
-    C.n_mults = P.tl.n_products;   // H:2194 / H:3984
+    C.n_mults = P.tl.n_products + P.old_mults;   // H:2194 / H:3984; accumulate: + C_old's as add does (H:1719)
+    P.replace_table = false;
+    P.old_mults = 0;
     if (n_mults) *n_mults = P.tl.n_products;
     if (n_blocks) *n_blocks = C.L;   // get_n_blocks(), H:7311
     hbsm_stage_times st{};
@@ -879,7 +991,7 @@ void op_product_from_host(Matrix& A, const HostTiles& ha, bool tA, Matrix& B, co
     };
     if (&A == &B) throw Error(HBSM_E_ARG, "hbsm_b200: product_from_host needs two distinct operand handles");
     int AM = 0, BN = 0;
-    check_operands(A, tA, B, tB, C, o.spamm, AM, BN);
+    check_operands(A, tA, B, tB, C, o.spamm, false, AM, BN);
     if ((ha.n && (!ha.bi || !ha.bj || !ha.tiles)) || (hb.n && (!hb.bi || !hb.bj || !hb.tiles)))
         throw Error(HBSM_E_ARG, "hbsm_b200: product_from_host: null tile arrays");
     const uint64_t launches0 = e.launches;

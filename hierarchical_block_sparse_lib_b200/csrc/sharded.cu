@@ -133,9 +133,6 @@ void dispatch_real(int dtype, F&& f) {
 }
 
 // ---- kernels ----
-template <typename T> struct DT;   // un-fused round-to-nearest products: the predicate's arithmetic (H:2008) exactly
-template <> struct DT<double> { static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); } };
-template <> struct DT<float> { static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); } };
 template <typename T> struct IntOf;
 template <> struct IntOf<double> { typedef long long I; };
 template <> struct IntOf<float> { typedef int I; };

@@ -150,6 +150,23 @@ class HierarchicalBlockSparseMatrix:
         return nm.value, nr.value
 
     @staticmethod
+    def multiply_accumulate(A, tA, B, tB, Cm, alpha, beta):
+        """Cm <- alpha*op(A)*op(B) + beta*Cm in one call (hbsm_multiply_accumulate); Cm may be A and/or B, or unsized.
+        Returns (n_mults, n_resizes): the leaf products executed and Cm's tile count."""
+        nm = C.c_size_t(0); nr = C.c_size_t(0)
+        check(lib().hbsm_multiply_accumulate(A._h, int(bool(tA)), B._h, int(bool(tB)), Cm._h, float(alpha), float(beta), 0, 0.0, 1,
+                                             C.byref(nm), C.byref(nr)))
+        return nm.value, nr.value
+
+    @staticmethod
+    def spamm_accumulate(A, tA, B, tB, Cm, alpha, beta, tau, updated=True):
+        """Cm <- alpha*spamm(op(A), op(B), tau) + beta*Cm in one call, otherwise as multiply_accumulate."""
+        nm = C.c_size_t(0); nr = C.c_size_t(0)
+        check(lib().hbsm_multiply_accumulate(A._h, int(bool(tA)), B._h, int(bool(tB)), Cm._h, float(alpha), float(beta), 1, float(tau),
+                                             int(bool(updated)), C.byref(nm), C.byref(nr)))
+        return nm.value, nr.value
+
+    @staticmethod
     def product_from_host(A, a_bi, a_bj, a_tiles, tA, B, b_bi, b_bj, b_tiles, tB, Cm, spamm=False, tau=0.0, out_tiles=None,
                           n_slabs=0):
         """Host-to-host multiply / SpAMM as one pipeline (hbsm_product_from_host): A and B are sized, tile-less matrices

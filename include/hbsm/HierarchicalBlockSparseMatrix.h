@@ -171,6 +171,26 @@ public:
         if (no_of_resizes) *no_of_resizes = nr;
     }
 
+    // engine extras: C <- alpha * op(A) * op(B) + beta * C in one call (hbsm_multiply_accumulate); C may be A and/or B, or empty.
+    // The out-parameters are those of multiply / spamm: products executed, and C's block count.
+    static void multiply_accumulate(HierarchicalBlockSparseMatrix<Treal> const& A, bool tA, HierarchicalBlockSparseMatrix<Treal> const& B,
+                                    bool tB, HierarchicalBlockSparseMatrix<Treal>& C, Treal alpha, Treal beta,
+                                    size_t* no_of_block_multiplies = NULL, size_t* no_of_resizes = NULL) {
+        size_t nm = 0, nr = 0;
+        detail::check(hbsm_multiply_accumulate(A.h_, tA ? 1 : 0, B.h_, tB ? 1 : 0, C.h_, (double)alpha, (double)beta, 0, 0.0, 1, &nm, &nr));
+        if (no_of_block_multiplies) *no_of_block_multiplies = nm;
+        if (no_of_resizes) *no_of_resizes = nr;
+    }
+    static void spamm_accumulate(HierarchicalBlockSparseMatrix<Treal> const& A, bool tA, HierarchicalBlockSparseMatrix<Treal> const& B,
+                                 bool tB, HierarchicalBlockSparseMatrix<Treal>& C, Treal alpha, Treal beta, const Treal tau,
+                                 bool updated = true, size_t* no_of_block_multiplies = NULL, size_t* no_of_resizes = NULL) {
+        size_t nm = 0, nr = 0;
+        detail::check(hbsm_multiply_accumulate(A.h_, tA ? 1 : 0, B.h_, tB ? 1 : 0, C.h_, (double)alpha, (double)beta, 1, (double)tau,
+                                               updated ? 1 : 0, &nm, &nr));
+        if (no_of_block_multiplies) *no_of_block_multiplies = nm;
+        if (no_of_resizes) *no_of_resizes = nr;
+    }
+
     static int get_blocksize(Params const& param, int /*max_dimension*/) { return param.blocksize; }   // H:315
 
     bool check_if_matrix_is_consistent() const { int v = 0; detail::check(hbsm_is_consistent(h_, &v)); return v != 0; }   // H:396

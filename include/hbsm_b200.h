@@ -235,6 +235,29 @@ int hbsm_spectral_block_trunc(hbsm_handle A, int symmetric_upper, double eps, in
 int hbsm_truncation_spectral_errors(hbsm_handle A, int symmetric_upper, size_t n, const double* taus, int max_iter, double rel_tol,
                                     double* out_norms, int* out_iters);
 
+/* ---- accumulating product (engine extra; BLAS form: the reference's multiply / spamm need an empty C) ----
+ * C <- alpha * op(A) * op(B) + beta * C: multiply (spamm = 0) or SpAMM with tau (as hbsm_spamm, `updated` included), in one
+ * call, without a stored product or temporaries the size of C.  P below is what hbsm_multiply / hbsm_spamm would compute.
+ * - C may be the same handle as A, as B, or as both (X <- 2X - X*X is one call): only the old contents of every operand are
+ *   read, and C's new table is installed after the leaf GEMMs.
+ * - C may be unsized: it is then a zero matrix of the product's shape and gets sized.  A sized C must have op(A)'s row
+ *   count, op(B)'s column count, A's dtype and leaf size.
+ * - Values, bit for bit, are those of add(rescale(P, alpha), rescale(C, beta)): tiles of P and of C, fl(fl(alpha p) +
+ *   fl(beta c)) where both have the tile, fl(alpha p) or fl(beta c) where one has it.  beta == 0 never reads C (NaN or Inf
+ *   there does not propagate) and the result is rescale(P, alpha), P's tiles only.  In fp32 alpha and beta are rounded to
+ *   float first, as hbsm_rescale does.  A single-leaf product whose one leaf product SpAMM skips is P's zero leaf, as
+ *   hbsm_spamm leaves it: fl(fl(alpha 0) + fl(beta c)), signs of zeros and non-finite alpha included.
+ * - *n_block_multiplies = the leaf products executed, *n_resizes = C's tile count after the call.  C's n_mults is the
+ *   executed count, plus C's previous n_mults when beta != 0 (as hbsm_add adds them).  Cached leaf norms are stale and
+ *   the cached root norm is 0, as after a product.  The task hooks (hbsm_export_tasks, hbsm_task_checksum, hbsm_export_tile_tasks) report this call's products (none for a tile that
+ *   came only from the old C), hbsm_stage_times_last is filled in (gemm_ms includes the scaling of the old-only tiles).
+ *   A committed halo of B takes part as in hbsm_multiply; a halo on C is dropped.
+ * - Deterministic (bitwise repeatable).  HBSM_E_ARG before any device work: the operand errors of hbsm_multiply /
+ *   hbsm_spamm (same codes and messages; only "C must be empty" is dropped), a sized C of the wrong shape, dtype or leaf
+ *   size, and a product already in flight on this thread (hbsm_product_begin). */
+int hbsm_multiply_accumulate(hbsm_handle A, int tA, hbsm_handle B, int tB, hbsm_handle C, double alpha, double beta,
+                             int spamm, double tau, int updated, size_t* n_block_multiplies, size_t* n_resizes);
+
 /* ---- parity / bench hooks ---- */
 /* executed products of the call that produced C, sorted by (Morton key of (ci,cj), k); cap=0 -> count */
 int hbsm_export_tasks(hbsm_handle C, size_t cap, int64_t* ci, int64_t* cj, int64_t* k, size_t* n);
