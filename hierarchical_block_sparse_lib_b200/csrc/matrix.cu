@@ -1492,19 +1492,20 @@ void op_assemble_quadrants(Matrix& C, int M, int N, const Matrix* quads[4]) {
     for (int q = 0; q < 4; ++q) if (quads[q] && !quads[q]->empty()) { if (!first) first = quads[q]; }
     if (!first) throw Error(HBSM_E_ARG, "hbsm_b200: assemble_quadrants needs at least one quadrant");
     for (int q = 0; q < 4; ++q) if (quads[q] == &C) throw Error(HBSM_E_ARG, "hbsm_b200: assemble_quadrants: target aliases a quadrant");
-    C.clear();
-    C.dtype = first->dtype;
-    C.b = first->b;
-    C.resize(M, N);
-    const int P = C.vdepth();
+    if (M < 0 || N < 0) throw Error(HBSM_E_ARG, "hbsm_b200: negative dimension");
+    const int P = Matrix::depth_for(M, N, first->b);   // every check before C is cleared: a refused call leaves C as it was
     if (P == 0) throw Error(HBSM_E_ARG, "hbsm_b200: assemble_quadrants: the target is a single leaf");
     size_t total = 0;
     for (int q = 0; q < 4; ++q) {
         if (!quads[q] || quads[q]->empty()) continue;
-        if (quads[q]->vdepth() != P - 1 || quads[q]->b != C.b || quads[q]->dtype != C.dtype)
+        if (quads[q]->vdepth() != P - 1 || quads[q]->b != first->b || quads[q]->dtype != first->dtype)
             throw Error(HBSM_E_ARG, "hbsm_b200: assemble_quadrants: quadrant shape does not fit the target");
         total += quads[q]->L;
     }
+    C.clear();
+    C.dtype = first->dtype;
+    C.b = first->b;
+    C.resize(M, N);
     if (total == 0) return;
     DevBuf<uint64_t> keys(total);
     DevBuf<char> tiles(total * C.tile_bytes());
@@ -1527,6 +1528,7 @@ void op_leaf_inv_chol(const Matrix& A, Matrix& Z, int zdim, int valid) {
     ensure_engine();
     if (A.empty() || A.vdepth() != 0 || A.L != 1) throw Error(HBSM_E_ARG, "hbsm_b200: leaf_inv_chol wants a single-leaf matrix");
     if (zdim <= 0 || zdim > A.b) throw Error(HBSM_E_ARG, "hbsm_b200: leaf_inv_chol: bad result dimension");
+    if (valid > zdim) throw Error(HBSM_E_ARG, "hbsm_b200: leaf_inv_chol: the factored block is larger than the result");
     if (A.b > 256) throw Error(HBSM_E_ARG, "hbsm_b200: leaf_inv_chol supports leaves up to 256");
     Z.dtype = A.dtype;
     Z.b = A.b;

@@ -452,7 +452,7 @@ public:
     // inv_chol H:3110: inverse Cholesky factor Z (upper triangular, Z^T A Z = I) by the reference's block recursion
     //   Z00 = invchol(A00);  X = -Z00 (Z00^T A01);  Z11 = invchol(A10 X + A11);  Z01 = X Z11
     // The recursion runs on the host over quadrant matrices; every product / sum in it is the engine's multiply / add /
-    // rescale on the GPU, only the b x b leaf factor (the scalar loop of H:3118-3140) is computed on the host.
+    // rescale on the GPU, and the b x b leaf factor (the scalar loop of H:3118-3140) is one device kernel, hbsm_leaf_inv_chol.
     static void inv_chol(HierarchicalBlockSparseMatrix<Treal> const& A, HierarchicalBlockSparseMatrix<Treal>& Z) {
         if (!Z.empty()) throw std::runtime_error("Error in HierarchicalBlockSparseMatrix::inv_chol(): non-empty matrix to write result!");
         if (A.get_n_rows() != A.get_n_cols()) throw std::runtime_error("Error in HierarchicalBlockSparseMatrix::inv_chol(): call for non-square matrix!");

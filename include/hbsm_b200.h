@@ -155,7 +155,7 @@ int hbsm_leaf_norms(hbsm_handle h, size_t cap, void* out, size_t* n);
 int hbsm_extract_quadrant(hbsm_handle A, int q, hbsm_handle C, int* exists);   /* *exists = 0: the child is absent */
 int hbsm_assemble_quadrants(hbsm_handle C, int n_rows, int n_cols, hbsm_handle q0, hbsm_handle q1, hbsm_handle q2, hbsm_handle q3);
 /* the dense leaf step of inv_chol (H:3118-3147) on device: A = a single-leaf matrix, Z <- zdim x zdim single-leaf inverse
- * Cholesky factor (upper triangular, Z^T A Z = I) of its leading valid x valid block */
+ * Cholesky factor (upper triangular, Z^T A Z = I) of its leading valid x valid block; valid <= zdim <= b <= 256 */
 int hbsm_leaf_inv_chol(hbsm_handle A, hbsm_handle Z, int zdim, int valid);
 
 /* ---- a-priori estimators from the CACHED norms (count_skips H:4945, get_spamm_errors H:5236); taus in double ---- */
