@@ -651,12 +651,27 @@ struct PendingProduct {
     bool upper_only = false;     // finish zeroes the strict lower part of C's diagonal tiles (H:3563 via triu)
     bool replace_table = false;  // finish installs the planned table even without products (accumulate into a sized C)
     size_t old_mults = 0;        // C_old's n_mults when it takes part (accumulate, beta != 0)
+    bool c_was_empty = false;    // begin sized C: an abort returns it to the empty state (dtype and leaf size as they were)
+    int c_dtype = 0, c_b = -1;
     uint64_t launches0 = 0;
     EventTimer t_total, t_norm, t_index, t_task, t_gemm, t_gemm2;
 };
 PendingProduct& pending() {
     thread_local PendingProduct p;   // per host thread: products of different threads do not meet
     return p;
+}
+
+// drops the planned product's buffers; a C that begin sized goes back to the empty state it was in
+void drop_pending(PendingProduct& P) {
+    P.tl = TaskList(); P.ct.release(); P.later.release(); P.first.release(); P.first_pending = false;
+    P.replace_table = false;
+    P.old_mults = 0;
+    if (P.c_was_empty && P.C) {
+        P.C->clear();
+        P.C->dtype = P.c_dtype;
+        P.C->b = P.c_b;
+    }
+    P.c_was_empty = false;
 }
 
 }  // namespace
@@ -671,6 +686,11 @@ void op_product_begin(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix
     if (accumulate && (o.c_old != &C || defer_halo_tiles || !launch || o.upper_only))
         throw Error(HBSM_E_ARG, "hbsm_b200: an accumulating product runs in one call, on C's own table");
     check_operands(A, tA, B, tB, C, o.spamm, accumulate, AM, BN);
+    // every other rejection comes before C is touched, too
+    const int kbits = coord_bits(A, B, AM, BN, A.b);
+    if (3 * kbits > 64) throw Error(HBSM_E_ARG, "hbsm_b200: block grid too deep for 64-bit task keys (depth > 21)");
+    if (o.spamm && !o.updated && B.n_halo > 0)
+        throw Error(HBSM_E_ARG, "hbsm_b200: spamm(updated=false) on an operand with a committed halo");
     Engine& e = engine();
     P.launches0 = e.launches;
     P.t_total.start();
@@ -679,13 +699,20 @@ void op_product_begin(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix
     const bool use_old = sized_old && o.beta != 0.0 && C.L > 0;   // beta == 0: C_old is not read (BLAS)
     P.replace_table = sized_old;
     P.old_mults = sized_old && o.beta != 0.0 ? C.n_mults : 0;
+    P.C = &C;
+    P.c_was_empty = !sized_old;   // (a product that is not accumulating requires an empty C)
+    P.c_dtype = C.dtype;
+    P.c_b = C.b;
+    struct Undo {   // anything below that throws leaves C as it was at the call
+        PendingProduct& P;
+        bool armed;
+        ~Undo() { if (armed) drop_pending(P); }
+    } undo{P, true};
     if (!sized_old) {
         C.dtype = A.dtype;
         C.b = A.b;
         C.resize(AM, BN);
     }
-    const int kbits = coord_bits(A, B, AM, BN, A.b);
-    if (3 * kbits > 64) throw Error(HBSM_E_ARG, "hbsm_b200: block grid too deep for 64-bit task keys (depth > 21)");
 
     P.t_norm.start();
     // updated=false: the reference copies A and B, refreshes the COPIES and leaves the operands' caches alone (H:3990-4005;
@@ -694,7 +721,6 @@ void op_product_begin(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix
     const void* an = nullptr;
     const void* bn = nullptr;
     if (o.spamm && !o.updated) {
-        if (B.n_halo > 0) throw Error(HBSM_E_ARG, "hbsm_b200: spamm(updated=false) on an operand with a committed halo");
         fresh_a.alloc(std::max<size_t>(A.L, 1) * A.esize());
         compute_leaf_norms(A, fresh_a.p);
         an = fresh_a.p;
@@ -791,8 +817,9 @@ void op_product_begin(const Matrix& A, bool tA, const Matrix& B, bool tB, Matrix
     }
     if (use_old) scale_tiles_into(C, old_of.p, old_only.p, n_old_only, o.beta, P.ct.p);
     P.t_gemm.stop();
-    P.A = &A; P.B = &B; P.C = &C; P.tA = tA; P.tB = tB;
+    P.A = &A; P.B = &B; P.tA = tA; P.tB = tB;
     P.upper_only = o.upper_only;
+    undo.armed = false;
     P.active = true;
 }
 
@@ -801,6 +828,7 @@ void op_product_finish(Matrix& C, cudaEvent_t wait_for, size_t* n_mults, size_t*
     if (!P.active || P.C != &C) throw Error(HBSM_E_ARG, "hbsm_b200: product_finish without a matching product_begin");
     Engine& e = engine();
     P.active = false;
+    P.c_was_empty = false;
     if (P.first_pending) {   // begin left every launch to us: own-only tiles now, the halo readers once `wait_for` has fired
         P.t_gemm.start();
         launch_leaf_gemm(*P.A, P.tA, *P.B, P.tB, P.tl, P.first_is_list ? P.first.p : nullptr, P.n_first, P.ct.p);
@@ -853,7 +881,7 @@ void op_product_abort() {
     if (!P.active) return;
     P.active = false;
     cudaStreamSynchronize(engine().stream);
-    P.tl = TaskList(); P.ct.release(); P.later.release(); P.first.release(); P.first_pending = false;
+    drop_pending(P);
 }
 
 // product whose C tiles stream to HOST memory while later tiles are still being computed: the leaf GEMM is launched in

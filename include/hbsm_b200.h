@@ -108,7 +108,9 @@ int hbsm_spamm(hbsm_handle A, int tA, hbsm_handle B, int tB, hbsm_handle C, doub
 int hbsm_product_begin(hbsm_handle A, int tA, hbsm_handle B, int tB, hbsm_handle C, int spamm, double tau, int updated,
                        int defer_halo_tiles);
 int hbsm_product_finish(hbsm_handle C, void* cuda_event_or_null, size_t* n_block_multiplies, size_t* n_resizes);
-/* drops the calling thread's product in flight, if any (a caller whose transfer failed between begin and finish) */
+/* drops the calling thread's product in flight, if any (a caller whose transfer failed between begin and finish); a C
+ * that was empty at begin is empty again.  A rejected begin leaves C as it was; a finish on another C is refused and
+ * drops the product the same way. */
 int hbsm_product_abort(void);
 /* the same begin with the symmetric-family option: upper_only != 0 plans only the C tiles with ci <= cj and finish zeroes
  * the strict lower part of the diagonal tiles (symm_square H:3563 / symm_rk H:3711 on an expanded operand; sharded:

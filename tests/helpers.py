@@ -1,12 +1,48 @@
 """Shared helpers for the parity tests: build the same matrix in the CUDA engine (through the C ABI) and in the CPU
 oracle from one set of COO triplets, and compare results."""
+import ctypes as C
+
 import numpy as np
 
 import hierarchical_block_sparse_lib_b200 as hb
+from hierarchical_block_sparse_lib_b200 import _capi
 from hierarchical_block_sparse_lib_b200 import generators as G
 from oracle import pyoracle as po
 
 HBSM = hb.HierarchicalBlockSparseMatrix
+
+
+def morton(bi, bj):
+    key = 0
+    for bit in range(21):
+        key |= ((int(bi) >> bit) & 1) << (2 * bit) | ((int(bj) >> bit) & 1) << (2 * bit + 1)
+    return key
+
+
+def commit_halo(X, bi, bj, seed=0, tiles=None, norms=None, nan_tiles=False, capacity=0):
+    """hbsm_halo_reserve / hbsm_halo_commit: len(bi) halo tiles at (bi, bj) on X, written in the given order.  The tiles
+    are `tiles` (rows of b*b, column-major) or random values from `seed`; the norms are `norms` or the tiles' leaf norms.
+    nan_tiles: the keys and norms as above, but every tile NaN (tiles still in transit).  The reserve has room for
+    max(capacity, len(bi)) tiles.  Returns the device address of the first halo tile."""
+    b = X.get_params().blocksize
+    n = len(bi)
+    if tiles is None:
+        tiles = np.random.default_rng(seed).uniform(-1, 1, (n, b * b))
+    tiles = np.ascontiguousarray(tiles, X.dtype).reshape(n, b * b)
+    if norms is None:
+        norms = (tiles.astype(np.float64) ** 2).sum(1)
+    norms = np.ascontiguousarray(norms, X.dtype)
+    keys = np.array([morton(i, j) for i, j in zip(bi, bj)], np.uint64)
+    written = np.full_like(tiles, np.nan) if nan_tiles else tiles
+    dk, dn, dt = C.c_void_p(), C.c_void_p(), C.c_void_p()
+    _capi.check(_capi.lib().hbsm_halo_reserve(X._h, max(n, capacity), C.byref(dk), C.byref(dn), C.byref(dt)))
+    cu = C.CDLL("libcuda.so.1")
+    assert cu.cuCtxSynchronize() == 0   # the reserve's copies on the engine stream are done
+    for ptr, arr in ((dk, keys), (dn, norms), (dt, written)):
+        if arr.nbytes:
+            assert cu.cuMemcpyHtoD_v2(C.c_uint64(ptr.value), arr.ctypes.data_as(C.c_void_p), C.c_size_t(arr.nbytes)) == 0
+    _capi.check(_capi.lib().hbsm_halo_commit(X._h, n))
+    return dt.value
 
 
 def gpu_from_coo(b, m, n, r, c, v, dtype=np.float64, update=True):

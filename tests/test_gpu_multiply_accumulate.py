@@ -13,6 +13,7 @@ import pytest
 import hierarchical_block_sparse_lib_b200 as hb
 from hierarchical_block_sparse_lib_b200 import _capi
 from hierarchical_block_sparse_lib_b200 import generators as G
+from helpers import commit_halo
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HM = hb.HierarchicalBlockSparseMatrix
@@ -378,29 +379,6 @@ def test_spamm_in_place_purification(engine, dtype, b, updated):
         assert_bitwise(X, want)
         assert nm == len(P.export_tasks()) > 0 and nr == want.get_n_blocks()
         assert np.array_equal(X.export_tasks(), P.export_tasks())
-
-
-def morton(bi, bj):
-    key = 0
-    for bit in range(21):
-        key |= ((int(bi) >> bit) & 1) << (2 * bit) | ((int(bj) >> bit) & 1) << (2 * bit + 1)
-    return key
-
-
-def commit_halo(X, bi, bj, seed):
-    """hbsm_halo_reserve / hbsm_halo_commit: len(bi) halo tiles of random values at (bi, bj) on X"""
-    b = X.get_params().blocksize
-    rng = np.random.default_rng(seed)
-    t = rng.uniform(-1, 1, (len(bi), b * b)).astype(X.dtype)
-    keys = np.array([morton(i, j) for i, j in zip(bi, bj)], np.uint64)
-    nrm = (t.astype(np.float64) ** 2).sum(1).astype(X.dtype)
-    dk, dn, dt = C.c_void_p(), C.c_void_p(), C.c_void_p()
-    _capi.check(_capi.lib().hbsm_halo_reserve(X._h, len(bi), C.byref(dk), C.byref(dn), C.byref(dt)))
-    cu = C.CDLL("libcuda.so.1")
-    assert cu.cuCtxSynchronize() == 0   # the reserve's copies on the engine stream are done
-    for ptr, arr in ((dk, keys), (dn, nrm), (dt, t)):
-        assert cu.cuMemcpyHtoD_v2(C.c_uint64(ptr.value), arr.ctypes.data_as(C.c_void_p), C.c_size_t(arr.nbytes)) == 0
-    _capi.check(_capi.lib().hbsm_halo_commit(X._h, len(bi)))
 
 
 @gpu
