@@ -35,6 +35,15 @@ class TruncInfo(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class SpammTolInfo(C.Structure):
+    """hbsm_spamm_tol_info"""
+    _fields_ = [("tau", C.c_double), ("bound", C.c_double), ("level", C.c_double), ("n_candidates", C.c_size_t),
+                ("n_skipped", C.c_size_t), ("n_levels", C.c_size_t)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 _H = C.c_void_p
 _sz = C.c_size_t
 _P = C.c_void_p
@@ -107,6 +116,8 @@ SIGNATURES = {
                                C.POINTER(_I)]),
     "hbsm_spectral_block_trunc": (_I, [_H, _I, C.c_double, _I, _H, C.POINTER(TruncInfo)]),
     "hbsm_truncation_spectral_errors": (_I, [_H, _I, _sz, _P, _I, C.c_double, _P, _P]),
+    "hbsm_spamm_error_bounds": (_I, [_H, _I, _H, _I, _I, _I, _sz, _P, _P, _P]),
+    "hbsm_spamm_tau_for_error": (_I, [_H, _I, _H, _I, _I, _I, C.c_double, C.POINTER(SpammTolInfo)]),
     "hbsm_multiply_accumulate": (_I, [_H, _I, _H, _I, _H, C.c_double, C.c_double, _I, C.c_double, _I, C.POINTER(_sz), C.POINTER(_sz)]),
     "hbsm_export_tasks": (_I, [_H, _sz, _P, _P, _P, C.POINTER(_sz)]),
     "hbsm_export_leaves": (_I, [_H, _sz, _P, _P, _P, _P, C.POINTER(_sz)]),

@@ -441,6 +441,25 @@ int hbsm_truncation_spectral_errors(hbsm_handle A, int symmetric_upper, size_t n
     return guarded([&] { truncation_spectral_errors(M(A), symmetric_upper != 0, n, taus, max_iter, rel_tol, out_norms, out_iters); });
 }
 
+int hbsm_spamm_error_bounds(hbsm_handle A, int tA, hbsm_handle B, int tB, int symm_square, int updated, size_t n, const double* taus,
+                            double* bounds, size_t* n_skipped) {
+    return guarded([&] { spamm_error_bounds(M(A), tA != 0, M(B), tB != 0, symm_square != 0, updated != 0, n, taus, bounds, n_skipped); });
+}
+int hbsm_spamm_tau_for_error(hbsm_handle A, int tA, hbsm_handle B, int tB, int symm_square, int updated, double eps,
+                             hbsm_spamm_tol_info* info) {
+    return guarded([&] {
+        const SpammTol t = spamm_tau_for_error(M(A), tA != 0, M(B), tB != 0, symm_square != 0, updated != 0, eps);
+        if (info) {
+            info->tau = t.tau;
+            info->bound = t.bound;
+            info->level = t.level;
+            info->n_candidates = t.n_candidates;
+            info->n_skipped = t.n_skipped;
+            info->n_levels = t.n_levels;
+        }
+    });
+}
+
 int hbsm_export_tasks(hbsm_handle Ch, size_t cap, int64_t* ci, int64_t* cj, int64_t* k, size_t* n) {
     return guarded([&] {
         Matrix& C = M(Ch);

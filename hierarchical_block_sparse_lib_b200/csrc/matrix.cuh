@@ -180,6 +180,21 @@ void op_product_from_host(Matrix& A, const HostTiles& ha, bool tA, Matrix& B, co
                           size_t* n_mults, size_t* n_blocks);
 void op_product_abort();
 void product_row_counts(const Matrix& A, bool tA, const Matrix& B, bool tB, const ProductOpts& o, uint64_t* d_out);
+// op_product's operand checks of a SpAMM product (same codes and messages), without a target and before any device work
+void check_spamm_operands(const Matrix& A, bool tA, const Matrix& B, bool tB, bool updated);
+// The candidate leaf pairs of op(A)*op(B): every (ci, k, cj) with both tiles present (only C tiles with ci <= cj when
+// upper_only), planned by the task-list builder without SpAMM.  begin[n_ctiles + 1] and ab[Q] = (A tile, B tile), grouped by
+// C tile in the order the product runs them; returns Q (begin and ab stay unallocated when Q == 0).
+size_t product_candidates(const Matrix& A, bool tA, const Matrix& B, bool tB, bool upper_only, DevBuf<uint64_t>& begin,
+                          DevBuf<uint2>& ab, size_t* n_ctiles);
+// ---- spamm_error.cu: SpAMM error control (DESIGN section 12) ----
+struct SpammTol {
+    double tau, bound, level;
+    size_t n_candidates, n_skipped, n_levels;
+};
+void spamm_error_bounds(const Matrix& A, bool tA, const Matrix& B, bool tB, bool symm_square, bool updated, size_t n,
+                        const double* taus, double* bounds, size_t* n_skipped);
+SpammTol spamm_tau_for_error(const Matrix& A, bool tA, const Matrix& B, bool tB, bool symm_square, bool updated, double eps);
 // ---- dense.cu: Y = alpha*op(A)*X + beta*Y with dense column-major X, Y in A's dtype (op: HBSM_OP_*), Lanczos on it ----
 void validate_dense(const Matrix& A, int op, int m, long long ldx, long long ldy, const void* X, const void* Y);   // HBSM_E_ARG
 void dense_product_device(const Matrix& A, int op, int m, const void* d_X, long long ldx, void* d_Y, long long ldy, double alpha,

@@ -528,6 +528,27 @@ void product_row_counts(const Matrix& A, bool tA, const Matrix& B, bool tB, cons
     build_tasks(A, tA, B, tB, o, kb, tl, true, 0, (size_t)-1, nullptr, nullptr, d_out);
 }
 
+void check_spamm_operands(const Matrix& A, bool tA, const Matrix& B, bool tB, bool updated) {
+    const Matrix none;
+    int AM = 0, BN = 0;
+    check_operands(A, tA, B, tB, none, true, false, AM, BN);
+    if (3 * coord_bits(A, B, AM, BN, A.b) > 64) throw Error(HBSM_E_ARG, "hbsm_b200: block grid too deep for 64-bit task keys (depth > 21)");
+    if (!updated && B.n_halo > 0) throw Error(HBSM_E_ARG, "hbsm_b200: spamm(updated=false) on an operand with a committed halo");
+}
+
+size_t product_candidates(const Matrix& A, bool tA, const Matrix& B, bool tB, bool upper_only, DevBuf<uint64_t>& begin,
+                          DevBuf<uint2>& ab, size_t* n_ctiles) {
+    ensure_engine();
+    ProductOpts o;
+    o.upper_only = upper_only;
+    TaskList tl;
+    build_tasks(A, tA, B, tB, o, coord_bits(A, B, tA ? A.N : A.M, tB ? B.M : B.N, A.b), tl, false);
+    begin = std::move(tl.begin);
+    ab = std::move(tl.ab);
+    *n_ctiles = tl.n_ctiles;
+    return tl.n_products;
+}
+
 bool worth_product(const Matrix& A, bool tA, const Matrix& B, bool tB, bool spamm, double tau) {
     if (A.empty() || B.empty()) return false;
     ensure_engine();

@@ -232,6 +232,29 @@ class HierarchicalBlockSparseMatrix:
         check(lib().hbsm_spamm_errors(A._h, int(bool(tA)), B._h, int(bool(tB)), len(t), _ptr(t), _ptr(out), C.byref(n)))
         return out[:n.value].astype(A.dtype)
 
+    # ---- engine extras: SpAMM with error control (hbsm_spamm_error_bounds / hbsm_spamm_tau_for_error) ----
+    @staticmethod
+    def spamm_error_bounds(A, tA, B, tB, taus, updated=True, symm_square=False):
+        """For each tau, a rigorous bound on ||P_exact - P_tau||_F (hence ||.||_2) of spamm(A, tA, B, tB, tau, updated) --
+        or, with symm_square, of symm_square_spamm(A, tau) on sym(triu(.)) -- and the leaf pairs it skips.  The leaf GEMMs'
+        own rounding is not included.  Returns (bounds float64, n_skipped uint64) numpy arrays."""
+        t = np.ascontiguousarray(np.atleast_1d(np.asarray(taus, np.float64)))
+        out = np.zeros(len(t), np.float64)
+        ns = np.zeros(len(t), np.uint64)
+        check(lib().hbsm_spamm_error_bounds(A._h, int(bool(tA)), B._h, int(bool(tB)), int(bool(symm_square)), int(bool(updated)),
+                                            len(t), _ptr(t), _ptr(out), _ptr(ns)))
+        return out, ns
+
+    @staticmethod
+    def spamm_tau_for_error(A, tA, B, tB, eps, updated=True, symm_square=False):
+        """The largest-skipping tau whose bound (spamm_error_bounds) is <= eps.  Returns the hbsm_spamm_tol_info as a dict:
+        tau, bound, level (the largest skipped norm^2 product, -1 when nothing is skipped), n_candidates, n_skipped,
+        n_levels."""
+        info = _capi.SpammTolInfo()
+        check(lib().hbsm_spamm_tau_for_error(A._h, int(bool(tA)), B._h, int(bool(tB)), int(bool(symm_square)), int(bool(updated)),
+                                             float(eps), C.byref(info)))
+        return info.as_dict()
+
     def get_size(self):
         return self._size("hbsm_serialized_size")
 

@@ -448,6 +448,26 @@ public:
         detail::check(hbsm_spamm_errors(A.h_, tA ? 1 : 0, B.h_, tB ? 1 : 0, t.size(), t.data(), out.data(), &n));
         return std::vector<Treal>(out.begin(), out.begin() + n);
     }
+    // SpAMM with error control (engine extras, hbsm_spamm_error_bounds / hbsm_spamm_tau_for_error): bounds[i] = a rigorous
+    // bound on ||P_exact - P_tau||_F of spamm(A, tA, B, tB, taus[i], updated) -- of symm_square_spamm(A, taus[i]) with
+    // symm_square -- and n_skipped[i] the leaf pairs it skips; the tau whose bound meets eps, with its record
+    static void spamm_error_bounds(HierarchicalBlockSparseMatrix<Treal> const& A, const bool tA, HierarchicalBlockSparseMatrix<Treal> const& B,
+                                   const bool tB, std::vector<Treal> const& taus, std::vector<double>& bounds,
+                                   std::vector<size_t>& n_skipped, bool updated = true, bool symm_square = false) {
+        std::vector<double> t(taus.begin(), taus.end());
+        bounds.assign(taus.size(), 0.0);
+        n_skipped.assign(taus.size(), 0);
+        detail::check(hbsm_spamm_error_bounds(A.h_, tA ? 1 : 0, B.h_, tB ? 1 : 0, symm_square ? 1 : 0, updated ? 1 : 0, t.size(),
+                                              t.empty() ? NULL : &t[0], bounds.empty() ? NULL : &bounds[0],
+                                              n_skipped.empty() ? NULL : &n_skipped[0]));
+    }
+    static hbsm_spamm_tol_info spamm_tau_for_error(HierarchicalBlockSparseMatrix<Treal> const& A, const bool tA,
+                                                   HierarchicalBlockSparseMatrix<Treal> const& B, const bool tB, double eps,
+                                                   bool updated = true, bool symm_square = false) {
+        hbsm_spamm_tol_info info;
+        detail::check(hbsm_spamm_tau_for_error(A.h_, tA ? 1 : 0, B.h_, tB ? 1 : 0, symm_square ? 1 : 0, updated ? 1 : 0, eps, &info));
+        return info;
+    }
 
     // inv_chol H:3110: inverse Cholesky factor Z (upper triangular, Z^T A Z = I) by the reference's block recursion
     //   Z00 = invchol(A00);  X = -Z00 (Z00^T A01);  Z11 = invchol(A10 X + A11);  Z01 = X Z11

@@ -237,6 +237,40 @@ int hbsm_spectral_block_trunc(hbsm_handle A, int symmetric_upper, double eps, in
 int hbsm_truncation_spectral_errors(hbsm_handle A, int symmetric_upper, size_t n, const double* taus, int max_iter, double rel_tol,
                                     double* out_norms, int* out_iters);
 
+/* ---- SpAMM with error control (engine extras; hbsm_spamm_errors keeps the reference's a-priori estimate) ----
+ * Candidates: the leaf pairs (ci, k, cj) of the exact product with A_ik of op(A) and B_kj of op(B) present (what
+ * hbsm_multiply executes).  Candidate level p = fl(nsq(A_ik) * nsq(B_kj)) in the dtype, from the cached norms (updated = 1) or
+ * from fresh norms in temporaries that leave the caches alone (updated = 0), exactly as hbsm_spamm forms it.  At tau a
+ * candidate is skipped iff !(p > fl(tau * tau)) in the dtype (fp32: tau rounded to float first); a NaN p at every tau.
+ * The bound of tau: sqrt(w * sum over C tiles t of S_t^2), S_t = the sum over t's skipped candidates of
+ * s = sqrt(nsq_A) sqrt(nsq_B) / (1 - gamma), gamma = b^2 u / (1 - b^2 u) covering the rounding of the computed nsq (u the
+ * dtype's unit roundoff), w = 1.  It bounds ||P_exact - P_tau||_F, hence ||.||_2, every operation rounded upward.  It bounds
+ * the error of skipping in exact arithmetic: the rounding of the leaf GEMMs that do run is separate.
+ * symm_square != 0: the product of hbsm_symm_square_spamm(A, C, tau) -- B must be A, tA = tB = 0, A square; the candidates
+ * are those of sym_expand(A) (norms refreshed, so `updated` is ignored) with ci <= cj, the error operator sym(triu(E)), and
+ * w = 2 (||sym(T)||_F^2 <= 2 ||T||_F^2 for every tile).  A committed halo of B takes part, as in hbsm_spamm.
+ * A NaN level makes every bound +Inf.  No candidates: bounds 0, tau 0.  One device pass, deterministic (bitwise repeatable).
+ * HBSM_E_ARG (before any device work): hbsm_spamm's operand errors (same codes and messages), n > 0 with a null taus or
+ * bounds, eps < 0, NaN or infinite, symm_square with another B, a transpose or a non-square A, updated = 0 with a committed
+ * halo on B. */
+typedef struct {
+    double tau;            /* pass to hbsm_spamm / hbsm_multiply_accumulate(spamm = 1) / hbsm_symm_square_spamm */
+    double bound;          /* certified bound of that tau (<= eps), Frobenius and hence also spectral */
+    double level;          /* v: largest skipped p (dtype value), -1 when nothing is skipped */
+    size_t n_candidates;   /* Q */
+    size_t n_skipped;      /* candidates skipped at tau: the product executes Q - n_skipped */
+    size_t n_levels;       /* distinct p among the candidates */
+} hbsm_spamm_tol_info;
+/* bounds[i] = the bound of taus[i]; n_skipped[i] (may be NULL) = candidates skipped at taus[i] */
+int hbsm_spamm_error_bounds(hbsm_handle A, int tA, hbsm_handle B, int tB, int symm_square, int updated, size_t n,
+                            const double* taus, double* bounds, size_t* n_skipped);
+/* The largest-skipping tau whose bound is <= eps: the highest level v with bound <= eps and a tau with v <= fl(tau * tau) <
+ * the next level, so the product at tau executes exactly the candidates with p > v.  When no tau squares into that interval
+ * the level below is taken; nothing skippable gives tau = 0.  HBSM_E_ARG after the pass: a NaN level, or pairs whose norm
+ * product underflows to 0 (skipped at every tau) with a bound above eps. */
+int hbsm_spamm_tau_for_error(hbsm_handle A, int tA, hbsm_handle B, int tB, int symm_square, int updated, double eps,
+                             hbsm_spamm_tol_info* info);
+
 /* ---- accumulating product (engine extra; BLAS form: the reference's multiply / spamm need an empty C) ----
  * C <- alpha * op(A) * op(B) + beta * C: multiply (spamm = 0) or SpAMM with tau (as hbsm_spamm, `updated` included), in one
  * call, without a stored product or temporaries the size of C.  P below is what hbsm_multiply / hbsm_spamm would compute.
