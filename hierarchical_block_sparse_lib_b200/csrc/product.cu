@@ -944,6 +944,10 @@ void op_product_to_host(const Matrix& A, bool tA, const Matrix& B, bool tB, Matr
     }
     op_product_finish(C, nullptr, n_mults, n_blocks);
     if (!streamed && host_tiles && C.L && cap_tiles < C.L) throw Error(HBSM_E_ARG, "hbsm_b200: host buffer too small for the tiles of C");
+    if (!streamed && host_tiles && C.L) {   // no product ran: C is the zero leaf resize() gives a single-leaf C
+        HB_CUDA(cudaMemcpyAsync(host_tiles, C.tiles.p, C.L * C.tile_bytes(), cudaMemcpyDeviceToHost, e.stream));
+        sync_stream();
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1253,6 +1257,16 @@ void op_product_from_host(Matrix& A, const HostTiles& ha, bool tA, Matrix& B, co
                 HB_LAUNCH(k_gather_slab_tiles, grid, 256, 0, idx.p, d_off.p, d_ptr.p, S, tb / 16, (uint4*)t.p);
                 C.set_table(std::move(skeys), std::move(t), n_ct);
                 C.drop_tasks();
+            }
+        } else if (C.L > 0) {   // no product ran: C is the zero leaf resize() gives a single-leaf C, and the caller gets it
+            if (host_ok && cap_tiles >= C.L) {
+                HB_CUDA(cudaEventRecord(done[0], e.stream));   // behind resize()'s zero fill
+                HB_CUDA(cudaStreamWaitEvent(ss.d2h, done[0], 0));
+                HB_CUDA(cudaMemcpyAsync(host_c_tiles, C.tiles.p, C.L * tb, cudaMemcpyDeviceToHost, ss.d2h));
+                hk = C.keys.to_host();
+                hk.resize(C.L);
+            } else {
+                host_ok = false;
             }
         }
         t_total.stop();

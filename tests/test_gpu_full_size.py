@@ -8,7 +8,7 @@ import pytest
 import hierarchical_block_sparse_lib_b200 as hb
 from hierarchical_block_sparse_lib_b200 import generators as G
 from oracle import pyoracle as po
-from helpers import HBSM, both_from_coo, sort_tasks, rel_frob
+from helpers import HBSM, both_from_coo, flat_rule_tasks, sort_tasks, rel_frob
 
 pytestmark = pytest.mark.gpu
 
@@ -17,31 +17,6 @@ pytestmark = pytest.mark.gpu
 def _built(oracle_built):
     hb.init(0)
     return oracle_built
-
-
-def flat_rule_tasks(A, tA, B, tB, tau, g, upper_only=False):
-    """{(ci,cj,k)}: both tiles exist and fl(nsq(A_tile) * nsq(B_tile)) > fl(tau*tau) in Treal (tau None = exact multiply)."""
-    abi, abj, an, _ = A.export_leaves(tiles=False)
-    bbi, bbj, bn, _ = B.export_leaves(tiles=False)
-    if tA: abi, abj = abj, abi          # op(A): ci = abi, k = abj
-    if tB: bbi, bbj = bbj, bbi          # op(B): k = bbi, cj = bbj
-    T = an.dtype.type
-    tau2 = None if tau is None else T(tau) * T(tau)
-    oa = np.argsort(abj, kind="stable"); ob = np.argsort(bbi, kind="stable")
-    a_ci, a_k, a_n = abi[oa], abj[oa], an[oa]
-    b_k, b_cj, b_n = bbi[ob], bbj[ob], bn[ob]
-    sa = np.searchsorted(a_k, np.arange(g + 1)); sb = np.searchsorted(b_k, np.arange(g + 1))
-    out = []
-    for k in range(g):
-        ia = slice(sa[k], sa[k + 1]); ib = slice(sb[k], sb[k + 1])
-        if ia.start == ia.stop or ib.start == ib.stop:
-            continue
-        keep = np.ones((ia.stop - ia.start, ib.stop - ib.start), bool) if tau2 is None else (a_n[ia][:, None] * b_n[ib][None, :]) > tau2
-        if upper_only:
-            keep &= a_ci[ia][:, None] <= b_cj[ib][None, :]
-        x, y = np.nonzero(keep)
-        out.append(np.stack([a_ci[ia][x], b_cj[ib][y], np.full(len(x), k)], 1))
-    return np.concatenate(out) if out else np.zeros((0, 3), np.int64)
 
 
 def test_cfg1_exact_multiply_random_block_sparse_vs_oracle():

@@ -13,7 +13,7 @@ import pytest
 import hierarchical_block_sparse_lib_b200 as hb
 from hierarchical_block_sparse_lib_b200 import _capi
 from hierarchical_block_sparse_lib_b200 import generators as G
-from helpers import commit_halo
+from helpers import assert_bitwise, check_call, commit_halo, composition, copy_of
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HM = hb.HierarchicalBlockSparseMatrix
@@ -71,13 +71,6 @@ def operands(dtype, b, kind):
     return decay(dtype, b, n, 5 + b), decay(dtype, b, n, 6 + b)
 
 
-def copy_of(X):
-    Y = HM(X.dtype, X.get_params().blocksize)
-    if not X.empty():
-        Y.copy(X)
-    return Y
-
-
 def old_matrix(case, P, seed):
     """C_old for one of the OLD cases, relative to the pattern of the product P"""
     b = P.get_params().blocksize
@@ -102,51 +95,6 @@ def old_matrix(case, P, seed):
         keep = ~inP[gi, gj] | (rng.random(len(gi)) < 0.3)
         bi, bj = gi[keep], gj[keep]
     return with_tiles(P.dtype, b, m, n, bi, bj, rng)
-
-
-def composition(A, tA, B, tB, Cold, alpha, beta, spamm=None, updated=True):
-    """add(rescale(P, alpha), rescale(C_old, beta)) on copies, with its P"""
-    b = A.get_params().blocksize
-    P = HM(A.dtype, b)
-    if spamm is None:
-        HM.multiply(A, tA, B, tB, P)
-    else:
-        HM.spamm(A, tA, B, tB, P, spamm, updated)
-    P1 = HM(A.dtype, b)
-    P1.rescale(P, alpha)
-    if beta == 0.0 or Cold.empty():
-        return P1, P
-    C1 = HM(A.dtype, b)
-    C1.rescale(Cold, beta)
-    R = HM(A.dtype, b)
-    HM.add(P1, C1, R)
-    return R, P
-
-
-def assert_bitwise(X, Y):
-    xi, xj, _, xt = X.export_leaves(norms=False)
-    yi, yj, _, yt = Y.export_leaves(norms=False)
-    assert np.array_equal(xi, yi) and np.array_equal(xj, yj)
-    it = np.uint64 if X.dtype == np.float64 else np.uint32
-    assert X.dtype == Y.dtype and np.array_equal(xt.view(it), yt.view(it))
-    assert (X.get_n_rows(), X.get_n_cols()) == (Y.get_n_rows(), Y.get_n_cols())
-
-
-def check_call(A, tA, B, tB, Cold, alpha, beta, spamm=None, updated=True):
-    want, P = composition(A, tA, B, tB, Cold, alpha, beta, spamm, updated)
-    Cm = copy_of(Cold)
-    old_mults = Cm.get_n_block_multiplications() if not Cm.empty() else 0
-    if spamm is None:
-        nm, nr = HM.multiply_accumulate(A, tA, B, tB, Cm, alpha, beta)
-    else:
-        nm, nr = HM.spamm_accumulate(A, tA, B, tB, Cm, alpha, beta, spamm, updated)
-    assert_bitwise(Cm, want)
-    assert nm == len(P.export_tasks())
-    assert nr == Cm.get_n_blocks()
-    assert Cm.get_n_block_multiplications() == nm + (old_mults if beta != 0.0 else 0)
-    assert np.array_equal(Cm.export_tasks(), P.export_tasks())
-    assert Cm.task_checksum() == P.task_checksum()
-    return Cm, P
 
 
 CASES = [(d, b, t, k) for d in DTYPES for b in BS for t in TRANS for k in ("decay", "random")]

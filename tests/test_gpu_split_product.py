@@ -13,7 +13,7 @@ import pytest
 import hierarchical_block_sparse_lib_b200 as hb
 from hierarchical_block_sparse_lib_b200 import _capi
 from hierarchical_block_sparse_lib_b200 import generators as G
-from helpers import commit_halo, morton
+from helpers import bits, check_exact, commit_halo, grouped_bound, klist_sums, morton, tiles_rc
 
 HM = hb.HierarchicalBlockSparseMatrix
 gpu = pytest.mark.gpu
@@ -117,81 +117,6 @@ def promised_kernel(dtype, b):
     if b not in (32, 64, 128, 256):
         return 0
     return 1 if dtype == np.float64 else 3
-
-
-def tiles_rc(X):
-    """C's tiles as (n, b, b) arrays indexed (row, col), with their block coordinates"""
-    b = X.get_params().blocksize
-    bi, bj, _, t = X.export_leaves(norms=False)
-    return bi, bj, t.reshape(-1, b, b).transpose(0, 2, 1)
-
-
-def bits(x):
-    return x.view(np.uint64 if x.dtype == np.float64 else np.uint32)
-
-
-def klist_sums(A, tA, Bf, tB, Cref):
-    """per C tile of Cref, the float64 sums over its exported k-list of op(A)(i,k) op(B)(k,j) (r) and of
-    |op(A)(i,k)| |op(B)(k,j)| (s), and K = b * (length of the k-list); computed with torch on the device"""
-    import torch
-    b = A.get_params().blocksize
-    dev = torch.device("cuda")
-
-    def stack(X):
-        bi, bj, _, t = X.export_leaves(norms=False)
-        g = int(max(bi.max(initial=0), bj.max(initial=0))) + 1
-        where = np.full((g, g), -1, np.int64)
-        where[bi, bj] = np.arange(len(bi))
-        return where, torch.from_numpy(t.astype(np.float64).reshape(-1, b, b)).to(dev).transpose(1, 2)
-
-    wa, ta = stack(A)
-    wb, tb = stack(Bf)
-    ci, cj, _ = tiles_rc(Cref)
-    tasks = Cref.export_tasks()
-    pos = {(i, j): p for p, (i, j) in enumerate(zip(ci.tolist(), cj.tolist()))}
-    ct = np.array([pos[(i, j)] for i, j in zip(tasks[:, 0].tolist(), tasks[:, 1].tolist())], np.int64)
-    ti, tj, tk = tasks[:, 0], tasks[:, 1], tasks[:, 2]
-    ia = wa[tk, ti] if tA else wa[ti, tk]
-    ib = wb[tj, tk] if tB else wb[tk, tj]
-    assert (ia >= 0).all() and (ib >= 0).all()
-    r = torch.zeros((len(ci), b, b), dtype=torch.float64, device=dev)
-    s = torch.zeros_like(r)
-    step = max(1, (1 << 27) // (b * b * 8))
-    for lo in range(0, len(tasks), step):
-        a = ta[torch.from_numpy(ia[lo:lo + step]).to(dev)]
-        bb = tb[torch.from_numpy(ib[lo:lo + step]).to(dev)]
-        if tA:
-            a = a.transpose(1, 2)
-        if tB:
-            bb = bb.transpose(1, 2)
-        idx = torch.from_numpy(ct[lo:lo + step]).to(dev)
-        r.index_add_(0, idx, a @ bb)
-        s.index_add_(0, idx, a.abs() @ bb.abs())
-    K = b * np.bincount(ct, minlength=len(ci))
-    return r.cpu().numpy(), s.cpu().numpy(), K
-
-
-def grouped_bound(s, K):
-    """|c - r| <= bound, element by element, for the fp32 grouped kernels (r, s: klist_sums).
-    Operands: x = hi + lo exactly, hi = x with 13 mantissa bits cleared, |lo| < 2^-10 |x|; the tensor core reads lo with
-    13 mantissa bits cleared too, an error below 2^-21 |x|.  The 32-leaf kernel multiplies all four of hi/lo x hi/lo, the
-    64-leaf kernel drops lo*lo (< 2^-20 |a b|), so one product a*b is off by at most (2^-20 + 2 * 2^-21 + 2^-42) |a b|
-    <= 2^-19 (1 + 2^-22) |a b|; summed, at most 2^-19 (1 + 2^-22) s.
-    Sums: every addition, truncating in the tensor core or rounding in the epilogue, errs by less than 2^-23 times the sum
-    of the magnitudes of the terms under it, at most s (1 + 2^-8) (the hi/lo parts of a b add up to at most
-    (1 + 2^-10)^2 |a b|).  A term passes through at most 2b + 2n + 1 <= 3K additions (n = K / b products in the k-list,
-    b >= 32): at most 2b in one accumulator (two super-products of b k's, or hi and lo rows of one), two epilogue adds
-    per stage and one final add.  So the sums add less than 3K 2^-23 s (1 + 2^-8) (1 + 2^-23)^(3K), and the float64
-    reference is within 3K 2^-53 s of the exact sum.  Total: below (2^-19 + 3.3 K 2^-23) s for K < 2^18.  The bound
-    doubles the first term and takes 4K for 3.3K."""
-    assert (K < 2 ** 18).all()
-    return (2.0 ** -18 + 4.0 * K[:, None, None] * 2.0 ** -23) * s
-
-
-def check_exact(c, r):
-    """integer operands: every element is the exact integer (signs of zeros aside, so compared after adding +0)"""
-    assert np.array_equal(bits(c + c.dtype.type(0)), bits(r.astype(c.dtype) + c.dtype.type(0))), \
-        "max |c - r| = %g" % np.abs(c.astype(np.float64) - r).max()
 
 
 def split_groups(ci, cj, in_second):
